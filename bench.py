@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Benchmark of the Groth16 prove path (BASELINE.json metric: Groth16 prove ms & proofs/s).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload c5]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload c5] [--dump-outputs DIR]
 
 One "step" = one full proof of the workload circuit: constraint-row evaluation, witness map
 (7 NTTs), 4 G1 MSMs + 1 G2 MSM, combine, serialization -- from the assignment z to the 192 proof
@@ -22,6 +22,11 @@ constraints, domain 2^22) -- the north-star configuration; it fits one GPU (abou
 `--impl reference` times the CPU restatement end to end (key generation, row evaluation and proof
 all in oracle/cpu: the GPU library is never loaded); the Rust reference itself cannot be built
 here (no cargo, un-vendored crates).  Rank 0 only.
+
+`--dump-outputs DIR` writes, after the timed steps, the proof of the last timed step of the workload as
+DIR/proof.npy: its 192 serialized bytes (A, B, C compressed) as float32.  Circuit, key and r, s come from
+fixed seeds, so two builds (or the two arms) run with the same arguments can be compared byte for byte.
+Nothing is written into the source tree, which may be read-only.
 """
 import argparse
 import ctypes
@@ -35,6 +40,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True            # no __pycache__ in the (possibly read-only) tree
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -186,6 +192,8 @@ def run_reference(args, rank, world):
         "e2e": {"value": val, "unit": "proofs/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "setup_s": setup_s, "proof_sha": hashlib.sha256(proof).hexdigest()[:16],
     })
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, proof)
 
 
 _REAL_STDOUT = None
@@ -202,6 +210,13 @@ def emit(line):
         os.write(_REAL_STDOUT, data)
 
 
+def dump_outputs(out_dir, proof):
+    """--dump-outputs: the proof bytes of the last timed step as DIR/proof.npy (float32 holds bytes exactly)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "proof.npy"), np.frombuffer(bytes(proof), dtype=np.uint8).astype(np.float32))
+
+
 # ----------------------------------------------------------------------------------------------------
 # GPU arm
 # ----------------------------------------------------------------------------------------------------
@@ -216,6 +231,7 @@ class Bench:
         self.ctx = self.pkg.Context(local_rank)
         self.L = self.ctx._lib
         self.dist = None
+        self.last_proof = None                  # proof bytes of the workload's last timed step
         if world > 1:
             import torch.distributed as dist
             self.dist = dist
@@ -355,6 +371,8 @@ class Bench:
         clocks = ClockSampler(self.local_rank)
         clocks.start()
         dev_s, wall_s = self.timed(step_value, steps)
+        if main:
+            self.last_proof = proof.tobytes()
         clk = clocks.stop()
         launches = L.b2z_kernel_launches(ctx.handle) - launches0
         ms = (ctypes.c_double * 8)()
@@ -597,14 +615,15 @@ def main():
     ap.add_argument("--workload", default="c5", choices=sorted(WORKLOADS))
     ap.add_argument("--cpu-steps", type=int, default=1, help="proofs timed for cpu_baseline (0 = skip)")
     ap.add_argument("--no-extra", action="store_true", help="skip the extra c2 measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's proof to DIR/proof.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "reference":
-        big = args.workload == "c5"
-        args.steps = min(args.steps, 2 if big else 3)       # bounded sample: a CPU proof takes seconds
-        args.warmup = 0 if big else min(args.warmup, 1)
+        args.warmup = 0 if args.workload == "c5" else min(args.warmup, 1)     # a CPU proof takes seconds
         run_reference(args, rank, world)
         return
     if args.warmup < 3:
@@ -622,7 +641,7 @@ def main():
     res = b.measure(args.workload, args.steps, args.warmup, main=True)
     extra = {}
     if not args.no_extra and args.workload != "c2":
-        e = b.measure("c2", max(args.steps, 10), args.warmup, main=False)
+        e = b.measure("c2", args.steps, args.warmup, main=False)
         if rank == 0:
             extra["c2"] = {k: e[k] for k in ("config", "value", "ms_per_step", "e2e", "gpu_launches", "roofline",
                                              "collective", "bytes_equal_single_gpu", "proof_sha") if k in e}
@@ -640,6 +659,8 @@ def main():
             "extra": extra,
         }
         emit(line)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, b.last_proof)
     if world > 1:
         import torch.distributed as dist
         dist.destroy_process_group()

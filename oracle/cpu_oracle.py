@@ -4,7 +4,9 @@ include/b200zk.h: uint64 limb arrays, Fr/Fq in Montgomery form, MSM scalars
 canonical."""
 import ctypes
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -44,11 +46,35 @@ def build(force=False):
     return _LIB_PATH
 
 
+def _in_tree_current():
+    """True when build() made the in-tree library on a CPU with this one's ISA flags, after the last source edit."""
+    try:
+        with open(_STAMP) as f:
+            if f.read().strip() != _host_signature():
+                return False
+        return os.path.getmtime(_LIB_PATH) >= os.path.getmtime(os.path.join(_HERE, "cpu", "ark_cpu.cpp"))
+    except OSError:
+        return False
+
+
+def _load():
+    """The in-tree library when it is current; otherwise a private build in a temporary directory, so that
+    loading never writes into the tree (bench.py may run from a read-only checkout)."""
+    if _in_tree_current():
+        return ctypes.CDLL(_LIB_PATH)
+    tmp = tempfile.mkdtemp(prefix="ark_cpu_")
+    try:
+        path = os.path.join(tmp, "libark_cpu.so")
+        subprocess.run(["make", "-C", _HERE, "-s", "ARK_CPU_LIB=" + path], check=True)
+        return ctypes.CDLL(path)               # stays mapped after the directory is removed
+    finally:
+        shutil.rmtree(tmp, ignore_errors=True)
+
+
 def lib():
     global _lib
     if _lib is None:
-        build()                    # no-op when up to date and built for this CPU
-        L = ctypes.CDLL(_LIB_PATH)
+        L = _load()
         L.ark_cpu_set_threads.argtypes = [ctypes.c_int]
         L.ark_cpu_hardware_threads.restype = ctypes.c_int
         L.ark_cpu_ntt.argtypes = [vp, ctypes.c_uint32, ctypes.c_int, vp]

@@ -12,7 +12,7 @@ b = importlib.import_module("zksnark-finalproject_b200")
 fast = importlib.import_module("zksnark-finalproject_b200.circuits_fast")
 from oracle import bls12_381 as O
 
-BASE = {"B2Z_AFFINE_MIN_SEG": "128", "B2Z_AFFINE_G2": "0", "B2Z_AFFINE_MIN_PAIRS": "24", "B2Z_AFFINE_OCC": "2"}
+BASE = {"B2Z_AFFINE_MIN_SEG": "128", "B2Z_AFFINE_G2": "0", "B2Z_AFFINE_MIN_PAIRS": "24"}
 SETTINGS = {
     "xyzz": dict(BASE, B2Z_AFFINE_MIN_SEG="4000000000"),
     "affine": dict(BASE),
@@ -22,9 +22,7 @@ SETTINGS = {
     "affine_mp40": dict(BASE, B2Z_AFFINE_MIN_PAIRS="40"),
     "affine_mp48": dict(BASE, B2Z_AFFINE_MIN_PAIRS="48"),
     "affine_g2_mp32": dict(BASE, B2Z_AFFINE_G2="1", B2Z_AFFINE_MIN_PAIRS="32"),
-    "affine_occ3": dict(BASE, B2Z_AFFINE_OCC="3"),
     "affine_g2": dict(BASE, B2Z_AFFINE_G2="1"),
-    "affine_g2_occ3": dict(BASE, B2Z_AFFINE_G2="1", B2Z_AFFINE_OCC="3"),
     "affine_all": dict(BASE, B2Z_AFFINE_MIN_SEG="0", B2Z_AFFINE_G2="1"),
 }
 ap = argparse.ArgumentParser()

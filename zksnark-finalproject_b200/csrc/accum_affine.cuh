@@ -28,7 +28,8 @@
 namespace b2z {
 namespace aff {
 
-constexpr uint32_t kNegBit = 0x80000000u;
+constexpr uint32_t kNegBit = 0x80000000u;     // sign bit of a sorted point reference
+constexpr uint32_t kEmptyKey = 0xffffffffu;   // key of the partial slots of a segment past the end of the list
 constexpr uint32_t kMinPairsDefault = 24;
 
 // host emulation only: [0] completed rounds, [1] batched additions, [2] of which doublings, [3] division-free pairs
@@ -113,6 +114,96 @@ B2Z_HD void st_xyzz(typename C::Xyzz* dst, const typename C::Xyzz& v) {
   st_el(&dst->zzz, v.zzz);
 }
 
+// The segment protocol of both accumulation kernels (msm_impl.inc) and of the host emulation (hostcheck.cu).
+// The `total` sorted references are cut into nseg segments of seg_len = max(8, ceil(total / nseg)), one per thread;
+// segment `seg` covers [lo, hi).  The length follows the ACTUAL number of references (zero digits and identity bases
+// are gone), so the fixed grid stays busy whatever fraction of the scalars is zero or small.  A run of one bucket
+// that lies inside the segment goes straight to the bucket; a run cut by the segment's start goes to the leading
+// partial slot 2 seg, one cut by its end to the trailing slot 2 seg + 1.  Both slots are always written -- the
+// identity keyed by the first / last bucket when unused, kEmptyKey for a segment past the end -- so the partial list
+// stays sorted by key.
+template <class C>
+struct Segment {
+  using Xyzz = typename C::Xyzz;
+  uint32_t seg, seg_len, lo, hi, total;
+  uint32_t first, first_begin, first_end;   // first bucket: first_begin = offsets[first] <= lo < offsets[first + 1]
+  bool active;                              // seg < nseg and lo < total
+  bool wrote0, wrote1;
+  Xyzz* bucket_out;
+  uint32_t* part_keys;
+  Xyzz* part_pts;
+  uint32_t* maxrun;
+
+  B2Z_HD Segment(const uint32_t* offsets, uint32_t nbuckets, uint32_t nseg, uint32_t seg_, Xyzz* bucket_out_,
+                 uint32_t* part_keys_, Xyzz* part_pts_, uint32_t* maxrun_)
+      : seg(seg_), lo(0), hi(0), first(0), first_begin(0), first_end(0), wrote0(false), wrote1(false),
+        bucket_out(bucket_out_), part_keys(part_keys_), part_pts(part_pts_), maxrun(maxrun_) {
+    total = offsets[nbuckets];
+    seg_len = (total + nseg - 1) / nseg;
+    if (seg_len < 8) seg_len = 8;
+    active = seg < nseg && (uint64_t)seg * seg_len < total;
+    if (!active) return;
+    lo = seg * seg_len;
+    hi = umin(lo + seg_len, total);
+    uint32_t a = 0, z = nbuckets;   // largest bucket a with offsets[a] <= lo; invariant offsets[a] <= lo < offsets[z]
+    while (z - a > 1) {
+      const uint32_t mid = (a + z) >> 1;
+      if (offsets[mid] <= lo) a = mid; else z = mid;
+    }
+    first = a;
+    first_begin = offsets[a];
+    first_end = offsets[a + 1];
+    while (first_end <= lo) {        // skip empty buckets that share the same offset
+      first++;
+      first_begin = first_end;
+      first_end = offsets[first + 1];
+    }
+  }
+
+  // The run of bucket `key` (references [begin, end) of the whole list) ends inside this segment (end <= hi) with the
+  // sum `acc`: it goes to the leading slot or to the bucket.  This is flush() for a run that is not the segment's
+  // last: there (end - 1) / seg_len == seg, so its bound reduces to 2 (seg - begin / seg_len + 1).  The XYZZ kernel
+  // calls it inside its hot loop, where the trailing case of flush() costs the G2 kernel registers.
+  template <class Acc>
+  B2Z_HD void flush_inside(uint32_t key, uint32_t begin, const Acc& acc) {
+    if (begin < lo) {
+      part_keys[2 * seg] = key;
+      acc.store(part_pts + 2 * seg);
+      wrote0 = true;
+      raise_max(maxrun, 2 * (seg - begin / seg_len + 1));
+    } else {
+      acc.store(bucket_out + key);
+    }
+  }
+  // The segment's last run, of bucket `key` (references [begin, end) of the whole list), with the sum `acc`.
+  template <class Acc>
+  B2Z_HD void flush(uint32_t key, uint32_t begin, uint32_t end, const Acc& acc) {
+    if (begin < lo) {
+      part_keys[2 * seg] = key;
+      acc.store(part_pts + 2 * seg);
+      wrote0 = true;
+    } else if (end > hi) {
+      part_keys[2 * seg + 1] = key;
+      acc.store(part_pts + 2 * seg + 1);
+      wrote1 = true;
+    } else {
+      acc.store(bucket_out + key);
+    }
+    // entries this bucket can have in the partial list: 2 per segment it touches
+    if (begin < lo || end > hi) raise_max(maxrun, 2 * ((umin(end, total) - 1) / seg_len - begin / seg_len + 1));
+  }
+  // after the last run (keyed `last`) of an active segment
+  B2Z_HD void close(uint32_t last) {
+    if (!wrote0) { part_keys[2 * seg] = first; st_xyzz<C>(part_pts + 2 * seg, C::identity()); }
+    if (!wrote1) { part_keys[2 * seg + 1] = last; st_xyzz<C>(part_pts + 2 * seg + 1, C::identity()); }
+  }
+  // an inactive segment that is still in the grid
+  B2Z_HD void close_empty() {
+    part_keys[2 * seg] = kEmptyKey;
+    part_keys[2 * seg + 1] = kEmptyKey;
+  }
+};
+
 // The running sum of the XYZZ finish.  Default: the XYZZ point in registers (G1: 48 words).  The G2 kernel passes its
 // shared-memory sum instead (msm_impl.inc, RunningSum<G2>: 96 words do not fit beside an Fq2 product).
 template <class C>
@@ -195,33 +286,27 @@ struct List {
   B2Z_HD bool same_run(uint32_t j, uint32_t key) const { return refs ? lo + j < rnext : kin[j] == key; }
 };
 
-// One thread's segment [lo, hi) of the sorted references; `cur` = its first bucket (offsets[cur] <= lo <
-// offsets[cur + 1]).  Writes complete runs to bucket_out, cut runs to the two partial slots of `seg`.
-// active = false: a thread without a segment (it only takes part in the warp votes).
+// One thread's segment G of the sorted references: complete runs go to their buckets, cut runs to the partial slots
+// (Segment).  An inactive segment only takes part in the warp votes.
 template <class C, class Acc = RegAcc<C>>
 B2Z_HD void accum_segment(const typename C::Affine* points, const uint32_t* sorted, const uint32_t* offsets,
-                          bool active, uint32_t seg, uint32_t seg_len, uint32_t lo, uint32_t hi, uint32_t total,
-                          uint32_t cur, typename C::Xyzz* bucket_out, uint32_t* part_keys,
-                          typename C::Xyzz* part_pts, uint32_t* maxrun, const Scratch<C>& S,
-                          uint32_t kMinPairs = kMinPairsDefault, uint32_t* acc_ctx = nullptr) {
+                          Segment<C>& G, const Scratch<C>& S, uint32_t kMinPairs = kMinPairsDefault,
+                          uint32_t* acc_ctx = nullptr) {
   using F = typename C::Fld;
   using El = typename C::El;
   using Affine = typename C::Affine;
-  using Xyzz = typename C::Xyzz;
 
   List<C> L;
   L.points = points;
-  L.sorted = sorted + lo;
+  L.sorted = sorted + G.lo;
   L.offsets = offsets;
-  L.lo = lo;
+  L.lo = G.lo;
   L.in = nullptr;
   L.kin = nullptr;
   L.refs = true;
-  const uint32_t first_key = cur;
-  const uint32_t first_next = offsets[cur + 1];
-  L.rc = cur;
-  L.rnext = first_next;
-  uint32_t cnt = active ? hi - lo : 0;
+  L.rc = G.first;
+  L.rnext = G.first_end;
+  uint32_t cnt = G.active ? G.hi - G.lo : 0;
   int out_sel = 0;
 
   // ---- tree rounds
@@ -298,7 +383,7 @@ B2Z_HD void accum_segment(const typename C::Affine* points, const uint32_t* sort
     if (!warp_any(npairs >= kMinPairs)) {
       B2Z_AFF_STAT(4, 1);
       // not worth an inversion: the XYZZ finish takes the CURRENT list; rewind the run cursor
-      if (L.refs) { L.rc = first_key; L.rnext = first_next; }
+      if (L.refs) { L.rc = G.first; L.rnext = G.first_end; }
       break;
     }
     // -- one inversion, then the sums from the last pair to the first
@@ -375,32 +460,15 @@ B2Z_HD void accum_segment(const typename C::Affine* points, const uint32_t* sort
     cnt = o;
     out_sel ^= 1;
   }
-  if (!active) return;
+  if (!G.active) return;
 
   // ---- XYZZ finish over the current list
-  bool wrote0 = false, wrote1 = false;
   uint32_t cur_key = L.key_at(0);
   Acc acc(acc_ctx);
-  auto flush = [&](uint32_t k) {
-    const uint32_t b = offsets[k], e = offsets[k + 1];
-    if (b < lo) {
-      part_keys[2 * seg] = k;
-      acc.store(part_pts + 2 * seg);
-      wrote0 = true;
-    } else if (e > hi) {
-      part_keys[2 * seg + 1] = k;
-      acc.store(part_pts + 2 * seg + 1);
-      wrote1 = true;
-    } else {
-      acc.store(bucket_out + k);
-    }
-    // entries this bucket can have in the partial list: 2 per segment it touches
-    if (b < lo || e > hi) raise_max(maxrun, 2 * ((umin(e, total) - 1) / seg_len - b / seg_len + 1));
-  };
   for (uint32_t i = 0; i < cnt; i++) {
     const uint32_t key = L.key_at(i);
     if (key != cur_key) {
-      flush(cur_key);
+      G.flush_inside(cur_key, offsets[cur_key], acc);
       acc.reset();
       cur_key = key;
     }
@@ -412,9 +480,8 @@ B2Z_HD void accum_segment(const typename C::Affine* points, const uint32_t* sort
     B2Z_AFF_STAT(5, 1);
     acc.madd(q, L.ptr(h), L.negated(h), L.refs);
   }
-  flush(cur_key);
-  if (!wrote0) { part_keys[2 * seg] = first_key; st_xyzz<C>(part_pts + 2 * seg, C::identity()); }
-  if (!wrote1) { part_keys[2 * seg + 1] = cur_key; st_xyzz<C>(part_pts + 2 * seg + 1, C::identity()); }
+  G.flush(cur_key, offsets[cur_key], offsets[cur_key + 1], acc);
+  G.close(cur_key);
 }
 
 }  // namespace aff

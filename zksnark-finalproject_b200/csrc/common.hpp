@@ -169,6 +169,7 @@ struct Ctx {
   cudaStream_t aux[4] = {nullptr, nullptr, nullptr, nullptr};
   std::map<uint32_t, NttDomain> domains;
   bool ntt_attr_set[6] = {false, false, false, false, false, false};
+  bool msm_attr_set[2] = {false, false};   // the G2 accumulation kernels' shared-memory limit: XYZZ, batched-affine
   bool profile = false;
   std::vector<ProfileSpan> spans;
   // pools, so that an enabled profiler costs the launching thread two event records per span and nothing else

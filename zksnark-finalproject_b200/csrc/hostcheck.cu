@@ -63,35 +63,29 @@ int accum_affine_check(const uint32_t* points_raw, const uint32_t* sorted, const
   using Xyzz = typename C::Xyzz;
   using El = typename C::El;
   const Affine* points = reinterpret_cast<const Affine*>(points_raw);
-  const uint32_t total = offsets[nbuckets];
-  uint32_t seg_len = (total + nseg - 1) / nseg;
-  if (seg_len < 8) seg_len = 8;
   std::vector<Xyzz> bucket_out(nbuckets, C::identity()), part_pts(2 * (size_t)nseg, C::identity());
-  std::vector<uint32_t> part_keys(2 * (size_t)nseg, 0xffffffffu);
+  std::vector<uint32_t> part_keys(2 * (size_t)nseg, aff::kEmptyKey);
   uint32_t maxrun = 0;
-  const uint32_t cap = seg_len;
   (void)cap_override;
-  std::vector<Affine> b0(cap + 1), b1(cap + 1);
-  std::vector<uint32_t> k0(cap + 1), k1(cap + 1);
-  std::vector<El> pref(seg_len / 2 + 2);
-  std::vector<uint4> desc(seg_len / 2 + 2);
+  std::vector<Affine> b0, b1;
+  std::vector<uint32_t> k0, k1;
+  std::vector<El> pref;
+  std::vector<uint4> desc;
   for (uint32_t seg = 0; seg < nseg; seg++) {
-    const uint32_t lo = seg * seg_len;
-    if (lo >= total) continue;
-    const uint32_t hi = lo + seg_len < total ? lo + seg_len : total;
-    uint32_t a = 0, z = nbuckets;
-    while (z - a > 1) {
-      const uint32_t mid = (a + z) >> 1;
-      if (offsets[mid] <= lo) a = mid; else z = mid;
+    aff::Segment<C> G(offsets, nbuckets, nseg, seg, bucket_out.data(), part_keys.data(), part_pts.data(), &maxrun);
+    if (!G.active) {
+      G.close_empty();
+      continue;
     }
-    uint32_t cur = a;
-    while (offsets[cur + 1] <= lo) cur++;
+    const uint32_t cap = G.seg_len;
+    b0.resize(cap + 1); b1.resize(cap + 1);
+    k0.resize(cap + 1); k1.resize(cap + 1);
+    pref.resize(cap / 2 + 2); desc.resize(cap / 2 + 2);
     aff::Scratch<C> S;
     S.pts[0] = b0.data(); S.pts[1] = b1.data();
     S.keys[0] = k0.data(); S.keys[1] = k1.data();
     S.pref = pref.data(); S.desc = desc.data();
-    aff::accum_segment<C>(points, sorted, offsets, true, seg, seg_len, lo, hi, total, cur, bucket_out.data(),
-                          part_keys.data(), part_pts.data(), &maxrun, S);
+    aff::accum_segment<C>(points, sorted, offsets, G, S);
   }
   if (rounds_hint) {                       // [0] maxrun, [1..6] the emulation's counters (accum_affine.cuh)
     rounds_hint[0] = maxrun;

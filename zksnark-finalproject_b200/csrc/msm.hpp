@@ -136,6 +136,12 @@ void xyzz_to_affine_device(Ctx* ctx, const typename C::Xyzz* d_in, typename C::A
 // Fr Montgomery -> canonical integers (scalars for the MSM), out-of-place.
 void fr_from_mont_device(Ctx* ctx, const FrEl* in, FrEl* out, size_t n, cudaStream_t st);
 
+// identity flags (one u32 per point, non-zero = identity) -> bitmap words (bit i of word i / 32), n points
+void pack_flags_device(Ctx* ctx, const uint32_t* d_flags, uint32_t n, uint32_t* d_words, cudaStream_t st);
+
+// blocks of `threads` that cover n items
+inline uint32_t nblocks(uint64_t n, uint32_t threads) { return (uint32_t)((n + threads - 1) / threads); }
+
 // out[i] = scalars[i] * G (standard generator), affine; scalars canonical.
 void g1_fixed_base_mul_device(Ctx* ctx, const FrEl* d_scalars, G1::Affine* d_out, uint32_t* d_inf_words, uint32_t n,
                               cudaStream_t st);

@@ -51,19 +51,6 @@ __global__ void permute_bitrev_g1_kernel(const G1::Affine* __restrict__ src, con
   dst_flags[p] = inf ? 1u : 0u;
 }
 
-__global__ void pack_flags_kernel2(const uint32_t* flags, uint32_t n, uint32_t* words) {
-  const uint32_t w = blockIdx.x * blockDim.x + threadIdx.x;
-  if (w >= (n + 31) / 32) return;
-  uint32_t v = 0;
-  for (uint32_t j = 0; j < 32; j++) {
-    const uint32_t i = w * 32 + j;
-    if (i < n && flags[i]) v |= 1u << j;
-  }
-  words[w] = v;
-}
-
-inline uint32_t nblk(uint64_t n, uint32_t t) { return (uint32_t)((n + t - 1) / t); }
-
 constexpr uint32_t kCycBlock = 64;   // variables per block of the block-cyclic point sharding
 
 // local variable j of a block-cyclic shard -> global variable index
@@ -89,12 +76,28 @@ FrEl fr_load_host(const uint64_t v[4]) {
 // ---------------------------------------------------------------------------
 // Proving key
 // ---------------------------------------------------------------------------
+// The five MSMs of a proof, the G1 ones first.  (The partial sums leave in the order A | sA | rB1 | L | H | B,
+// B2Z_PARTIAL_BYTES.)
+enum Sum { SUM_A, SUM_B1, SUM_L, SUM_H, SUM_B, SUM_COUNT };
+
+// Where one MSM of a proof runs and what it leaves.
+struct ProofSum {
+  int slot = 0;                      // MSM scratch arena
+  cudaStream_t stream = nullptr;     // its accumulation (and, but for H, its sort)
+  uint32_t tail = 0;                 // its extra scalars: PkImpl::tail + this (not H)
+  void* d_result = nullptr;          // one XYZZ point (G2 for B)
+  MsmHostPlanes planes;              // its bit-plane sums, for the Horner pass on the host
+  cudaEvent_t accum = nullptr;       // accumulation kernel done (the next sum of the chain waits for it; not H)
+  cudaEvent_t done = nullptr;        // planes copied to the host (not H: prove_end synchronises its stream)
+  cudaEvent_t sorted = nullptr;      // L only: sort done (the G2 accumulation waits for it)
+  template <class C> typename C::Xyzz* result() const { return static_cast<typename C::Xyzz*>(d_result); }
+};
+
 struct PkImpl {
   // A key handle holds per-proof scratch (below), so it belongs to exactly ONE context: the one it was
   // uploaded through.  Every entry point checks this and returns B2Z_EINVAL for a foreign context.
   const Ctx* owner = nullptr;
   bool* assignment_flag = nullptr;   // b2z_groth16_shard_begin .. shard_finish window (r1cs.cu)
-  cudaStream_t h_stream = nullptr;   // where the H accumulation of the proof in flight runs
   uint32_t log_n = 0;
   uint64_t m = 0, l = 0;
   // shard: `ma` variables of the a/b queries -- either the contiguous range [lo, lo+ma) (cyc_world == 0) or,
@@ -111,26 +114,21 @@ struct PkImpl {
   MsmBases<G2> g2;             // [b_g2     | beta_2  delta_2]
   // per-proof device scratch
   DevBuf<FrEl> ea, eb, ec, z, zc, hc, tail;
-  DevBuf<G1::Xyzz> g1_out;     // 0 A, 3 L, 4 H, 5 B1 (1, 2 unused: s*A and r*B1 are made on the host)
-  DevBuf<G2::Xyzz> g2_out;     // B
+  DevBuf<G1::Xyzz> g1_out;     // results of the G1 sums, indexed by Sum (s*A and r*B1 are made on the host)
+  DevBuf<G2::Xyzz> g2_out;     // result of B
   uint32_t* h_out = nullptr;   // pinned: B2Z_PARTIAL_BYTES
   uint32_t* h_planes = nullptr;   // pinned: bit-plane sums of the five MSMs (host-side Horner, msm.hpp)
-  MsmHostPlanes hp[5];            // 0 A, 1 B (G2), 2 B1, 3 L, 4 H
+  ProofSum sums[SUM_COUNT];
   FrEl r_c, s_c;                  // the proof's r, s as canonical integers (prove_begin -> prove_end)
-  cudaEvent_t ev_z = nullptr, ev_done[4] = {nullptr, nullptr, nullptr, nullptr};
-  cudaEvent_t ev_sorted[4] = {nullptr, nullptr, nullptr, nullptr};
-  cudaEvent_t ev_accum[4] = {nullptr, nullptr, nullptr, nullptr};
+  cudaEvent_t ev_z = nullptr;
   cudaEvent_t ev_wm = nullptr;       // witness-map transforms of the proof in flight are done (gates the first accumulation)
   ~PkImpl() {
     if (h_out) cudaFreeHost(h_out);
     if (h_planes) cudaFreeHost(h_planes);
     if (ev_z) cudaEventDestroy(ev_z);
-    for (auto& e : ev_done)
-      if (e) cudaEventDestroy(e);
-    for (auto& e : ev_sorted)
-      if (e) cudaEventDestroy(e);
-    for (auto& e : ev_accum)
-      if (e) cudaEventDestroy(e);
+    for (ProofSum& S : sums)
+      for (cudaEvent_t e : {S.accum, S.done, S.sorted})
+        if (e) cudaEventDestroy(e);
     if (ev_wm) cudaEventDestroy(ev_wm);
   }
 };
@@ -254,7 +252,7 @@ static_assert(kPartialBytes == B2Z_PARTIAL_BYTES, "header constant out of sync")
 // prove_begin and prove_quotient while the z-only accumulations are already running.
 void prove_accums(Ctx& c, PkImpl& pk, cudaEvent_t gate = nullptr);
 void prove_begin(Ctx& c, PkImpl& pk, const FrEl* d_z, const uint64_t r[4], const uint64_t s[4], bool with_accums = true) {
-  cudaStream_t sA = c.aux[0], sB = c.aux[1], sB1 = c.aux[2], sL = c.aux[3];
+  ProofSum &A = pk.sums[SUM_A], &B1 = pk.sums[SUM_B1], &B = pk.sums[SUM_B], &L = pk.sums[SUM_L];
   // host-side scalars: r, s, -(r s) as canonical integers
   const FrEl r_m = Fr::reduce(fr_load_host(r)), s_m = Fr::reduce(fr_load_host(s));
   pk.r_c = Fr::from_mont(r_m);
@@ -263,28 +261,26 @@ void prove_begin(Ctx& c, PkImpl& pk, const FrEl* d_z, const uint64_t r[4], const
   FrEl one_c = Fr::zero();
   one_c.l[0] = 1;
   const FrEl tail_h[5] = {one_c, pk.r_c, one_c, pk.s_c, neg_rs};      // A: {1, r}; B1, B: {1, s}; L: {-rs}
-  B2Z_CUDA(cudaMemcpyAsync(pk.tail.p, tail_h, sizeof(tail_h), cudaMemcpyHostToDevice, sA));
+  B2Z_CUDA(cudaMemcpyAsync(pk.tail.p, tail_h, sizeof(tail_h), cudaMemcpyHostToDevice, A.stream));
   // this shard's variables of z as canonical integers
   if (pk.cyc_world == 0) {
-    fr_from_mont_device(&c, d_z + pk.lo, pk.zc.p, pk.ma, sA);
+    fr_from_mont_device(&c, d_z + pk.lo, pk.zc.p, pk.ma, A.stream);
   } else if (pk.ma) {
-    fr_from_mont_cyclic_kernel<<<nblk(pk.ma, 256), 256, 0, sA>>>(d_z, pk.zc.p, pk.ma, pk.cyc_rank, pk.cyc_world);
+    fr_from_mont_cyclic_kernel<<<nblocks(pk.ma, 256), 256, 0, A.stream>>>(d_z, pk.zc.p, pk.ma, pk.cyc_rank,
+                                                                          pk.cyc_world);
     B2Z_LAUNCHED(&c);
   }
-  B2Z_CUDA(cudaEventRecord(pk.ev_z, sA));
+  B2Z_CUDA(cudaEventRecord(pk.ev_z, A.stream));
   const FrEl* z_l = pk.zc.p + pk.l_skip;
   // ---- the four z-only sorts, concurrently
-  msm_sort<G1>(&c, 1, pk.a_set, pk.zc.p, pk.ma, pk.tail.p + 0, sA);
-  B2Z_CUDA(cudaEventRecord(pk.ev_sorted[0], sA));
-  B2Z_CUDA(cudaStreamWaitEvent(sB, pk.ev_z, 0));
-  msm_sort<G2>(&c, 2, pk.g2, pk.zc.p, pk.ma, pk.tail.p + 2, sB);
-  B2Z_CUDA(cudaEventRecord(pk.ev_sorted[1], sB));
-  B2Z_CUDA(cudaStreamWaitEvent(sB1, pk.ev_z, 0));
-  msm_sort<G1>(&c, 3, pk.b1_set, pk.zc.p, pk.ma, pk.tail.p + 2, sB1);
-  B2Z_CUDA(cudaEventRecord(pk.ev_sorted[2], sB1));
-  B2Z_CUDA(cudaStreamWaitEvent(sL, pk.ev_z, 0));
-  msm_sort<G1>(&c, 4, pk.l_set, z_l, pk.ml, pk.tail.p + 4, sL);
-  B2Z_CUDA(cudaEventRecord(pk.ev_sorted[3], sL));
+  msm_sort<G1>(&c, A.slot, pk.a_set, pk.zc.p, pk.ma, pk.tail.p + A.tail, A.stream);
+  B2Z_CUDA(cudaStreamWaitEvent(B.stream, pk.ev_z, 0));
+  msm_sort<G2>(&c, B.slot, pk.g2, pk.zc.p, pk.ma, pk.tail.p + B.tail, B.stream);
+  B2Z_CUDA(cudaStreamWaitEvent(B1.stream, pk.ev_z, 0));
+  msm_sort<G1>(&c, B1.slot, pk.b1_set, pk.zc.p, pk.ma, pk.tail.p + B1.tail, B1.stream);
+  B2Z_CUDA(cudaStreamWaitEvent(L.stream, pk.ev_z, 0));
+  msm_sort<G1>(&c, L.slot, pk.l_set, z_l, pk.ml, pk.tail.p + L.tail, L.stream);
+  B2Z_CUDA(cudaEventRecord(L.sorted, L.stream));
   if (with_accums) prove_accums(c, pk);
 }
 
@@ -294,8 +290,7 @@ void prove_begin(Ctx& c, PkImpl& pk, const FrEl* d_z, const uint64_t r[4], const
 // phase -- sorts (latency / atomics bound) next to row evaluation and transforms (integer-pipe bound) -- overlaps
 // well instead, and the accumulations then run back to back with the H sort hidden under them.
 void prove_accums(Ctx& c, PkImpl& pk, cudaEvent_t gate) {
-  cudaStream_t sA = c.aux[0], sB = c.aux[1], sB1 = c.aux[2], sL = c.aux[3];
-  G1::Xyzz* g1o = pk.g1_out.p;
+  ProofSum &A = pk.sums[SUM_A], &B1 = pk.sums[SUM_B1], &B = pk.sums[SUM_B], &L = pk.sums[SUM_L];
   // ---- accumulations chained by events (order below).  Each accumulation kernel is sized to fill the GPU by
   // itself; the G2 one (255 registers) leaves room for nothing, a G1 one leaves room on every SM for sort /
   // transform / tail blocks (the tail kernels are register-capped for exactly that), so tails overlap the next sums.
@@ -308,60 +303,61 @@ void prove_accums(Ctx& c, PkImpl& pk, cudaEvent_t gate) {
   // kernels' latencies (Fibonacci: 5 variables; an eighth of the 16x16 matrix circuit) -- those run concurrently.
   auto big = [](uint64_t n, uint32_t windows) { return n * windows >= (1u << 18); };
   const bool chain = big(pk.g2.n, pk.g2.windows) || big(pk.a_set.n, pk.a_set.windows);
+  auto after = [chain](const ProofSum& prev) { return chain ? prev.accum : nullptr; };
   // Order A -> B1 -> B (G2) -> L (-> H).  Two G1 sums open the chain because a G1 accumulation leaves a quarter of
   // every SM's registers free: the sorts of the other z-only MSMs (atomics-bound, starved while the transforms ran)
   // finish BESIDE them instead of in front of the G2 accumulation, which takes every register of every SM.  The
   // streams' priorities (api.cu) make the sorts finish in the order their sums need them.
-  if (gate) B2Z_CUDA(cudaStreamWaitEvent(sA, gate, 0));
-  msm_finish<G1>(&c, 1, pk.a_set, g1o + 0, sA, nullptr, pk.ev_accum[0], &pk.hp[0]);
-  B2Z_CUDA(cudaEventRecord(pk.ev_done[0], sA));
+  if (gate) B2Z_CUDA(cudaStreamWaitEvent(A.stream, gate, 0));
+  msm_finish<G1>(&c, A.slot, pk.a_set, A.result<G1>(), A.stream, nullptr, A.accum, &A.planes);
+  B2Z_CUDA(cudaEventRecord(A.done, A.stream));
   if (!chain && gate) {
-    B2Z_CUDA(cudaStreamWaitEvent(sB1, gate, 0));
-    B2Z_CUDA(cudaStreamWaitEvent(sB, gate, 0));
+    B2Z_CUDA(cudaStreamWaitEvent(B1.stream, gate, 0));
+    B2Z_CUDA(cudaStreamWaitEvent(B.stream, gate, 0));
   }
-  msm_finish<G1>(&c, 3, pk.b1_set, g1o + 5, sB1, chain ? pk.ev_accum[0] : nullptr, pk.ev_accum[1], &pk.hp[2]);
-  B2Z_CUDA(cudaEventRecord(pk.ev_done[2], sB1));
-  if (chain) B2Z_CUDA(cudaStreamWaitEvent(sB, pk.ev_sorted[3], 0));     // nothing runs beside the G2 sum: L's sort first
-  msm_finish<G2>(&c, 2, pk.g2, pk.g2_out.p, sB, chain ? pk.ev_accum[1] : nullptr, pk.ev_accum[3], &pk.hp[1]);
-  B2Z_CUDA(cudaEventRecord(pk.ev_done[1], sB));
-  msm_finish<G1>(&c, 4, pk.l_set, g1o + 3, sL, chain ? pk.ev_accum[3] : nullptr, pk.ev_accum[2], &pk.hp[3]);
-  B2Z_CUDA(cudaEventRecord(pk.ev_done[3], sL));
+  msm_finish<G1>(&c, B1.slot, pk.b1_set, B1.result<G1>(), B1.stream, after(A), B1.accum, &B1.planes);
+  B2Z_CUDA(cudaEventRecord(B1.done, B1.stream));
+  if (chain) B2Z_CUDA(cudaStreamWaitEvent(B.stream, L.sorted, 0));     // nothing runs beside the G2 sum: L's sort first
+  msm_finish<G2>(&c, B.slot, pk.g2, B.result<G2>(), B.stream, after(B1), B.accum, &B.planes);
+  B2Z_CUDA(cudaEventRecord(B.done, B.stream));
+  msm_finish<G1>(&c, L.slot, pk.l_set, L.result<G1>(), L.stream, after(B), L.accum, &L.planes);
+  B2Z_CUDA(cudaEventRecord(L.done, L.stream));
 }
 
 // d_a, d_b, d_c: evaluations of the three QAP combinations on the coset g H (d_a is clobbered)
 void prove_h_finish(Ctx& c, PkImpl& pk, cudaStream_t st = nullptr) {
   const bool chain = (uint64_t)pk.h.n * pk.h.windows >= (1u << 18);
-  pk.h_stream = st ? st : c.stream;
-  msm_finish<G1>(&c, 0, pk.h, pk.g1_out.p + 4, pk.h_stream, chain ? pk.ev_accum[2] : nullptr, nullptr, &pk.hp[4]);
+  ProofSum& H = pk.sums[SUM_H];
+  H.stream = st ? st : c.stream;
+  msm_finish<G1>(&c, H.slot, pk.h, H.result<G1>(), H.stream, chain ? pk.sums[SUM_L].accum : nullptr, nullptr,
+                 &H.planes);
 }
 void prove_quotient(Ctx& c, PkImpl& pk, FrEl* d_a, const FrEl* d_b, const FrEl* d_c, bool with_h_finish = true) {
   cudaStream_t st = c.stream;
   witness_map_quotient(&c, d_a, d_b, d_c, pk.log_n, /*natural_out=*/false, st);    // whole domain, every shard
   B2Z_CUDA(cudaEventRecord(pk.ev_wm, st));
   fr_from_mont_device(&c, d_a + pk.h_lo, pk.hc.p, pk.hn, st);
-  msm_sort<G1>(&c, 0, pk.h, pk.hc.p, pk.hn, nullptr, st);
+  msm_sort<G1>(&c, pk.sums[SUM_H].slot, pk.h, pk.hc.p, pk.hn, nullptr, st);
   if (with_h_finish) prove_h_finish(c, pk);
 }
 
 void prove_end(Ctx& c, PkImpl& pk, uint8_t* partial_out) {
-  auto g1_result = [&](int i) {
-    return host::g1_planes_horner(static_cast<const uint32_t*>(pk.hp[i].host), pk.hp[i].nplanes, kMsmChunkLog);
-  };
+  auto planes = [&](Sum k) { return static_cast<const uint32_t*>(pk.sums[k].planes.host); };
+  auto g1_result = [&](Sum k) { return host::g1_planes_horner(planes(k), pk.sums[k].planes.nplanes, kMsmChunkLog); };
   // A, s*A, B1, r*B1 while the GPU works on L and H
-  B2Z_CUDA(cudaEventSynchronize(pk.ev_done[0]));
-  const host::G1Xyzz A = g1_result(0);
+  B2Z_CUDA(cudaEventSynchronize(pk.sums[SUM_A].done));
+  const host::G1Xyzz A = g1_result(SUM_A);
   host::g1_to_device_layout(A, pk.h_out + 0 * kG1Bytes / 4);
   host::g1_to_device_layout(host::g1_mul_scalar(A, pk.s_c.l), pk.h_out + 1 * kG1Bytes / 4);
-  B2Z_CUDA(cudaEventSynchronize(pk.ev_done[2]));
-  host::g1_to_device_layout(host::g1_mul_scalar(g1_result(2), pk.r_c.l), pk.h_out + 2 * kG1Bytes / 4);
-  B2Z_CUDA(cudaEventSynchronize(pk.ev_done[1]));
-  host::g2_to_device_layout(
-      host::g2_planes_horner(static_cast<const uint32_t*>(pk.hp[1].host), pk.hp[1].nplanes, kMsmChunkLog),
-      pk.h_out + 5 * kG1Bytes / 4);
-  B2Z_CUDA(cudaEventSynchronize(pk.ev_done[3]));
-  host::g1_to_device_layout(g1_result(3), pk.h_out + 3 * kG1Bytes / 4);
-  B2Z_CUDA(cudaStreamSynchronize(pk.h_stream ? pk.h_stream : c.stream));
-  host::g1_to_device_layout(g1_result(4), pk.h_out + 4 * kG1Bytes / 4);
+  B2Z_CUDA(cudaEventSynchronize(pk.sums[SUM_B1].done));
+  host::g1_to_device_layout(host::g1_mul_scalar(g1_result(SUM_B1), pk.r_c.l), pk.h_out + 2 * kG1Bytes / 4);
+  B2Z_CUDA(cudaEventSynchronize(pk.sums[SUM_B].done));
+  host::g2_to_device_layout(host::g2_planes_horner(planes(SUM_B), pk.sums[SUM_B].planes.nplanes, kMsmChunkLog),
+                            pk.h_out + 5 * kG1Bytes / 4);
+  B2Z_CUDA(cudaEventSynchronize(pk.sums[SUM_L].done));
+  host::g1_to_device_layout(g1_result(SUM_L), pk.h_out + 3 * kG1Bytes / 4);
+  B2Z_CUDA(cudaStreamSynchronize(pk.sums[SUM_H].stream));
+  host::g1_to_device_layout(g1_result(SUM_H), pk.h_out + 4 * kG1Bytes / 4);
   std::memcpy(partial_out, pk.h_out, kPartialBytes);
 }
 
@@ -451,7 +447,7 @@ uint32_t pk_h_chunk(const b2z_pk* pk, uint32_t* h_lo) {
 void prove_dist_h_sort_on(Ctx& c, const b2z_pk* pk, const FrEl* d_h, cudaStream_t st) {
   PkImpl& P = pk_of(c, pk, "b2z_dist_prove");
   fr_from_mont_device(&c, d_h, P.hc.p, P.hn, st);
-  msm_sort<G1>(&c, 0, P.h, P.hc.p, P.hn, nullptr, st);
+  msm_sort<G1>(&c, P.sums[SUM_H].slot, P.h, P.hc.p, P.hn, nullptr, st);
 }
 // all five accumulations, chained: the first once `wm_done` has fired (the witness map's transform kernels need the
 // SMs the accumulations would fill), H on `h_st` -- the stream its sort was queued on, which therefore hides under
@@ -630,25 +626,40 @@ static b2z_status pk_upload_impl(b2z_ctx* ctx, const b2z_pk_desc* d, uint32_t fr
         src_inf.alloc(hw.size());
         B2Z_CUDA(cudaMemcpyAsync(src_inf.p, hw.data(), hw.size() * 4, cudaMemcpyHostToDevice, st));
       }
-      permute_bitrev_g1_kernel<<<nblk(n, 256), 256, 0, st>>>(src.p, src_inf.p, (uint32_t)(n - 1), P.log_n, dst.p,
-                                                             flags.p);
+      permute_bitrev_g1_kernel<<<nblocks(n, 256), 256, 0, st>>>(src.p, src_inf.p, (uint32_t)(n - 1), P.log_n, dst.p,
+                                                                flags.p);
       B2Z_LAUNCHED(&c);
-      pack_flags_kernel2<<<nblk((P.hn + 31) / 32 + 1, 128), 128, 0, st>>>(flags.p + h_lo, P.hn, words.p);
-      B2Z_LAUNCHED(&c);
+      pack_flags_device(&c, flags.p + h_lo, P.hn, words.p, st);
       msm_bases_build<G1>(&c, P.h, dst.p + h_lo, words.p, P.hn, pre, 0, st);
       B2Z_CUDA(cudaStreamSynchronize(st));
     }
     P.ea.alloc(n); P.eb.alloc(n); P.ec.alloc(n); P.hc.alloc(P.hn ? P.hn : 1);
     P.z.alloc(m); P.zc.alloc(P.ma ? P.ma : 1); P.tail.alloc(5);
-    P.g1_out.alloc(6); P.g2_out.alloc(1);
+    P.g1_out.alloc(SUM_B); P.g2_out.alloc(1);
     B2Z_CUDA(cudaMallocHost(&P.h_out, kPartialBytes));
-    B2Z_CUDA(cudaMallocHost(&P.h_planes, 5 * kPlaneSlotBytes));
-    for (int i = 0; i < 5; i++) P.hp[i].host = P.h_planes + (size_t)i * kPlaneSlotBytes / 4;
-    B2Z_CUDA(cudaEventCreateWithFlags(&P.ev_z, cudaEventDisableTiming));
-    for (auto& e : P.ev_done) B2Z_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    for (auto& e : P.ev_sorted) B2Z_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    for (auto& e : P.ev_accum) B2Z_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    B2Z_CUDA(cudaEventCreateWithFlags(&P.ev_wm, cudaEventDisableTiming));
+    B2Z_CUDA(cudaMallocHost(&P.h_planes, SUM_COUNT * kPlaneSlotBytes));
+    auto new_event = [](cudaEvent_t* e) { B2Z_CUDA(cudaEventCreateWithFlags(e, cudaEventDisableTiming)); };
+    auto init = [&](Sum k, int slot, cudaStream_t stream, uint32_t tail, void* d_result) {
+      ProofSum& S = P.sums[k];
+      S.slot = slot;
+      S.stream = stream;
+      S.tail = tail;
+      S.d_result = d_result;
+      S.planes.host = P.h_planes + (size_t)k * kPlaneSlotBytes / 4;
+      if (k != SUM_H) {
+        new_event(&S.accum);
+        new_event(&S.done);
+      }
+    };
+    // arena slot, stream (H: the one prove_h_finish names), offset of the tail scalars in {1, r, 1, s, -rs}, result
+    init(SUM_A, 1, c.aux[0], 0, P.g1_out.p + SUM_A);
+    init(SUM_B1, 3, c.aux[2], 2, P.g1_out.p + SUM_B1);
+    init(SUM_L, 4, c.aux[3], 4, P.g1_out.p + SUM_L);
+    init(SUM_H, 0, c.stream, 0, P.g1_out.p + SUM_H);
+    init(SUM_B, 2, c.aux[1], 2, P.g2_out.p);
+    new_event(&P.sums[SUM_L].sorted);
+    new_event(&P.ev_z);
+    new_event(&P.ev_wm);
     *out = pk.release();
   });
 }

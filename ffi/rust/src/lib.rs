@@ -8,6 +8,7 @@
 //! | `Radix2EvaluationDomain::{fft,ifft}_in_place`, `get_coset`                                | [`ntt_in_place`] |
 //! | `prepare_verifying_key` + `serialize_compressed` (matrix_proof.rs:134-136, io.rs:62-68)    | [`prepared_vk_bytes`] |
 //! | `Groth16::verify_with_processed_vk` (matrix_proof.rs:199-206)                              | [`verify_with_processed_vk`] |
+//! | `Groth16::<Bls12_381>::setup` (matrix_proof.rs:128-131, fibbonaci_handler.rs:107)          | [`DeviceKey::setup`] |
 //!
 //! SOURCE ONLY -- never compiled in the build image (no Rust toolchain there).  arkworks' `Fp` / `Affine` are
 //! `repr(Rust)`: limbs are copied explicitly (`x.0 .0`), never transmuted.  Field elements cross in Montgomery form
@@ -44,6 +45,16 @@ pub mod sys {
         pub beta_g2: *const u64, pub delta_g2: *const u64,
     }
     #[repr(C)]
+    pub struct b2z_setup_desc {
+        pub alpha: *const u64, pub beta: *const u64, pub gamma: *const u64, pub delta: *const u64, pub tau: *const u64,
+        pub g1_generator: *const u64, pub g2_generator: *const u64,
+    }
+    #[repr(C)]
+    pub struct b2z_vk_out {
+        pub alpha_g1: [u64; 12], pub beta_g2: [u64; 24], pub gamma_g2: [u64; 24], pub delta_g2: [u64; 24],
+        pub gamma_abc_g1: *mut u64, pub gamma_abc_inf: *mut u8,
+    }
+    #[repr(C)]
     pub struct b2z_vk_desc {
         pub num_instance: u64,
         pub alpha_g1: *const u64, pub beta_g2: *const u64, pub gamma_g2: *const u64, pub delta_g2: *const u64,
@@ -56,6 +67,8 @@ pub mod sys {
     extern "C" {
         pub fn b2z_ctx_create(device_id: i32, out: *mut *mut b2z_ctx) -> i32;
         pub fn b2z_ctx_destroy(ctx: *mut b2z_ctx);
+        pub fn b2z_groth16_setup(ctx: *mut b2z_ctx, r1cs: *mut b2z_r1cs, desc: *const b2z_setup_desc,
+                                 pk_out: *mut *mut b2z_pk, vk_out: *mut b2z_vk_out) -> i32;
         pub fn b2z_last_error(ctx: *const b2z_ctx) -> *const c_char;
         pub fn b2z_ntt_fr(ctx: *mut b2z_ctx, data: *mut u64, log_n: u32, inverse: i32, coset_gen: *const u64) -> i32;
         pub fn b2z_witness_map(ctx: *mut b2z_ctx, a: *const u64, b: *const u64, c: *const u64, log_n: u32, h: *mut u64) -> i32;
@@ -199,6 +212,56 @@ impl<'c> DeviceKey<'c> {
         status(ctx.raw, unsafe { b2z_pk_upload(ctx.raw, &desc, &mut raw) })?;
         Ok(Self { ctx, raw })
     }
+}
+impl<'c> DeviceKey<'c> {
+    /// `Groth16::<Bls12_381>::setup(circuit, rng)` after synthesis, with the key made on the GPU (b2z_groth16_setup):
+    /// the draws are arkworks' own, in its order (alpha, beta, gamma, delta, g1, g2, tau), so the key and the
+    /// verifying key equal what `Groth16::setup` returns for the same rng.  `m`: the circuit's matrices on `ctx`.
+    pub fn setup<R: RngCore>(ctx: &'c Context, m: &DeviceMatrices<'c>, num_constraints: usize, num_instance: usize,
+                             rng: &mut R) -> Result<(Self, VerifyingKey<Bls12_381>), SynthesisError> {
+        let domain = ark_poly::Radix2EvaluationDomain::<Fr>::new(num_constraints + num_instance)
+            .ok_or(SynthesisError::PolynomialDegreeTooLarge)?;
+        let (alpha, beta, gamma, delta) = (Fr::rand(rng), Fr::rand(rng), Fr::rand(rng), Fr::rand(rng));
+        let g1 = G1Projective::rand(rng);
+        let g2 = G2Projective::rand(rng);
+        let tau = loop {
+            let t = Fr::rand(rng);
+            if !domain.evaluate_vanishing_polynomial(t).is_zero() { break t; }
+        };
+        let (g1a, g2a): (G1Affine, G2Affine) = (g1.into(), g2.into());
+        let (g1l, g2l) = (pack_g1(&[g1a]).0, pack_g2(&[g2a]).0);
+        let els = pack_fr(&[alpha, beta, gamma, delta, tau]);
+        let desc = b2z_setup_desc {
+            alpha: els[0..].as_ptr(), beta: els[4..].as_ptr(), gamma: els[8..].as_ptr(), delta: els[12..].as_ptr(),
+            tau: els[16..].as_ptr(), g1_generator: g1l.as_ptr(), g2_generator: g2l.as_ptr(),
+        };
+        let mut gabc = vec![0u64; num_instance * 12];
+        let mut gabc_inf = vec![0u8; (num_instance + 7) / 8];
+        let mut vk = b2z_vk_out {
+            alpha_g1: [0; 12], beta_g2: [0; 24], gamma_g2: [0; 24], delta_g2: [0; 24],
+            gamma_abc_g1: gabc.as_mut_ptr(), gamma_abc_inf: gabc_inf.as_mut_ptr(),
+        };
+        let mut raw = ptr::null_mut();
+        status(ctx.raw, unsafe { b2z_groth16_setup(ctx.raw, m.raw, &desc, &mut raw, &mut vk) })?;
+        let g1_of = |l: &[u64], inf: bool| -> G1Affine {
+            if inf { return G1Affine::identity(); }
+            G1Affine::new_unchecked(unpack_fq(&l[0..6]), unpack_fq(&l[6..12]))
+        };
+        let g2_of = |l: &[u64]| -> G2Affine {
+            let f2 = |a: &[u64]| ark_bls12_381::Fq2::new(unpack_fq(&a[0..6]), unpack_fq(&a[6..12]));
+            G2Affine::new_unchecked(f2(&l[0..12]), f2(&l[12..24]))
+        };
+        let vk = VerifyingKey {
+            alpha_g1: g1_of(&vk.alpha_g1, false), beta_g2: g2_of(&vk.beta_g2), gamma_g2: g2_of(&vk.gamma_g2),
+            delta_g2: g2_of(&vk.delta_g2),
+            gamma_abc_g1: (0..num_instance).map(|i| g1_of(&gabc[i * 12..i * 12 + 12], (gabc_inf[i >> 3] >> (i & 7)) & 1 == 1))
+                .collect(),
+        };
+        Ok((Self { ctx, raw }, vk))
+    }
+}
+fn unpack_fq(l: &[u64]) -> ark_bls12_381::Fq {
+    ark_ff::Fp(BigInt([l[0], l[1], l[2], l[3], l[4], l[5]]), core::marker::PhantomData)
 }
 impl Drop for DeviceKey<'_> { fn drop(&mut self) { unsafe { b2z_pk_free(self.ctx.raw, self.raw) } } }
 

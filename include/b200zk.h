@@ -203,6 +203,45 @@ B2Z_API b2z_status b2z_fixed_base_mul_g1(b2z_ctx* ctx, const uint64_t* scalars, 
 B2Z_API b2z_status b2z_fixed_base_mul_g2(b2z_ctx* ctx, const uint64_t* scalars, uint64_t n,
                                          uint64_t* out_points, uint8_t* out_inf);
 
+/* ---- ark_groth16::generator::generate_parameters_with_qap::<LibsnarkReduction> on the device --------------------
+ * Groth16::setup (matrix_proof.rs:128-131, fibbonaci_handler.rs:107, prime_snark.rs:111-115) after its random draws:
+ * the caller passes the toxic waste and the generators (ark draws alpha, beta, gamma, delta, then g1, g2, then tau).
+ * The matrices are those of b2z_r1cs_upload (same context).  Lagrange coefficients at tau, the QAP evaluation, the
+ * scalars and every fixed-base multiplication run on the GPU; the key is assembled in device memory and returned
+ * as a handle equal to what b2z_pk_upload makes from the same arrays (ready for b2z_groth16_prove / _prove_r1cs).
+ * Every input is checked on the host before any GPU work; B2Z_EINVAL with a message for: an element >= r, gamma or
+ * delta = 0, tau in the domain (tau^n = 1), a generator that is the identity, off the curve or outside the r-order
+ * subgroup, an r1cs of another context.  Size limits: those of b2z_pk_upload.                                     */
+typedef struct b2z_setup_desc {
+  const uint64_t* alpha; const uint64_t* beta; const uint64_t* gamma; const uint64_t* delta; const uint64_t* tau;
+                                   /* Fr, Montgomery limbs, each < r; gamma, delta != 0; tau^n != 1 */
+  const uint64_t* g1_generator;    /* affine, 12 limbs; NULL = the standard generator */
+  const uint64_t* g2_generator;    /* affine, 24 limbs; NULL = the standard generator */
+} b2z_setup_desc;
+typedef struct b2z_vk_out {        /* filled by the call */
+  uint64_t alpha_g1[12], beta_g2[24], gamma_g2[24], delta_g2[24];
+  uint64_t* gamma_abc_g1;          /* caller-allocated, num_instance x 12 */
+  uint8_t*  gamma_abc_inf;         /* caller-allocated, (num_instance + 7) / 8 */
+} b2z_vk_out;
+B2Z_API b2z_status b2z_groth16_setup(b2z_ctx* ctx, b2z_r1cs* r1cs, const b2z_setup_desc* desc,
+                                     b2z_pk** pk_out, b2z_vk_out* vk_out);
+/* A whole key (b2z_pk_upload or b2z_groth16_setup) back in the b2z_pk_desc layout: h_query in natural order, n - 1
+ * points.  The arrays are caller-allocated with b2z_pk_desc's sizes (h: NULL when n = 1, l: NULL when m = l); the
+ * counts and the five single points are filled by the call.  A shard returns B2Z_EINVAL.  For callers that persist a
+ * key, or shard one with b2z_pk_upload_shard.                                                                       */
+typedef struct b2z_pk_arrays {
+  uint64_t num_variables;
+  uint64_t num_instance;
+  uint32_t log_domain;
+  uint64_t* a_query;   uint8_t* a_inf;
+  uint64_t* b_g1_query; uint8_t* b_g1_inf;
+  uint64_t* b_g2_query; uint8_t* b_g2_inf;
+  uint64_t* h_query;   uint8_t* h_inf;
+  uint64_t* l_query;   uint8_t* l_inf;
+  uint64_t alpha_g1[12], beta_g1[12], delta_g1[12], beta_g2[24], delta_g2[24];
+} b2z_pk_arrays;
+B2Z_API b2z_status b2z_pk_download(b2z_ctx* ctx, const b2z_pk* pk, b2z_pk_arrays* out);
+
 /* ---- ark_groth16 verifier over the reference's wire formats (host only: no GPU, no ctx) -----------------
  * b2z_groth16_prepare_verifying_key = ark_groth16::prepare_verifying_key followed by
  * PreparedVerifyingKey::serialize_compressed -- the bytes encode_pvk base64-encodes

@@ -32,6 +32,27 @@ class VkDesc(ctypes.Structure):
                 ("delta_g2", vp), ("gamma_abc_g1", vp), ("gamma_abc_inf", vp)]
 
 
+class SetupDesc(ctypes.Structure):
+    _fields_ = [("alpha", vp), ("beta", vp), ("gamma", vp), ("delta", vp), ("tau", vp),
+                ("g1_generator", vp), ("g2_generator", vp)]
+
+
+class VkOut(ctypes.Structure):
+    _fields_ = [("alpha_g1", ctypes.c_uint64 * 12), ("beta_g2", ctypes.c_uint64 * 24), ("gamma_g2", ctypes.c_uint64 * 24),
+                ("delta_g2", ctypes.c_uint64 * 24), ("gamma_abc_g1", vp), ("gamma_abc_inf", vp)]
+
+
+class PkArrays(ctypes.Structure):
+    _fields_ = [
+        ("num_variables", ctypes.c_uint64), ("num_instance", ctypes.c_uint64), ("log_domain", ctypes.c_uint32),
+        ("a_query", vp), ("a_inf", vp), ("b_g1_query", vp), ("b_g1_inf", vp),
+        ("b_g2_query", vp), ("b_g2_inf", vp), ("h_query", vp), ("h_inf", vp),
+        ("l_query", vp), ("l_inf", vp),
+        ("alpha_g1", ctypes.c_uint64 * 12), ("beta_g1", ctypes.c_uint64 * 12), ("delta_g1", ctypes.c_uint64 * 12),
+        ("beta_g2", ctypes.c_uint64 * 24), ("delta_g2", ctypes.c_uint64 * 24),
+    ]
+
+
 class PoseidonDesc(ctypes.Structure):
     _fields_ = [("full_rounds", ctypes.c_uint32), ("partial_rounds", ctypes.c_uint32), ("alpha", ctypes.c_uint64),
                 ("width", ctypes.c_uint32), ("rate", ctypes.c_uint32), ("capacity", ctypes.c_uint32),
@@ -71,6 +92,8 @@ SIGNATURES = {
     "b2z_groth16_prove_device": (ctypes.c_int32, [vp, vp, vp, vp, vp, vp, vp, vp, vp]),
     "b2z_fixed_base_mul_g1": (ctypes.c_int32, [vp, vp, ctypes.c_uint64, vp, vp]),
     "b2z_fixed_base_mul_g2": (ctypes.c_int32, [vp, vp, ctypes.c_uint64, vp, vp]),
+    "b2z_groth16_setup": (ctypes.c_int32, [vp, vp, ctypes.POINTER(SetupDesc), ctypes.POINTER(vp), ctypes.POINTER(VkOut)]),
+    "b2z_pk_download": (ctypes.c_int32, [vp, vp, ctypes.POINTER(PkArrays)]),
     "b2z_profile_enable": (ctypes.c_int32, [vp, ctypes.c_int]),
     "b2z_profile_read": (ctypes.c_int32, [vp, vp, vp, vp, ctypes.c_int]),
     "b2z_profile_spans": (ctypes.c_int, [vp, ctypes.c_int, vp, vp, vp]),

@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 BUILD = os.path.join(CSRC, "_build")
 LIB = os.path.join(HERE, "libb200zk.so")
-SOURCES = ["api.cu", "ntt.cu", "msm_g1.cu", "msm_g2.cu", "prove.cu", "r1cs.cu", "hostcheck.cu", "verify.cu", "witness.cu", "setup_host.cu"]
+SOURCES = ["api.cu", "ntt.cu", "msm_g1.cu", "msm_g2.cu", "prove.cu", "r1cs.cu", "hostcheck.cu", "verify.cu", "witness.cu", "setup_host.cu", "setup.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-std=c++17", "-O3", "-lineinfo",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden",

@@ -73,7 +73,9 @@ struct MsmScratch {
   MsmArena slot[8];
 };
 
-// Fixed-base tables of the standard generators: [window][digit], 8-bit windows.
+// Fixed-base tables: [window][digit], 8-bit windows.  The context caches the standard generators' tables; key
+// generation with a caller's generator builds its own (32 x 256 points).
+constexpr uint32_t kFbWindows = 32, kFbEntries = 256;
 template <class C>
 struct FbTable {
   DevBuf<typename C::Affine> table;
@@ -141,6 +143,17 @@ void pack_flags_device(Ctx* ctx, const uint32_t* d_flags, uint32_t n, uint32_t* 
 
 // blocks of `threads` that cover n items
 inline uint32_t nblocks(uint64_t n, uint32_t threads) { return (uint32_t)((n + threads - 1) / threads); }
+
+// table for the generator `gen` (affine, Montgomery limbs, not the identity)
+template <class C>
+void fb_build(Ctx* ctx, FbTable<C>& t, const typename C::Affine& gen, cudaStream_t st);
+// the standard generator's table, built on first use and cached in the context
+template <class C>
+const FbTable<C>& fb_standard_table(Ctx* ctx, cudaStream_t st);
+// out[i] = scalars[i] * G for the table's G: affine points, identity bitmap words; scalars canonical.  Returns when done.
+template <class C>
+void fixed_base_mul(Ctx* ctx, const FbTable<C>& t, const FrEl* d_scalars, typename C::Affine* d_out,
+                    uint32_t* d_inf_words, uint32_t n, cudaStream_t st);
 
 // out[i] = scalars[i] * G (standard generator), affine; scalars canonical.
 void g1_fixed_base_mul_device(Ctx* ctx, const FrEl* d_scalars, G1::Affine* d_out, uint32_t* d_inf_words, uint32_t n,

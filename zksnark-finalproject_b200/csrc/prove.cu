@@ -135,6 +135,11 @@ struct PkImpl {
 
 namespace {
 
+constexpr size_t kG1Bytes = sizeof(G1::Xyzz), kG2Bytes = sizeof(G2::Xyzz);
+constexpr size_t kPartialBytes = 5 * kG1Bytes + kG2Bytes;   // A | sA | rB1 | L | H | B
+constexpr size_t kPlaneSlotBytes = kMsmMaxPlanes * sizeof(G2::Xyzz);
+static_assert(kPartialBytes == B2Z_PARTIAL_BYTES, "header constant out of sync");
+
 // copies `count` points (+ identity bits) from host arrays into dst[at ...)
 template <class Affine>
 void stage_points(Affine* d_dst, std::vector<uint32_t>& words, uint64_t at, const uint64_t* pts, const uint8_t* inf,
@@ -146,15 +151,60 @@ void stage_points(Affine* d_dst, std::vector<uint32_t>& words, uint64_t at, cons
       if ((inf[i >> 3] >> (i & 7)) & 1) words[(at + i) >> 5] |= 1u << ((at + i) & 31);
 }
 
-size_t pk_precompute_bytes(const b2z_pk_desc* d) {
+// `num` / `den` of the key's precomputed window copies fit in half the free device memory
+bool pk_precompute_fits_slice(uint32_t log_n, uint64_t m, uint64_t l, uint32_t num, uint32_t den) {
   auto cost = [](uint64_t n, size_t pt) {
     if (n == 0) return (size_t)0;
     const uint32_t c = msm_pick_c(n, true);
     return (size_t)n * pt * msm_windows(c);
   };
-  const uint64_t n = 1ull << d->log_domain;
-  return 2 * cost(d->num_variables + 2, 96) + cost(d->num_variables - d->num_instance + 1, 96) +
-         cost(d->num_variables + 2, 192) + cost(n, 96);
+  const uint64_t n = 1ull << log_n;
+  const size_t bytes = 2 * cost(m + 2, 96) + cost(m - l + 1, 96) + cost(m + 2, 192) + cost(n, 96);
+  size_t free_b = 0, total_b = 0;
+  B2Z_CUDA(cudaMemGetInfo(&free_b, &total_b));
+  return bytes / den * num < free_b / 2;
+}
+
+// the sizes of a whole key
+void pk_init_whole(Ctx& c, PkImpl& P, uint32_t log_n, uint64_t m, uint64_t l) {
+  P.owner = &c;
+  P.log_n = log_n;
+  P.m = m;
+  P.l = l;
+  P.lo = 0; P.ma = (uint32_t)m; P.l_skip = (uint32_t)l; P.ml = (uint32_t)(m - l);
+  P.h_lo = 0; P.hn = 1u << log_n; P.with_vk = 1;
+}
+
+// per-proof scratch, the proof's sums (arena slot, stream, tail offset, result) and events; after the shard fields
+void pk_alloc_scratch(Ctx& c, PkImpl& P) {
+  const uint64_t n = 1ull << P.log_n;
+  P.ea.alloc(n); P.eb.alloc(n); P.ec.alloc(n); P.hc.alloc(P.hn ? P.hn : 1);
+  P.z.alloc(P.m); P.zc.alloc(P.ma ? P.ma : 1); P.tail.alloc(5);
+  P.g1_out.alloc(SUM_B); P.g2_out.alloc(1);
+  B2Z_CUDA(cudaMallocHost(&P.h_out, kPartialBytes));
+  B2Z_CUDA(cudaMallocHost(&P.h_planes, SUM_COUNT * kPlaneSlotBytes));
+  auto new_event = [](cudaEvent_t* e) { B2Z_CUDA(cudaEventCreateWithFlags(e, cudaEventDisableTiming)); };
+  auto init = [&](Sum k, int slot, cudaStream_t stream, uint32_t tail, void* d_result) {
+    ProofSum& S = P.sums[k];
+    S.slot = slot;
+    S.stream = stream;
+    S.tail = tail;
+    S.d_result = d_result;
+    S.planes.host = P.h_planes + (size_t)k * kPlaneSlotBytes / 4;
+    if (k != SUM_H) {
+      new_event(&S.accum);
+      new_event(&S.done);
+    }
+  };
+  // arena slot, stream (H: the one prove_h_finish names), offset of the tail scalars in {1, r, 1, s, -rs}, result
+  init(SUM_A, 1, c.aux[0], 0, P.g1_out.p + SUM_A);
+  init(SUM_B1, 3, c.aux[2], 2, P.g1_out.p + SUM_B1);
+  init(SUM_L, 4, c.aux[3], 4, P.g1_out.p + SUM_L);
+  init(SUM_H, 0, c.stream, 0, P.g1_out.p + SUM_H);
+  init(SUM_B, 2, c.aux[1], 2, P.g2_out.p);
+  new_event(&P.sums[SUM_L].sorted);
+  new_event(&P.ev_z);
+  new_event(&P.ev_wm);
 }
 
 template <class C>
@@ -238,10 +288,6 @@ void fixed_base_entry(Ctx& c, const uint64_t* scalars, uint64_t n, uint64_t* out
   std::memcpy(out_inf, words.data(), (n + 7) / 8);
 }
 
-constexpr size_t kG1Bytes = sizeof(G1::Xyzz), kG2Bytes = sizeof(G2::Xyzz);
-constexpr size_t kPartialBytes = 5 * kG1Bytes + kG2Bytes;   // A | sA | rB1 | L | H | B
-constexpr size_t kPlaneSlotBytes = kMsmMaxPlanes * sizeof(G2::Xyzz);
-static_assert(kPartialBytes == B2Z_PARTIAL_BYTES, "header constant out of sync");
 
 // GPU part of a proof on this key (a whole key or one shard of it): leaves the XYZZ partial
 // sums A, s*A, r*B1, L, H (G1) and B (G2) in partial_out (host memory).
@@ -421,6 +467,21 @@ PkImpl& pk_of(Ctx& c, const b2z_pk* pk, const char* who) {
                                                      "belongs to one context; upload one copy per context)"};
   return P;
 }
+bool pk_precompute_fits(uint32_t log_n, uint64_t m, uint64_t l) { return pk_precompute_fits_slice(log_n, m, l, 1, 1); }
+b2z_pk* pk_from_device_sets(Ctx& c, uint32_t log_n, uint64_t m, uint64_t l, const PkDeviceSets& S, bool pre) {
+  std::unique_ptr<b2z_pk> pk(new b2z_pk());
+  PkImpl& P = pk->impl;
+  pk_init_whole(c, P, log_n, m, l);
+  cudaStream_t st = c.stream;
+  msm_bases_build<G1>(&c, P.a_set, S.a, S.a_words, (uint32_t)m + 2, pre, 0, st);
+  msm_bases_build<G1>(&c, P.b1_set, S.b1, S.b1_words, (uint32_t)m + 2, pre, 0, st);
+  msm_bases_build<G1>(&c, P.l_set, S.l, S.l_words, (uint32_t)(m - l) + 1, pre, 0, st);
+  msm_bases_build<G2>(&c, P.g2, S.b2, S.b2_words, (uint32_t)m + 2, pre, 0, st);
+  msm_bases_build<G1>(&c, P.h, S.h, S.h_words, P.hn, pre, 0, st);
+  B2Z_CUDA(cudaStreamSynchronize(st));
+  pk_alloc_scratch(c, P);
+  return pk.release();
+}
 bool pk_matches(const b2z_pk* pk, uint32_t log_n, uint64_t m, uint64_t l) {
   return pk->impl.log_n == log_n && pk->impl.m == m && pk->impl.l == l;
 }
@@ -514,10 +575,7 @@ static b2z_status pk_upload_impl(b2z_ctx* ctx, const b2z_pk_desc* d, uint32_t fr
                 B2Z_EINVAL, "b2z_pk_upload: NULL query array");
     std::unique_ptr<b2z_pk> pk(new b2z_pk());
     PkImpl& P = pk->impl;
-    P.owner = &c;
-    P.log_n = d->log_domain;
-    P.m = m;
-    P.l = l;
+    pk_init_whole(c, P, d->log_domain, m, l);
     // the variables of this shard, in local order
     if (cyc_world > 0 && l > kCycBlock) cyc_world = 0;   // the instance variables must sit in block 0
     uint64_t lo = m * from / den, hi = m * to / den;
@@ -539,9 +597,7 @@ static b2z_status pk_upload_impl(b2z_ctx* ctx, const b2z_pk_desc* d, uint32_t fr
     P.h_lo = (uint32_t)h_lo; P.hn = (uint32_t)(h_hi - h_lo);
     P.with_vk = from == 0 ? 1u : 0u;
     cudaStream_t st = c.stream;
-    size_t free_b = 0, total_b = 0;
-    B2Z_CUDA(cudaMemGetInfo(&free_b, &total_b));
-    const bool pre = pk_precompute_bytes(d) / den * (to - from) < free_b / 2;
+    const bool pre = pk_precompute_fits_slice(P.log_n, m, l, to - from, den);
     // `count` points of a query, starting at local variable `skip` of this shard, as one contiguous host array
     // (query index = variable index - shift) + identity bits; contiguous shards point straight into the caller's array
     struct Picked {
@@ -633,34 +689,85 @@ static b2z_status pk_upload_impl(b2z_ctx* ctx, const b2z_pk_desc* d, uint32_t fr
       msm_bases_build<G1>(&c, P.h, dst.p + h_lo, words.p, P.hn, pre, 0, st);
       B2Z_CUDA(cudaStreamSynchronize(st));
     }
-    P.ea.alloc(n); P.eb.alloc(n); P.ec.alloc(n); P.hc.alloc(P.hn ? P.hn : 1);
-    P.z.alloc(m); P.zc.alloc(P.ma ? P.ma : 1); P.tail.alloc(5);
-    P.g1_out.alloc(SUM_B); P.g2_out.alloc(1);
-    B2Z_CUDA(cudaMallocHost(&P.h_out, kPartialBytes));
-    B2Z_CUDA(cudaMallocHost(&P.h_planes, SUM_COUNT * kPlaneSlotBytes));
-    auto new_event = [](cudaEvent_t* e) { B2Z_CUDA(cudaEventCreateWithFlags(e, cudaEventDisableTiming)); };
-    auto init = [&](Sum k, int slot, cudaStream_t stream, uint32_t tail, void* d_result) {
-      ProofSum& S = P.sums[k];
-      S.slot = slot;
-      S.stream = stream;
-      S.tail = tail;
-      S.d_result = d_result;
-      S.planes.host = P.h_planes + (size_t)k * kPlaneSlotBytes / 4;
-      if (k != SUM_H) {
-        new_event(&S.accum);
-        new_event(&S.done);
-      }
-    };
-    // arena slot, stream (H: the one prove_h_finish names), offset of the tail scalars in {1, r, 1, s, -rs}, result
-    init(SUM_A, 1, c.aux[0], 0, P.g1_out.p + SUM_A);
-    init(SUM_B1, 3, c.aux[2], 2, P.g1_out.p + SUM_B1);
-    init(SUM_L, 4, c.aux[3], 4, P.g1_out.p + SUM_L);
-    init(SUM_H, 0, c.stream, 0, P.g1_out.p + SUM_H);
-    init(SUM_B, 2, c.aux[1], 2, P.g2_out.p);
-    new_event(&P.sums[SUM_L].sorted);
-    new_event(&P.ev_z);
-    new_event(&P.ev_wm);
+    pk_alloc_scratch(c, P);
     *out = pk.release();
+  });
+}
+
+}  // extern "C"
+
+namespace b2z {
+namespace {
+// copy 0 of a base set (the points as uploaded) and its identity bits, on the host
+template <class C>
+void download_set(const MsmBases<C>& B, std::vector<typename C::Affine>& pts, std::vector<uint32_t>& words,
+                  cudaStream_t st) {
+  pts.resize(B.n);
+  words.assign((B.n + 31) / 32, 0u);
+  if (B.n) B2Z_CUDA(cudaMemcpyAsync(pts.data(), B.points.p, B.n * sizeof(pts[0]), cudaMemcpyDeviceToHost, st));
+  if (B.n && B.inf_words.p)
+    B2Z_CUDA(cudaMemcpyAsync(words.data(), B.inf_words.p, words.size() * 4, cudaMemcpyDeviceToHost, st));
+  B2Z_CUDA(cudaStreamSynchronize(st));
+}
+inline bool word_bit(const std::vector<uint32_t>& w, uint64_t i) { return (w[i >> 5] >> (i & 31)) & 1; }
+// points [from, from + count) of a downloaded set -> caller's limbs + identity bitmap
+template <class Affine>
+void put_query(const std::vector<Affine>& pts, const std::vector<uint32_t>& words, uint64_t count, uint64_t* out,
+               uint8_t* inf) {
+  if (count == 0) return;
+  std::memcpy(out, pts.data(), count * sizeof(Affine));
+  std::memset(inf, 0, (count + 7) / 8);
+  for (uint64_t i = 0; i < count; i++)
+    if (word_bit(words, i)) inf[i >> 3] |= (uint8_t)(1u << (i & 7));
+}
+}  // namespace
+}  // namespace b2z
+
+extern "C" {
+
+b2z_status b2z_pk_download(b2z_ctx* ctx, const b2z_pk* pk, b2z_pk_arrays* out) {
+  return guarded(ctx, [&](Ctx& c) {
+    B2Z_REQUIRE(out != nullptr, B2Z_EINVAL, "b2z_pk_download: NULL argument");
+    const PkImpl& P = pk_of(c, pk, "b2z_pk_download");
+    const uint64_t n = 1ull << P.log_n, m = P.m, l = P.l;
+    B2Z_REQUIRE(P.with_vk && P.cyc_world == 0 && P.lo == 0 && P.ma == m && P.hn == n, B2Z_EINVAL,
+                "b2z_pk_download: the key is a shard; only whole keys (b2z_pk_upload, b2z_groth16_setup) download");
+    B2Z_REQUIRE(out->a_query && out->a_inf && out->b_g1_query && out->b_g1_inf && out->b_g2_query && out->b_g2_inf &&
+                    (n == 1 || (out->h_query && out->h_inf)) && (m == l || (out->l_query && out->l_inf)),
+                B2Z_EINVAL, "b2z_pk_download: NULL query array");
+    cudaStream_t st = c.stream;
+    out->num_variables = m;
+    out->num_instance = l;
+    out->log_domain = P.log_n;
+    std::vector<G1::Affine> p1;
+    std::vector<G2::Affine> p2;
+    std::vector<uint32_t> w;
+    download_set<G1>(P.a_set, p1, w, st);                  // [a_query | alpha_1 delta_1]
+    put_query(p1, w, m, out->a_query, out->a_inf);
+    std::memcpy(out->alpha_g1, &p1[m], sizeof(G1::Affine));
+    std::memcpy(out->delta_g1, &p1[m + 1], sizeof(G1::Affine));
+    download_set<G1>(P.b1_set, p1, w, st);                 // [b_g1_query | beta_1 delta_1]
+    put_query(p1, w, m, out->b_g1_query, out->b_g1_inf);
+    std::memcpy(out->beta_g1, &p1[m], sizeof(G1::Affine));
+    download_set<G1>(P.l_set, p1, w, st);                  // [l_query | delta_1]
+    put_query(p1, w, m - l, out->l_query, out->l_inf);
+    download_set<G2>(P.g2, p2, w, st);                     // [b_g2_query | beta_2 delta_2]
+    put_query(p2, w, m, out->b_g2_query, out->b_g2_inf);
+    std::memcpy(out->beta_g2, &p2[m], sizeof(G2::Affine));
+    std::memcpy(out->delta_g2, &p2[m + 1], sizeof(G2::Affine));
+    if (n > 1) {                                           // h: bit-reversed, padded to n -> natural order, n - 1 points
+      download_set<G1>(P.h, p1, w, st);
+      std::vector<G1::Affine> nat(n - 1);
+      std::vector<uint32_t> nat_w((n + 31) / 32, 0u);
+      for (uint64_t p = 0; p < n; p++) {
+        uint64_t j = 0;
+        for (uint32_t b = 0; b < P.log_n; b++) j |= ((p >> b) & 1) << (P.log_n - 1 - b);
+        if (j >= n - 1) continue;
+        nat[j] = p1[p];
+        if (word_bit(w, p)) nat_w[j >> 5] |= 1u << (j & 31);
+      }
+      put_query(nat, nat_w, n - 1, out->h_query, out->h_inf);
+    }
   });
 }
 

@@ -1,10 +1,37 @@
-// Entry points of prove.cu used by r1cs.cu.
+// Entry points of prove.cu and r1cs.cu used by the other translation units (r1cs.cu, setup.cu).
 #pragma once
 #include "common.hpp"
+#include "ec.cuh"
 
 struct b2z_pk;
+struct b2z_r1cs;
 
 namespace b2z {
+// one constraint matrix on the device, CSR as uploaded (column indices < num_variables, Montgomery coefficients)
+struct CsrDev {
+  DevBuf<uint32_t> row_ptr, cols;
+  DevBuf<FrEl> coeffs;
+};
+// the matrices of an uploaded r1cs; B2Z_EINVAL when the handle belongs to another context
+struct R1csView {
+  uint64_t nc, l, m;
+  uint32_t log_n;
+  const CsrDev* mat;   // A, B, C
+};
+R1csView r1cs_view(Ctx& c, b2z_r1cs* r, const char* who);
+
+// A whole key's five base sets in device memory (points + identity bitmap words), the layout b2z_pk_upload assembles:
+// a, b1, b2: m + 2 points [query | alpha_1 delta_1] / [query | beta_1 delta_1] / [query | beta_2 delta_2];
+// l: m - l + 1 points [l_query | delta_1]; h: n points, h_query in bit-reversed order, position n - 1 the flagged identity.
+struct PkDeviceSets {
+  const G1::Affine *a, *b1, *l, *h;
+  const G2::Affine* b2;
+  const uint32_t *a_words, *b1_words, *l_words, *h_words, *b2_words;
+};
+// b2z_pk_upload's rule for precomputed window copies: they fit in half the free device memory
+bool pk_precompute_fits(uint32_t log_n, uint64_t m, uint64_t l);
+// the key handle for those sets (copied; the caller keeps its buffers); `pre` from pk_precompute_fits
+b2z_pk* pk_from_device_sets(Ctx& c, uint32_t log_n, uint64_t m, uint64_t l, const PkDeviceSets& sets, bool pre);
 bool pk_matches(const b2z_pk* pk, uint32_t log_n, uint64_t m, uint64_t l);
 // whole-key proof from device-resident a/b/c evaluations (clobbered) and assignment
 void prove_on_device_buffers(Ctx& c, const b2z_pk* pk, FrEl* d_a, FrEl* d_b, FrEl* d_c, const FrEl* d_z,

@@ -15,11 +15,6 @@
 
 namespace b2z {
 
-struct CsrDev {
-  DevBuf<uint32_t> row_ptr, cols;
-  DevBuf<FrEl> coeffs;
-};
-
 // Two-pass row evaluation.  The rows of these circuits are wildly uneven (1 entry for a multiplication gate, up to
 // 33 for an inlined Poseidon MDS row; a warp of 32 consecutive rows does 3.3x the multiplications it needs when one
 // thread owns one row), so the multiplications are done per ENTRY (perfectly balanced; entries whose coefficient is
@@ -256,6 +251,10 @@ R1csImpl& r1cs_of(Ctx& c, b2z_r1cs* r, const char* who) {
   return r->impl;
 }
 }  // namespace
+R1csView r1cs_view(Ctx& c, b2z_r1cs* r, const char* who) {
+  const R1csImpl& R = r1cs_of(c, r, who);
+  return R1csView{R.nc, R.l, R.m, R.log_n, R.mat};
+}
 }  // namespace b2z
 
 extern "C" {

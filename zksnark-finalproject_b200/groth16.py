@@ -358,6 +358,9 @@ class ProvingKey:
         it) to the device, once per circuit.  weights (one positive integer per rank): uneven
         shards through b2z_pk_upload_slice -- rank k gets weights[k] / sum(weights) of the points."""
         spec = (int(rank), int(world), tuple(int(w) for w in weights) if weights is not None else None)
+        if self._handle is None and self.a_query is None:
+            raise ValueError("ProvingKey has no host arrays (it was generated on the device and freed before "
+                             "download()); download() it before free() to upload it again")
         if self._handle is not None:
             # a handle holds per-proof scratch and belongs to ONE context and ONE shard: never hand back a
             # handle that does not match what the caller asked for (free() first to re-upload)
@@ -399,6 +402,27 @@ class ProvingKey:
             ctx.check(ctx._lib.b2z_pk_upload_shard(ctx.handle, ctypes.byref(d), int(rank), int(world), ctypes.byref(h)))
         self._ctx, self._handle, self._spec = ctx, h, spec
         self.shard = (int(rank), int(world))
+        return self
+
+    def download(self):
+        """b2z_pk_download: fills the host arrays from the device copy of a whole key (the key
+        generate_parameters_on_device returns has none until then).  Returns self."""
+        if self._handle is None:
+            raise ValueError("ProvingKey is not on a device: nothing to download")
+        m, l, n = self.num_variables, self.num_instance, self.domain_size
+        arrays = {"a_query": (m, 12), "b_g1_query": (m, 12), "b_g2_query": (m, 24), "h_query": (n - 1, 12),
+                  "l_query": (m - l, 12)}
+        out = {k: (np.zeros(shape, dtype=np.uint64), np.zeros((shape[0] + 7) // 8, dtype=np.uint8))
+               for k, shape in arrays.items()}
+        d = _ffi.PkArrays()
+        for k, (pts, inf) in out.items():
+            setattr(d, k, _ptr(pts) if pts.size else None)
+            setattr(d, k.replace("_query", "_inf"), _ptr(inf) if pts.size else None)
+        self._ctx.check(self._ctx._lib.b2z_pk_download(self._ctx.handle, self._handle, ctypes.byref(d)))
+        for k in self.FIELDS:
+            setattr(self, k, out[k])
+        for k, w in (("alpha_g1", 12), ("beta_g1", 12), ("delta_g1", 12), ("beta_g2", 24), ("delta_g2", 24)):
+            setattr(self, k, np.array(getattr(d, k)[:w], dtype=np.uint64))
         return self
 
     def free(self):
@@ -706,6 +730,41 @@ class Groth16:
         pk = ProvingKey(m, l, n, g1(at_b), g1(bt_b), g2(bt_b), g1(bigint(hs)), g1(bigint(l_sc)),
                         singles1[0], singles1[1], singles1[2], singles2[0], singles2[2])
         vk = VerifyingKey(singles1[0], singles2[0], singles2[1], singles2[2], g1(bigint(g_sc)))
+        return pk, vk
+
+    @staticmethod
+    def generate_parameters_on_device(ctx, cm, alpha, beta, gamma, delta, tau, g1_generator=None, g2_generator=None):
+        """generate_parameters_with_qap for uploaded matrices, entirely on the GPU (b2z_groth16_setup), with the
+        caller's toxic waste (canonical ints) and generators (affine Montgomery limb arrays, 12 / 24 uint64; None = the
+        standard ones) -- what Groth16::setup does after its draws (oracle/ark_rng.py: setup_draws gives them in ark's
+        order).  Returns (ProvingKey, VerifyingKey).  The ProvingKey is already uploaded through ctx; its host arrays
+        stay None until pk.download()."""
+        cm.upload(ctx)
+        els = codec.fr_to_mont_limbs([alpha, beta, gamma, delta, tau])
+        keep = [els]
+        d = _ffi.SetupDesc()
+        d.alpha, d.beta, d.gamma, d.delta, d.tau = (_ptr(els[k:k + 1]) for k in range(5))
+        for name, g, width in (("g1_generator", g1_generator, 12), ("g2_generator", g2_generator, 24)):
+            if g is not None:
+                g = np.ascontiguousarray(g, dtype=np.uint64).reshape(-1)
+                if g.shape[0] != width:
+                    raise ValueError("%s: %d limbs expected" % (name, width))
+                keep.append(g)
+                setattr(d, name, _ptr(g))
+        l, m, n = cm.num_instance_variables, cm.num_variables, cm.domain_size
+        gabc = np.zeros((l, 12), dtype=np.uint64)
+        gabc_inf = np.zeros((l + 7) // 8, dtype=np.uint8)
+        vk_out = _ffi.VkOut()
+        vk_out.gamma_abc_g1, vk_out.gamma_abc_inf = _ptr(gabc), _ptr(gabc_inf)
+        h = ctypes.c_void_p()
+        ctx.check(ctx._lib.b2z_groth16_setup(ctx.handle, cm._handle, ctypes.byref(d), ctypes.byref(h),
+                                             ctypes.byref(vk_out)))
+        pk = ProvingKey(m, l, n, None, None, None, None, None, None, None, None, None, None)
+        pk._ctx, pk._handle, pk._spec = ctx, h, (0, 1, None)
+        pk.shard = (0, 1)
+        pt = lambda arr, w: np.array(arr[:w], dtype=np.uint64)
+        vk = VerifyingKey(pt(vk_out.alpha_g1, 12), pt(vk_out.beta_g2, 24), pt(vk_out.gamma_g2, 24),
+                          pt(vk_out.delta_g2, 24), (gabc, gabc_inf))
         return pk, vk
 
     @staticmethod

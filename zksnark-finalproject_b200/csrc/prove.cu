@@ -71,70 +71,6 @@ FrEl fr_load_host(const uint64_t v[4]) {
   return x;
 }
 
-}  // namespace
-
-// ---------------------------------------------------------------------------
-// Proving key
-// ---------------------------------------------------------------------------
-// The five MSMs of a proof, the G1 ones first.  (The partial sums leave in the order A | sA | rB1 | L | H | B,
-// B2Z_PARTIAL_BYTES.)
-enum Sum { SUM_A, SUM_B1, SUM_L, SUM_H, SUM_B, SUM_COUNT };
-
-// Where one MSM of a proof runs and what it leaves.
-struct ProofSum {
-  int slot = 0;                      // MSM scratch arena
-  cudaStream_t stream = nullptr;     // its accumulation (and, but for H, its sort)
-  uint32_t tail = 0;                 // its extra scalars: PkImpl::tail + this (not H)
-  void* d_result = nullptr;          // one XYZZ point (G2 for B)
-  MsmHostPlanes planes;              // its bit-plane sums, for the Horner pass on the host
-  cudaEvent_t accum = nullptr;       // accumulation kernel done (the next sum of the chain waits for it; not H)
-  cudaEvent_t done = nullptr;        // planes copied to the host (not H: prove_end synchronises its stream)
-  cudaEvent_t sorted = nullptr;      // L only: sort done (the G2 accumulation waits for it)
-  template <class C> typename C::Xyzz* result() const { return static_cast<typename C::Xyzz*>(d_result); }
-};
-
-struct PkImpl {
-  // A key handle holds per-proof scratch (below), so it belongs to exactly ONE context: the one it was
-  // uploaded through.  Every entry point checks this and returns B2Z_EINVAL for a foreign context.
-  const Ctx* owner = nullptr;
-  bool* assignment_flag = nullptr;   // b2z_groth16_shard_begin .. shard_finish window (r1cs.cu)
-  uint32_t log_n = 0;
-  uint64_t m = 0, l = 0;
-  // shard: `ma` variables of the a/b queries -- either the contiguous range [lo, lo+ma) (cyc_world == 0) or,
-  // block-cyclic, the blocks cyc_rank, cyc_rank + cyc_world, ... of kCycBlock variables (balanced whatever the
-  // witness structure: Groth16 assignments have long stretches of small / Boolean values); the first l_skip of
-  // them are instance variables (not in l_query), ml = ma - l_skip; bit-reversed h positions [h_lo, h_lo+hn);
-  // alpha/beta/delta terms on shard 0 only
-  uint32_t lo = 0, ma = 0, l_skip = 0, ml = 0, h_lo = 0, hn = 0, with_vk = 1;
-  uint32_t cyc_world = 0, cyc_rank = 0;
-  MsmBases<G1> a_set;          // [a_query  | alpha_1 delta_1]
-  MsmBases<G1> b1_set;         // [b_g1     | beta_1  delta_1]
-  MsmBases<G1> l_set;          // [l_query  | delta_1]
-  MsmBases<G1> h;              // h_query, bit-reversed order, padded to n (this shard's positions)
-  MsmBases<G2> g2;             // [b_g2     | beta_2  delta_2]
-  // per-proof device scratch
-  DevBuf<FrEl> ea, eb, ec, z, zc, hc, tail;
-  DevBuf<G1::Xyzz> g1_out;     // results of the G1 sums, indexed by Sum (s*A and r*B1 are made on the host)
-  DevBuf<G2::Xyzz> g2_out;     // result of B
-  uint32_t* h_out = nullptr;   // pinned: B2Z_PARTIAL_BYTES
-  uint32_t* h_planes = nullptr;   // pinned: bit-plane sums of the five MSMs (host-side Horner, msm.hpp)
-  ProofSum sums[SUM_COUNT];
-  FrEl r_c, s_c;                  // the proof's r, s as canonical integers (prove_begin -> prove_end)
-  cudaEvent_t ev_z = nullptr;
-  cudaEvent_t ev_wm = nullptr;       // witness-map transforms of the proof in flight are done (gates the first accumulation)
-  ~PkImpl() {
-    if (h_out) cudaFreeHost(h_out);
-    if (h_planes) cudaFreeHost(h_planes);
-    if (ev_z) cudaEventDestroy(ev_z);
-    for (ProofSum& S : sums)
-      for (cudaEvent_t e : {S.accum, S.done, S.sorted})
-        if (e) cudaEventDestroy(e);
-    if (ev_wm) cudaEventDestroy(ev_wm);
-  }
-};
-
-namespace {
-
 constexpr size_t kG1Bytes = sizeof(G1::Xyzz), kG2Bytes = sizeof(G2::Xyzz);
 constexpr size_t kPartialBytes = 5 * kG1Bytes + kG2Bytes;   // A | sA | rB1 | L | H | B
 constexpr size_t kPlaneSlotBytes = kMsmMaxPlanes * sizeof(G2::Xyzz);
@@ -196,11 +132,11 @@ void pk_alloc_scratch(Ctx& c, PkImpl& P) {
       new_event(&S.done);
     }
   };
-  // arena slot, stream (H: the one prove_h_finish names), offset of the tail scalars in {1, r, 1, s, -rs}, result
+  // arena slot, stream (H: set by proof_h_sort), offset of the tail scalars in {1, r, 1, s, -rs}, result
   init(SUM_A, 1, c.aux[0], 0, P.g1_out.p + SUM_A);
   init(SUM_B1, 3, c.aux[2], 2, P.g1_out.p + SUM_B1);
   init(SUM_L, 4, c.aux[3], 4, P.g1_out.p + SUM_L);
-  init(SUM_H, 0, c.stream, 0, P.g1_out.p + SUM_H);
+  init(SUM_H, 0, nullptr, 0, P.g1_out.p + SUM_H);
   init(SUM_B, 2, c.aux[1], 2, P.g2_out.p);
   new_event(&P.sums[SUM_L].sorted);
   new_event(&P.ev_z);
@@ -289,15 +225,25 @@ void fixed_base_entry(Ctx& c, const uint64_t* scalars, uint64_t n, uint64_t* out
 }
 
 
-// GPU part of a proof on this key (a whole key or one shard of it): leaves the XYZZ partial
-// sums A, s*A, r*B1, L, H (G1) and B (G2) in partial_out (host memory).
-// A proof in three steps that share the key's scratch (PkImpl): prove_begin launches everything that
-// depends on z only, prove_quotient what needs the three coset evaluation vectors, prove_end waits and
-// does the host epilogue.  The single-GPU prover runs them back to back; the sharded prover with a
-// distributed witness map (b2z_groth16_shard_*) lets the caller exchange the coset evaluations between
-// prove_begin and prove_quotient while the z-only accumulations are already running.
-void prove_accums(Ctx& c, PkImpl& pk, cudaEvent_t gate = nullptr);
-void prove_begin(Ctx& c, PkImpl& pk, const FrEl* d_z, const uint64_t r[4], const uint64_t s[4], bool with_accums = true) {
+// the host-side a/b/c evaluations and assignment of b2z_groth16_prove[_partial] into the key's scratch: z on the
+// stream that prepares the MSM scalars, the evaluations on the main stream
+void stage_host_inputs(Ctx& c, PkImpl& P, const uint64_t* a, const uint64_t* b, const uint64_t* cc, const uint64_t* z) {
+  const size_t n = (size_t)1 << P.log_n;
+  B2Z_CUDA(cudaMemcpyAsync(P.z.p, z, P.m * sizeof(FrEl), cudaMemcpyHostToDevice, c.aux[0]));
+  B2Z_CUDA(cudaMemcpyAsync(P.ea.p, a, n * sizeof(FrEl), cudaMemcpyHostToDevice, c.stream));
+  B2Z_CUDA(cudaMemcpyAsync(P.eb.p, b, n * sizeof(FrEl), cudaMemcpyHostToDevice, c.stream));
+  B2Z_CUDA(cudaMemcpyAsync(P.ec.p, cc, n * sizeof(FrEl), cudaMemcpyHostToDevice, c.stream));
+}
+
+}  // namespace
+
+// ---------------------------------------------------------------------------
+// The five phases of a proof (prove_internal.hpp).  prove_partial_device and b2z_dist_prove issue the light work
+// first -- scalar prep, the sorts, the witness map, the H sort -- and then the GPU-filling accumulations back to back;
+// b2z_groth16_shard_begin starts the z-only accumulations at once, while the caller exchanges the coset evaluations
+// that b2z_groth16_shard_finish takes.
+// ---------------------------------------------------------------------------
+void proof_begin(Ctx& c, PkImpl& pk, const FrEl* d_z, const uint64_t r[4], const uint64_t s[4]) {
   ProofSum &A = pk.sums[SUM_A], &B1 = pk.sums[SUM_B1], &B = pk.sums[SUM_B], &L = pk.sums[SUM_L];
   // host-side scalars: r, s, -(r s) as canonical integers
   const FrEl r_m = Fr::reduce(fr_load_host(r)), s_m = Fr::reduce(fr_load_host(s));
@@ -327,7 +273,13 @@ void prove_begin(Ctx& c, PkImpl& pk, const FrEl* d_z, const uint64_t r[4], const
   B2Z_CUDA(cudaStreamWaitEvent(L.stream, pk.ev_z, 0));
   msm_sort<G1>(&c, L.slot, pk.l_set, z_l, pk.ml, pk.tail.p + L.tail, L.stream);
   B2Z_CUDA(cudaEventRecord(L.sorted, L.stream));
-  if (with_accums) prove_accums(c, pk);
+}
+
+void proof_h_sort(Ctx& c, PkImpl& pk, const FrEl* d_h, cudaStream_t st) {
+  ProofSum& H = pk.sums[SUM_H];
+  H.stream = st;
+  fr_from_mont_device(&c, d_h, pk.hc.p, pk.hn, st);
+  msm_sort<G1>(&c, H.slot, pk.h, pk.hc.p, pk.hn, nullptr, st);
 }
 
 // gate: fired when the witness map's transforms are done.  An accumulation kernel fills every SM for its whole
@@ -335,13 +287,13 @@ void prove_begin(Ctx& c, PkImpl& pk, const FrEl* d_z, const uint64_t r[4], const
 // accumulations and the H sum then waits for it with an idle GPU (8.7 of 100 ms at 2^22 before this gate).  The light
 // phase -- sorts (latency / atomics bound) next to row evaluation and transforms (integer-pipe bound) -- overlaps
 // well instead, and the accumulations then run back to back with the H sort hidden under them.
-void prove_accums(Ctx& c, PkImpl& pk, cudaEvent_t gate) {
+void proof_accums(Ctx& c, PkImpl& pk, cudaEvent_t gate) {
   ProofSum &A = pk.sums[SUM_A], &B1 = pk.sums[SUM_B1], &B = pk.sums[SUM_B], &L = pk.sums[SUM_L];
   // ---- accumulations chained by events (order below).  Each accumulation kernel is sized to fill the GPU by
   // itself; the G2 one (255 registers) leaves room for nothing, a G1 one leaves room on every SM for sort /
   // transform / tail blocks (the tail kernels are register-capped for exactly that), so tails overlap the next sums.
   // Every reduction stops at its bit-plane sums; the serial Horner pass over them, s*A and r*B1 are done
-  // by the HOST (prove_end) while the GPU is still busy with L and H.  (With the scalar multiplications
+  // by the HOST (proof_end) while the GPU is still busy with L and H.  (With the scalar multiplications
   // on the GPU -- 1.5 ms each even with lane-cooperative arithmetic -- every order tried put one of them
   // on the critical path: 7.65-8.3 ms per C2 proof.)
   // Chaining only pays when an accumulation fills the GPU (148 SMs x 256 threads x >= 8 references each): below
@@ -370,24 +322,14 @@ void prove_accums(Ctx& c, PkImpl& pk, cudaEvent_t gate) {
   B2Z_CUDA(cudaEventRecord(L.done, L.stream));
 }
 
-// d_a, d_b, d_c: evaluations of the three QAP combinations on the coset g H (d_a is clobbered)
-void prove_h_finish(Ctx& c, PkImpl& pk, cudaStream_t st = nullptr) {
+void proof_h_finish(Ctx& c, PkImpl& pk) {
   const bool chain = (uint64_t)pk.h.n * pk.h.windows >= (1u << 18);
   ProofSum& H = pk.sums[SUM_H];
-  H.stream = st ? st : c.stream;
   msm_finish<G1>(&c, H.slot, pk.h, H.result<G1>(), H.stream, chain ? pk.sums[SUM_L].accum : nullptr, nullptr,
                  &H.planes);
 }
-void prove_quotient(Ctx& c, PkImpl& pk, FrEl* d_a, const FrEl* d_b, const FrEl* d_c, bool with_h_finish = true) {
-  cudaStream_t st = c.stream;
-  witness_map_quotient(&c, d_a, d_b, d_c, pk.log_n, /*natural_out=*/false, st);    // whole domain, every shard
-  B2Z_CUDA(cudaEventRecord(pk.ev_wm, st));
-  fr_from_mont_device(&c, d_a + pk.h_lo, pk.hc.p, pk.hn, st);
-  msm_sort<G1>(&c, pk.sums[SUM_H].slot, pk.h, pk.hc.p, pk.hn, nullptr, st);
-  if (with_h_finish) prove_h_finish(c, pk);
-}
 
-void prove_end(Ctx& c, PkImpl& pk, uint8_t* partial_out) {
+void proof_end(Ctx& c, PkImpl& pk, uint8_t* partial_out) {
   auto planes = [&](Sum k) { return static_cast<const uint32_t*>(pk.sums[k].planes.host); };
   auto g1_result = [&](Sum k) { return host::g1_planes_horner(planes(k), pk.sums[k].planes.nplanes, kMsmChunkLog); };
   // A, s*A, B1, r*B1 while the GPU works on L and H
@@ -409,15 +351,16 @@ void prove_end(Ctx& c, PkImpl& pk, uint8_t* partial_out) {
 
 void prove_partial_device(Ctx& c, PkImpl& pk, FrEl* d_a, FrEl* d_b, FrEl* d_c, const FrEl* d_z, const uint64_t r[4],
                           const uint64_t s[4], uint8_t* partial_out) {
-  // issue order: everything light first (sorts, witness map, H sort), then the GPU-filling accumulations
-  prove_begin(c, pk, d_z, r, s, /*with_accums=*/false);
+  proof_begin(c, pk, d_z, r, s);
   witness_map_transform3(&c, d_a, d_b, d_c, pk.log_n, c.stream);
-  prove_quotient(c, pk, d_a, d_b, d_c, /*with_h_finish=*/false);
+  witness_map_quotient(&c, d_a, d_b, d_c, pk.log_n, /*natural_out=*/false, c.stream);    // whole domain, every shard
+  B2Z_CUDA(cudaEventRecord(pk.ev_wm, c.stream));
+  proof_h_sort(c, pk, d_a + pk.h_lo, c.stream);
   // small domains: the transforms run in 128-thread CTAs that fit on an SM beside a G1 accumulation and fill its
   // idle issue slots (the accumulations are latency-bound there), so no gate
-  prove_accums(c, pk, pk.log_n >= 19 ? pk.ev_wm : nullptr);
-  prove_h_finish(c, pk);
-  prove_end(c, pk, partial_out);
+  proof_accums(c, pk, pk.log_n >= 19 ? pk.ev_wm : nullptr);
+  proof_h_finish(c, pk);
+  proof_end(c, pk, partial_out);
 }
 
 // Host epilogue: sum the partials of all shards, normalise, serialise (host_fq.hpp).
@@ -441,14 +384,12 @@ void combine_partials(const uint8_t* partials, uint32_t world, uint8_t proof_out
 
 void prove_device(Ctx& c, PkImpl& pk, FrEl* d_a, FrEl* d_b, FrEl* d_c, const FrEl* d_z, const uint64_t r[4],
                   const uint64_t s[4], uint8_t proof_out[192]) {
-  B2Z_REQUIRE(pk.with_vk && pk.ma == pk.m && pk.hn == (1u << pk.log_n), B2Z_EINVAL,
+  B2Z_REQUIRE(pk.whole(), B2Z_EINVAL,
               "b2z_groth16_prove needs a whole key; use b2z_groth16_prove_partial + b2z_groth16_combine on shards");
   uint8_t partial[kPartialBytes];
   prove_partial_device(c, pk, d_a, d_b, d_c, d_z, r, s, partial);
   combine_partials(partial, 1, proof_out);
 }
-
-}  // namespace
 }  // namespace b2z
 
 using namespace b2z;
@@ -481,56 +422,6 @@ b2z_pk* pk_from_device_sets(Ctx& c, uint32_t log_n, uint64_t m, uint64_t l, cons
   B2Z_CUDA(cudaStreamSynchronize(st));
   pk_alloc_scratch(c, P);
   return pk.release();
-}
-bool pk_matches(const b2z_pk* pk, uint32_t log_n, uint64_t m, uint64_t l) {
-  return pk->impl.log_n == log_n && pk->impl.m == m && pk->impl.l == l;
-}
-void prove_on_device_buffers(Ctx& c, const b2z_pk* pk, FrEl* d_a, FrEl* d_b, FrEl* d_c, const FrEl* d_z,
-                             const uint64_t r[4], const uint64_t s[4], uint8_t proof_out[192]) {
-  prove_device(c, pk_of(c, pk, "b2z_groth16_prove"), d_a, d_b, d_c, d_z, r, s, proof_out);
-}
-void prove_partial_on_device_buffers(Ctx& c, const b2z_pk* pk, FrEl* d_a, FrEl* d_b, FrEl* d_c, const FrEl* d_z,
-                                     const uint64_t r[4], const uint64_t s[4], uint8_t* partial_out) {
-  prove_partial_device(c, pk_of(c, pk, "b2z_groth16_prove_partial"), d_a, d_b, d_c, d_z, r, s, partial_out);
-}
-void prove_begin_on(Ctx& c, const b2z_pk* pk, const FrEl* d_z, const uint64_t r[4], const uint64_t s[4]) {
-  prove_begin(c, pk_of(c, pk, "b2z_groth16_shard_begin"), d_z, r, s);
-}
-// ---- pieces of a proof for the tile-sharded (distributed witness map) prover in r1cs.cu
-void prove_begin_sorts_on(Ctx& c, const b2z_pk* pk, const FrEl* d_z, const uint64_t r[4], const uint64_t s[4]) {
-  prove_begin(c, pk_of(c, pk, "b2z_dist_prove"), d_z, r, s, /*with_accums=*/false);
-}
-uint32_t pk_h_chunk(const b2z_pk* pk, uint32_t* h_lo) {
-  if (h_lo) *h_lo = pk->impl.h_lo;
-  return pk->impl.hn;
-}
-// d_h: this shard's hn coefficients of h (bit-reversed positions [h_lo, h_lo + hn)), canonical Montgomery form
-void prove_dist_h_sort_on(Ctx& c, const b2z_pk* pk, const FrEl* d_h, cudaStream_t st) {
-  PkImpl& P = pk_of(c, pk, "b2z_dist_prove");
-  fr_from_mont_device(&c, d_h, P.hc.p, P.hn, st);
-  msm_sort<G1>(&c, P.sums[SUM_H].slot, P.h, P.hc.p, P.hn, nullptr, st);
-}
-// all five accumulations, chained: the first once `wm_done` has fired (the witness map's transform kernels need the
-// SMs the accumulations would fill), H on `h_st` -- the stream its sort was queued on, which therefore hides under
-// the other accumulations; then the host epilogue
-void prove_dist_finish_on(Ctx& c, const b2z_pk* pk, cudaEvent_t wm_done, cudaStream_t h_st, uint8_t* partial_out) {
-  PkImpl& P = pk_of(c, pk, "b2z_dist_prove");
-  prove_accums(c, P, wm_done);                            // the G2 accumulation opens the chain
-  prove_h_finish(c, P, h_st);
-  prove_end(c, P, partial_out);
-}
-void combine_partials_host(const uint8_t* partials, uint32_t world, uint8_t proof_out[192]) {
-  combine_partials(partials, world, proof_out);
-}
-void pk_bind_assignment_flag(const b2z_pk* pk, bool* flag) { const_cast<b2z_pk*>(pk)->impl.assignment_flag = flag; }
-void prove_finish_on(Ctx& c, const b2z_pk* pk, FrEl* d_a, const FrEl* d_b, const FrEl* d_c, uint8_t* partial_out) {
-  PkImpl& P = pk_of(c, pk, "b2z_groth16_shard_finish");
-  if (P.assignment_flag != nullptr) {
-    *P.assignment_flag = false;
-    P.assignment_flag = nullptr;
-  }
-  prove_quotient(c, P, d_a, d_b, d_c);
-  prove_end(c, P, partial_out);
 }
 }  // namespace b2z
 
@@ -730,7 +621,7 @@ b2z_status b2z_pk_download(b2z_ctx* ctx, const b2z_pk* pk, b2z_pk_arrays* out) {
     B2Z_REQUIRE(out != nullptr, B2Z_EINVAL, "b2z_pk_download: NULL argument");
     const PkImpl& P = pk_of(c, pk, "b2z_pk_download");
     const uint64_t n = 1ull << P.log_n, m = P.m, l = P.l;
-    B2Z_REQUIRE(P.with_vk && P.cyc_world == 0 && P.lo == 0 && P.ma == m && P.hn == n, B2Z_EINVAL,
+    B2Z_REQUIRE(P.whole(), B2Z_EINVAL,
                 "b2z_pk_download: the key is a shard; only whole keys (b2z_pk_upload, b2z_groth16_setup) download");
     B2Z_REQUIRE(out->a_query && out->a_inf && out->b_g1_query && out->b_g1_inf && out->b_g2_query && out->b_g2_inf &&
                     (n == 1 || (out->h_query && out->h_inf)) && (m == l || (out->l_query && out->l_inf)),
@@ -796,11 +687,7 @@ b2z_status b2z_groth16_prove_partial(b2z_ctx* ctx, const b2z_pk* pk_c, const uin
     B2Z_REQUIRE(pk_c && a_evals && b_evals && c_evals && z && r && s && partial_out, B2Z_EINVAL,
                 "b2z_groth16_prove_partial: NULL argument");
     PkImpl& P = pk_of(c, pk_c, "b2z_groth16_prove_partial");
-    const size_t n = (size_t)1 << P.log_n;
-    B2Z_CUDA(cudaMemcpyAsync(P.z.p, z, P.m * sizeof(FrEl), cudaMemcpyHostToDevice, c.aux[0]));
-    B2Z_CUDA(cudaMemcpyAsync(P.ea.p, a_evals, n * sizeof(FrEl), cudaMemcpyHostToDevice, c.stream));
-    B2Z_CUDA(cudaMemcpyAsync(P.eb.p, b_evals, n * sizeof(FrEl), cudaMemcpyHostToDevice, c.stream));
-    B2Z_CUDA(cudaMemcpyAsync(P.ec.p, c_evals, n * sizeof(FrEl), cudaMemcpyHostToDevice, c.stream));
+    stage_host_inputs(c, P, a_evals, b_evals, c_evals, z);
     prove_partial_device(c, P, P.ea.p, P.eb.p, P.ec.p, P.z.p, r, s, partial_out);
   });
 }
@@ -830,11 +717,7 @@ b2z_status b2z_groth16_prove(b2z_ctx* ctx, const b2z_pk* pk_c, const uint64_t* a
     B2Z_REQUIRE(pk_c && a_evals && b_evals && c_evals && z && r && s && proof_out, B2Z_EINVAL,
                 "b2z_groth16_prove: NULL argument");
     PkImpl& P = pk_of(c, pk_c, "b2z_groth16_prove");
-    const size_t n = (size_t)1 << P.log_n;
-    B2Z_CUDA(cudaMemcpyAsync(P.z.p, z, P.m * sizeof(FrEl), cudaMemcpyHostToDevice, c.aux[0]));
-    B2Z_CUDA(cudaMemcpyAsync(P.ea.p, a_evals, n * sizeof(FrEl), cudaMemcpyHostToDevice, c.stream));
-    B2Z_CUDA(cudaMemcpyAsync(P.eb.p, b_evals, n * sizeof(FrEl), cudaMemcpyHostToDevice, c.stream));
-    B2Z_CUDA(cudaMemcpyAsync(P.ec.p, c_evals, n * sizeof(FrEl), cudaMemcpyHostToDevice, c.stream));
+    stage_host_inputs(c, P, a_evals, b_evals, c_evals, z);
     prove_device(c, P, P.ea.p, P.eb.p, P.ec.p, P.z.p, r, s, proof_out);
   });
 }

@@ -1,7 +1,8 @@
-// Entry points of prove.cu and r1cs.cu used by the other translation units (r1cs.cu, setup.cu).
+// The proving key and the phases of a proof on it, shared by prove.cu, r1cs.cu and setup.cu.
 #pragma once
 #include "common.hpp"
 #include "ec.cuh"
+#include "msm.hpp"
 
 struct b2z_pk;
 struct b2z_r1cs;
@@ -32,24 +33,96 @@ struct PkDeviceSets {
 bool pk_precompute_fits(uint32_t log_n, uint64_t m, uint64_t l);
 // the key handle for those sets (copied; the caller keeps its buffers); `pre` from pk_precompute_fits
 b2z_pk* pk_from_device_sets(Ctx& c, uint32_t log_n, uint64_t m, uint64_t l, const PkDeviceSets& sets, bool pre);
-bool pk_matches(const b2z_pk* pk, uint32_t log_n, uint64_t m, uint64_t l);
-// whole-key proof from device-resident a/b/c evaluations (clobbered) and assignment
-void prove_on_device_buffers(Ctx& c, const b2z_pk* pk, FrEl* d_a, FrEl* d_b, FrEl* d_c, const FrEl* d_z,
-                             const uint64_t r[4], const uint64_t s[4], uint8_t proof_out[192]);
-// the same for one shard of a key: B2Z_PARTIAL_BYTES of partial sums
-void prove_partial_on_device_buffers(Ctx& c, const b2z_pk* pk, FrEl* d_a, FrEl* d_b, FrEl* d_c, const FrEl* d_z,
-                                     const uint64_t r[4], const uint64_t s[4], uint8_t* partial_out);
-// the same in two calls (sharded prover with a distributed witness map): z-only work first (returns while the
-// GPU is busy), then quotient + H + host epilogue from the three COSET evaluation vectors (d_a is clobbered)
-void prove_begin_on(Ctx& c, const b2z_pk* pk, const FrEl* d_z, const uint64_t r[4], const uint64_t s[4]);
-// tile-sharded prover (r1cs.cu: b2z_dist_*): z-only sorts; the H sort from this shard's chunk of h; the chained
-// accumulations + host epilogue once `ready` has fired
-void prove_begin_sorts_on(Ctx& c, const b2z_pk* pk, const FrEl* d_z, const uint64_t r[4], const uint64_t s[4]);
-uint32_t pk_h_chunk(const b2z_pk* pk, uint32_t* h_lo);
-void prove_dist_h_sort_on(Ctx& c, const b2z_pk* pk, const FrEl* d_h, cudaStream_t st);
-void prove_dist_finish_on(Ctx& c, const b2z_pk* pk, cudaEvent_t wm_done, cudaStream_t h_st, uint8_t* partial_out);
-void combine_partials_host(const uint8_t* partials, uint32_t world, uint8_t proof_out[192]);
-// remembers where the "assignment uploaded" flag of the r1cs used by shard_begin lives; prove_finish_on clears it
-void pk_bind_assignment_flag(const b2z_pk* pk, bool* flag);
-void prove_finish_on(Ctx& c, const b2z_pk* pk, FrEl* d_a, const FrEl* d_b, const FrEl* d_c, uint8_t* partial_out);
+
+// ---------------------------------------------------------------------------
+// Proving key
+// ---------------------------------------------------------------------------
+// The five MSMs of a proof, the G1 ones first.  (The partial sums leave in the order A | sA | rB1 | L | H | B,
+// B2Z_PARTIAL_BYTES.)
+enum Sum { SUM_A, SUM_B1, SUM_L, SUM_H, SUM_B, SUM_COUNT };
+
+// Where one MSM of a proof runs and what it leaves.
+struct ProofSum {
+  int slot = 0;                      // MSM scratch arena
+  cudaStream_t stream = nullptr;     // its accumulation (and, but for H, its sort); H: set by proof_h_sort
+  uint32_t tail = 0;                 // its extra scalars: PkImpl::tail + this (not H)
+  void* d_result = nullptr;          // one XYZZ point (G2 for B)
+  MsmHostPlanes planes;              // its bit-plane sums, for the Horner pass on the host
+  cudaEvent_t accum = nullptr;       // accumulation kernel done (the next sum of the chain waits for it; not H)
+  cudaEvent_t done = nullptr;        // planes copied to the host (not H: proof_end synchronises its stream)
+  cudaEvent_t sorted = nullptr;      // L only: sort done (the G2 accumulation waits for it)
+  template <class C> typename C::Xyzz* result() const { return static_cast<typename C::Xyzz*>(d_result); }
+};
+
+struct PkImpl {
+  // A key handle holds per-proof scratch (below), so it belongs to exactly ONE context: the one it was
+  // uploaded through.  Every entry point checks this and returns B2Z_EINVAL for a foreign context.
+  const Ctx* owner = nullptr;
+  bool* assignment_flag = nullptr;   // b2z_groth16_shard_begin .. shard_finish window (r1cs.cu)
+  uint32_t log_n = 0;
+  uint64_t m = 0, l = 0;
+  // shard: `ma` variables of the a/b queries -- either the contiguous range [lo, lo+ma) (cyc_world == 0) or,
+  // block-cyclic, the blocks cyc_rank, cyc_rank + cyc_world, ... of kCycBlock variables (balanced whatever the
+  // witness structure: Groth16 assignments have long stretches of small / Boolean values); the first l_skip of
+  // them are instance variables (not in l_query), ml = ma - l_skip; bit-reversed h positions [h_lo, h_lo+hn);
+  // alpha/beta/delta terms on shard 0 only
+  uint32_t lo = 0, ma = 0, l_skip = 0, ml = 0, h_lo = 0, hn = 0, with_vk = 1;
+  uint32_t cyc_world = 0, cyc_rank = 0;
+  MsmBases<G1> a_set;          // [a_query  | alpha_1 delta_1]
+  MsmBases<G1> b1_set;         // [b_g1     | beta_1  delta_1]
+  MsmBases<G1> l_set;          // [l_query  | delta_1]
+  MsmBases<G1> h;              // h_query, bit-reversed order, padded to n (this shard's positions)
+  MsmBases<G2> g2;             // [b_g2     | beta_2  delta_2]
+  // per-proof device scratch
+  DevBuf<FrEl> ea, eb, ec, z, zc, hc, tail;
+  DevBuf<G1::Xyzz> g1_out;     // results of the G1 sums, indexed by Sum (s*A and r*B1 are made on the host)
+  DevBuf<G2::Xyzz> g2_out;     // result of B
+  uint32_t* h_out = nullptr;   // pinned: B2Z_PARTIAL_BYTES
+  uint32_t* h_planes = nullptr;   // pinned: bit-plane sums of the five MSMs (host-side Horner, msm.hpp)
+  ProofSum sums[SUM_COUNT];
+  FrEl r_c, s_c;                  // the proof's r, s as canonical integers (proof_begin -> proof_end)
+  cudaEvent_t ev_z = nullptr;
+  cudaEvent_t ev_wm = nullptr;       // witness-map transforms of the proof in flight are done (gates the first accumulation)
+  // every variable, every h position and the alpha/beta/delta terms: not a shard
+  bool whole() const { return with_vk && cyc_world == 0 && lo == 0 && ma == m && hn == (1ull << log_n); }
+  ~PkImpl() {
+    if (h_out) cudaFreeHost(h_out);
+    if (h_planes) cudaFreeHost(h_planes);
+    if (ev_z) cudaEventDestroy(ev_z);
+    for (ProofSum& S : sums)
+      for (cudaEvent_t e : {S.accum, S.done, S.sorted})
+        if (e) cudaEventDestroy(e);
+    if (ev_wm) cudaEventDestroy(ev_wm);
+  }
+};
+
+// the key behind a handle; B2Z_EINVAL naming `who` when it is NULL or was uploaded through another context
+PkImpl& pk_of(Ctx& c, const b2z_pk* pk, const char* who);
+
+// ---------------------------------------------------------------------------
+// A proof on a key (a whole key or one shard of it) in five phases that share the key's scratch.  Each driver calls
+// them around its own witness map: proof_begin first, proof_end last, proof_h_finish after proof_h_sort (its stream)
+// and proof_accums (the event it chains after).
+//   proof_begin     everything that depends on z only: the tail scalars {1, r, 1, s, -rs}, this shard's variables
+//                   of z (Montgomery form, d_z) as canonical integers, and the sorts of A, B (G2), B1 and L
+//   proof_h_sort    this shard's h coefficients (bit-reversed positions [h_lo, h_lo + hn), Montgomery form, d_h) to
+//                   canonical form, then the sort of H, on `st`; H accumulates on `st` too
+//   proof_accums    the accumulations A -> B1 -> B -> L, chained; the first waits for `gate` (nullptr: none)
+//   proof_h_finish  the accumulation of H, after L's
+//   proof_end       waits for the five sums and does the host epilogue: XYZZ partial sums A, s*A, r*B1, L, H (G1)
+//                   and B (G2) in partial_out (B2Z_PARTIAL_BYTES, host memory)
+void proof_begin(Ctx& c, PkImpl& P, const FrEl* d_z, const uint64_t r[4], const uint64_t s[4]);
+void proof_h_sort(Ctx& c, PkImpl& P, const FrEl* d_h, cudaStream_t st);
+void proof_accums(Ctx& c, PkImpl& P, cudaEvent_t gate);
+void proof_h_finish(Ctx& c, PkImpl& P);
+void proof_end(Ctx& c, PkImpl& P, uint8_t* partial_out);
+
+// the single-GPU proof from device-resident a/b/c evaluations (d_a is clobbered) and assignment: this shard's partial
+// sums; prove_device: the 192 proof bytes, on a whole key only (B2Z_EINVAL otherwise)
+void prove_partial_device(Ctx& c, PkImpl& P, FrEl* d_a, FrEl* d_b, FrEl* d_c, const FrEl* d_z, const uint64_t r[4],
+                          const uint64_t s[4], uint8_t* partial_out);
+void prove_device(Ctx& c, PkImpl& P, FrEl* d_a, FrEl* d_b, FrEl* d_c, const FrEl* d_z, const uint64_t r[4],
+                  const uint64_t s[4], uint8_t proof_out[192]);
+// host epilogue of a proof: sum the partials of `world` shards, normalise, serialise
+void combine_partials(const uint8_t* partials, uint32_t world, uint8_t proof_out[192]);
 }  // namespace b2z

@@ -212,10 +212,6 @@ void upload_csr(CsrDev& d, const uint64_t* row_ptr, const uint32_t* cols, const 
   B2Z_CUDA(cudaStreamSynchronize(st));   // rp is a local
 }
 
-void eval_rows(Ctx& c, R1csImpl& R, const FrEl* d_z, FrEl* a, FrEl* b, FrEl* cc, cudaStream_t st) {
-  run_plan(c, R.plan, d_z, a, b, cc, st);
-}
-
 // rows of ONE matrix (0 = A with the instance rows appended, 1 = B, 2 = C) against z, zero-padded to the domain
 void eval_one(Ctx& c, R1csImpl& R, uint32_t which, const FrEl* d_z, FrEl* out, cudaStream_t st) {
   const size_t n = (size_t)1 << R.log_n;
@@ -249,6 +245,21 @@ R1csImpl& r1cs_of(Ctx& c, b2z_r1cs* r, const char* who) {
     throw StatusError{B2Z_EINVAL, std::string(who) + ": this b2z_r1cs was uploaded through another b2z_ctx (a handle "
                                                      "belongs to one context; upload one copy per context)"};
   return r->impl;
+}
+// the key of a proof on these matrices: uploaded through this context, for a circuit of the same shape
+PkImpl& pk_for(Ctx& c, const b2z_pk* pk, const R1csImpl& R, const char* who) {
+  PkImpl& P = pk_of(c, pk, who);
+  if (P.log_n != R.log_n || P.m != R.m || P.l != R.l)
+    throw StatusError{B2Z_EINVAL, std::string(who) + ": key and matrices disagree"};
+  return P;
+}
+// z goes up once, on the stream that prepares the MSM scalars; the row evaluation reads it on the main stream
+// after an event.  cudaMemcpyDefault: z may also be a DEVICE pointer (assignment already resident).
+void stage_z_and_rows(Ctx& c, R1csImpl& R, const uint64_t* z) {
+  B2Z_CUDA(cudaMemcpyAsync(R.z.p, z, R.m * sizeof(FrEl), cudaMemcpyDefault, c.aux[0]));
+  B2Z_CUDA(cudaEventRecord(R.ev_z, c.aux[0]));
+  B2Z_CUDA(cudaStreamWaitEvent(c.stream, R.ev_z, 0));
+  run_plan(c, R.plan, R.z.p, R.ea.p, R.eb.p, R.ec.p, c.stream);
 }
 }  // namespace
 R1csView r1cs_view(Ctx& c, b2z_r1cs* r, const char* who) {
@@ -320,7 +331,7 @@ b2z_status b2z_r1cs_eval(b2z_ctx* ctx, b2z_r1cs* r, const uint64_t* z, uint64_t*
     const size_t n = (size_t)1 << R.log_n;
     cudaStream_t st = c.stream;
     B2Z_CUDA(cudaMemcpyAsync(R.z.p, z, R.m * sizeof(FrEl), cudaMemcpyHostToDevice, st));
-    eval_rows(c, R, R.z.p, R.ea.p, R.eb.p, R.ec.p, st);
+    run_plan(c, R.plan, R.z.p, R.ea.p, R.eb.p, R.ec.p, st);
     B2Z_CUDA(cudaMemcpyAsync(a_out, R.ea.p, n * sizeof(FrEl), cudaMemcpyDeviceToHost, st));
     B2Z_CUDA(cudaMemcpyAsync(b_out, R.eb.p, n * sizeof(FrEl), cudaMemcpyDeviceToHost, st));
     B2Z_CUDA(cudaMemcpyAsync(c_out, R.ec.p, n * sizeof(FrEl), cudaMemcpyDeviceToHost, st));
@@ -354,7 +365,7 @@ b2z_status b2z_witness_map_from_matrices(b2z_ctx* ctx, b2z_r1cs* r, const uint64
     const size_t n = (size_t)1 << R.log_n;
     cudaStream_t st = c.stream;
     B2Z_CUDA(cudaMemcpyAsync(R.z.p, z, R.m * sizeof(FrEl), cudaMemcpyHostToDevice, st));
-    eval_rows(c, R, R.z.p, R.ea.p, R.eb.p, R.ec.p, st);
+    run_plan(c, R.plan, R.z.p, R.ea.p, R.eb.p, R.ec.p, st);
     witness_map_device(&c, R.ea.p, R.eb.p, R.ec.p, R.log_n, /*natural_out=*/true, st);
     B2Z_CUDA(cudaMemcpyAsync(h_out, R.ea.p, n * sizeof(FrEl), cudaMemcpyDeviceToHost, st));
     B2Z_CUDA(cudaStreamSynchronize(st));
@@ -366,14 +377,9 @@ b2z_status b2z_groth16_prove_r1cs(b2z_ctx* ctx, const b2z_pk* pk, b2z_r1cs* r, c
   return guarded(ctx, [&](Ctx& c) {
     B2Z_REQUIRE(pk && r && z && rr && ss && proof_out, B2Z_EINVAL, "b2z_groth16_prove_r1cs: NULL argument");
     R1csImpl& R = r1cs_of(c, r, "b2z_groth16_prove_r1cs");
-    B2Z_REQUIRE(pk_matches(pk, R.log_n, R.m, R.l), B2Z_EINVAL, "b2z_groth16_prove_r1cs: key and matrices disagree");
-    // z goes up once, on the stream that prepares the MSM scalars; the row evaluation reads it on the
-    // main stream after an event.  cudaMemcpyDefault: z may also be a DEVICE pointer (assignment already resident).
-    B2Z_CUDA(cudaMemcpyAsync(R.z.p, z, R.m * sizeof(FrEl), cudaMemcpyDefault, c.aux[0]));
-    B2Z_CUDA(cudaEventRecord(R.ev_z, c.aux[0]));
-    B2Z_CUDA(cudaStreamWaitEvent(c.stream, R.ev_z, 0));
-    eval_rows(c, R, R.z.p, R.ea.p, R.eb.p, R.ec.p, c.stream);
-    prove_on_device_buffers(c, pk, R.ea.p, R.eb.p, R.ec.p, R.z.p, rr, ss, proof_out);
+    PkImpl& P = pk_for(c, pk, R, "b2z_groth16_prove_r1cs");
+    stage_z_and_rows(c, R, z);
+    prove_device(c, P, R.ea.p, R.eb.p, R.ec.p, R.z.p, rr, ss, proof_out);
   });
 }
 
@@ -382,12 +388,9 @@ b2z_status b2z_groth16_prove_partial_r1cs(b2z_ctx* ctx, const b2z_pk* pk, b2z_r1
   return guarded(ctx, [&](Ctx& c) {
     B2Z_REQUIRE(pk && r && z && rr && ss && partial_out, B2Z_EINVAL, "b2z_groth16_prove_partial_r1cs: NULL argument");
     R1csImpl& R = r1cs_of(c, r, "b2z_groth16_prove_partial_r1cs");
-    B2Z_REQUIRE(pk_matches(pk, R.log_n, R.m, R.l), B2Z_EINVAL, "b2z_groth16_prove_partial_r1cs: key and matrices disagree");
-    B2Z_CUDA(cudaMemcpyAsync(R.z.p, z, R.m * sizeof(FrEl), cudaMemcpyDefault, c.aux[0]));
-    B2Z_CUDA(cudaEventRecord(R.ev_z, c.aux[0]));
-    B2Z_CUDA(cudaStreamWaitEvent(c.stream, R.ev_z, 0));
-    eval_rows(c, R, R.z.p, R.ea.p, R.eb.p, R.ec.p, c.stream);
-    prove_partial_on_device_buffers(c, pk, R.ea.p, R.eb.p, R.ec.p, R.z.p, rr, ss, partial_out);
+    PkImpl& P = pk_for(c, pk, R, "b2z_groth16_prove_partial_r1cs");
+    stage_z_and_rows(c, R, z);
+    prove_partial_device(c, P, R.ea.p, R.eb.p, R.ec.p, R.z.p, rr, ss, partial_out);
   });
 }
 
@@ -410,13 +413,14 @@ b2z_status b2z_groth16_shard_begin(b2z_ctx* ctx, const b2z_pk* pk, b2z_r1cs* r, 
   return guarded(ctx, [&](Ctx& c) {
     B2Z_REQUIRE(pk && r && rr && ss, B2Z_EINVAL, "b2z_groth16_shard_begin: NULL argument");
     R1csImpl& R = r1cs_of(c, r, "b2z_groth16_shard_begin");
-    B2Z_REQUIRE(pk_matches(pk, R.log_n, R.m, R.l), B2Z_EINVAL, "b2z_groth16_shard_begin: key and matrices disagree");
+    PkImpl& P = pk_for(c, pk, R, "b2z_groth16_shard_begin");
     shard_assignment(c, R, z, "b2z_groth16_shard_begin");
     B2Z_CUDA(cudaStreamWaitEvent(c.aux[0], R.ev_z, 0));
-    prove_begin_on(c, pk, R.z.p, rr, ss);
+    proof_begin(c, P, R.z.p, rr, ss);
+    proof_accums(c, P, nullptr);
     // the uploaded assignment is valid for THIS proof only: shard_finish clears the flag, so a later call with
     // z == NULL outside a begin/finish window fails instead of silently proving a stale assignment
-    pk_bind_assignment_flag(pk, &R.z_valid);
+    P.assignment_flag = &R.z_valid;
   });
 }
 
@@ -438,8 +442,17 @@ b2z_status b2z_groth16_shard_finish(b2z_ctx* ctx, const b2z_pk* pk, uint64_t* d_
                                     const uint64_t* d_c, uint8_t* partial_out) {
   return guarded(ctx, [&](Ctx& c) {
     B2Z_REQUIRE(pk && d_a && d_b && d_c && partial_out, B2Z_EINVAL, "b2z_groth16_shard_finish: NULL argument");
-    prove_finish_on(c, pk, reinterpret_cast<FrEl*>(d_a), reinterpret_cast<const FrEl*>(d_b),
-                    reinterpret_cast<const FrEl*>(d_c), partial_out);
+    PkImpl& P = pk_of(c, pk, "b2z_groth16_shard_finish");
+    if (P.assignment_flag != nullptr) {
+      *P.assignment_flag = false;
+      P.assignment_flag = nullptr;
+    }
+    FrEl* a = reinterpret_cast<FrEl*>(d_a);
+    witness_map_quotient(&c, a, reinterpret_cast<const FrEl*>(d_b), reinterpret_cast<const FrEl*>(d_c), P.log_n,
+                         /*natural_out=*/false, c.stream);    // whole domain, every shard
+    proof_h_sort(c, P, a + P.h_lo, c.stream);
+    proof_h_finish(c, P);
+    proof_end(c, P, partial_out);
   });
 }
 
@@ -459,7 +472,7 @@ struct DistImpl {
   uint32_t rank = 0, world = 1, wbits = 0, log_n = 0;
   uint64_t m = 0;
   size_t nl = 0, z_bytes = 0, region_bytes = 0;
-  const b2z_pk* pk = nullptr;
+  PkImpl* pk = nullptr;
   b2z_r1cs* r1cs = nullptr;
   DevBuf<uint8_t> region;                 // [ z (m x 32 B) | X_a X_b X_c | Y_a Y_b Y_c ]  (n / W elements each)
   uint8_t* peer_region[8] = {};
@@ -511,7 +524,7 @@ bool shared_combine(void* shared_host, uint32_t rank, uint32_t world, uint32_t* 
   uint8_t* partials = static_cast<uint8_t*>(shared_host) + (size_t)world * kFlagStride * 4;
   if (my_partial != partials + (size_t)rank * kPartial) std::memcpy(partials + (size_t)rank * kPartial, my_partial, kPartial);
   if (!shared_barrier(flags, rank, world, epoch)) return false;
-  combine_partials_host(partials, world, proof_out);
+  combine_partials(partials, world, proof_out);
   return shared_barrier(flags, rank, world, epoch);
 }
 }  // namespace
@@ -539,20 +552,18 @@ b2z_status b2z_dist_create(b2z_ctx* ctx, const b2z_pk* pk, b2z_r1cs* r, uint32_t
     B2Z_REQUIRE((world == 2 || world == 4 || world == 8) && rank < world, B2Z_EINVAL,
                 "b2z_dist_create: world must be 2, 4 or 8 and rank < world");
     R1csImpl& R = r1cs_of(c, r, "b2z_dist_create");
-    B2Z_REQUIRE(pk_matches(pk, R.log_n, R.m, R.l), B2Z_EINVAL, "b2z_dist_create: key and matrices disagree");
+    PkImpl& P = pk_for(c, pk, R, "b2z_dist_create");
     uint32_t wbits = 0;
     while ((1u << wbits) < world) wbits++;
     B2Z_REQUIRE(ntt_dist_supported(R.log_n, wbits), B2Z_ESIZE,
                 "b2z_dist_create: domain too small for a tile-sharded witness map (use b2z_groth16_prove_partial_r1cs)");
-    uint32_t h_lo = 0;
-    const uint32_t hn = pk_h_chunk(pk, &h_lo);
     const size_t n = (size_t)1 << R.log_n;
-    B2Z_REQUIRE(hn == n / world && h_lo == n / world * rank, B2Z_EINVAL,
+    B2Z_REQUIRE(P.hn == n / world && P.h_lo == n / world * rank, B2Z_EINVAL,
                 "b2z_dist_create: the key must be shard `rank` of `world` (b2z_pk_upload_shard)");
     std::unique_ptr<b2z_dist> d(new b2z_dist());
     DistImpl& D = d->impl;
     D.owner = &c; D.rank = rank; D.world = world; D.wbits = wbits; D.log_n = R.log_n; D.m = R.m;
-    D.pk = pk; D.r1cs = r;
+    D.pk = &P; D.r1cs = r;
     D.nl = n / world;
     D.z_bytes = ((R.m * sizeof(FrEl) + 255) / 256) * 256;
     D.region_bytes = D.z_bytes + 6 * D.nl * sizeof(FrEl);
@@ -643,6 +654,7 @@ b2z_status b2z_dist_prove(b2z_ctx* ctx, b2z_dist* d, const uint64_t* z, int z_is
     for (uint32_t p = 0; p < D.world; p++)
       B2Z_REQUIRE(D.peer_region[p] != nullptr, B2Z_EINVAL, "b2z_dist_prove: not every peer is attached (b2z_dist_attach)");
     R1csImpl& R = r1cs_of(c, D.r1cs, "b2z_dist_prove");
+    PkImpl& P = *D.pk;
     cudaStream_t ws = D.wm_st;
     // ---- the assignment: every rank moves 1 / W of it over PCIe and hands the slice to its peers over NVLink
     if (z_is_full_device_copy) {
@@ -664,7 +676,7 @@ b2z_status b2z_dist_prove(b2z_ctx* ctx, b2z_dist* d, const uint64_t* z, int z_is
     B2Z_CUDA(cudaEventRecord(R.ev_z, ws));
     // ---- light z-only work on the auxiliary streams: scalar conversion and the four sorts
     B2Z_CUDA(cudaStreamWaitEvent(c.aux[0], R.ev_z, 0));
-    prove_begin_sorts_on(c, D.pk, D.z(), rr, ss);
+    proof_begin(c, P, D.z(), rr, ss);
     // ---- tile-sharded witness map on its own high-priority stream
     NttDist& nd = D.nd;
     nd.wbits = D.wbits; nd.me = D.rank;
@@ -688,9 +700,12 @@ b2z_status b2z_dist_prove(b2z_ctx* ctx, b2z_dist* d, const uint64_t* z, int z_is
     dist_barrier(D, "witness-map step 3");
     wm_dist_step4(&c, nd, D.log_n, ws);
     B2Z_CUDA(cudaEventRecord(D.ev_ready, ws));
-    prove_dist_h_sort_on(c, D.pk, nd.y[0], ws);           // hides under the z-only accumulations
-    // ---- the five accumulations back to back, host epilogue of this shard
-    prove_dist_finish_on(c, D.pk, D.ev_ready, ws, D.partials + (size_t)D.rank * kPartial);
+    proof_h_sort(c, P, nd.y[0], ws);                       // hides under the z-only accumulations
+    // ---- the five accumulations back to back once the transforms are done (they need the SMs the accumulations
+    // fill), H on ws after its sort; host epilogue of this shard
+    proof_accums(c, P, D.ev_ready);
+    proof_h_finish(c, P);
+    proof_end(c, P, D.partials + (size_t)D.rank * kPartial);
     // ---- partial sums meet in the shared host memory; every rank combines
     if (!shared_combine(D.flags, D.rank, D.world, &D.epoch, D.partials + (size_t)D.rank * kPartial, proof_out))
       throw StatusError{B2Z_ECUDA, "b2z_dist_prove: a peer rank did not reach the barrier after the accumulations"};

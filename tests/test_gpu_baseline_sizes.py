@@ -17,6 +17,7 @@ import numpy as np
 import pytest
 
 from oracle import bls12_381 as O
+from helpers import dist_prove_virtual_ranks
 
 pytestmark = pytest.mark.gpu
 R = O.R_MOD
@@ -295,51 +296,6 @@ def test_fibonacci_route_seed_42_on_the_gpu(b2z, ctx, codec, circuits):
 
 
 # ------------------------------------------------------------------------------- tile-sharded prover (b2z_dist_*)
-def _dist_prove_virtual_ranks(b2z, codec, cm0, pk0, z, r, s, world, resident=False, proofs=1):
-    """`world` ranks as host threads, each with its own context / key shard / matrices on THIS GPU: the same code
-    path as one rank per GPU (peers attached by device pointer instead of IPC handle)."""
-    import threading
-    shared = np.zeros(b2z.DistributedProver.shared_bytes(world), dtype=np.uint8)
-    barrier = threading.Barrier(world)
-    exported, results, errors = [None] * world, [None] * world, []
-
-    def worker(rank):
-        try:
-            rctx = b2z.Context(0)
-            spk = b2z.ProvingKey(pk0.num_variables, pk0.num_instance, pk0.domain_size, pk0.a_query, pk0.b_g1_query,
-                                 pk0.b_g2_query, pk0.h_query, pk0.l_query, pk0.alpha_g1, pk0.beta_g1, pk0.delta_g1,
-                                 pk0.beta_g2, pk0.delta_g2)
-            rcm = b2z.ConstraintMatrices(cm0.num_instance_variables, cm0.num_witness_variables, cm0.num_constraints,
-                                         cm0.a, cm0.b, cm0.c)
-            dp = b2z.DistributedProver(rctx, spk, rcm, rank, world, shared)
-            exported[rank] = dp.export()[1]
-            barrier.wait()
-            for p in range(world):
-                if p != rank:
-                    dp.attach(p, device_ptr=exported[p])
-            barrier.wait()
-            zarg = z
-            if resident:
-                import torch
-                zt = torch.from_numpy(z.view(np.int64).copy()).cuda()
-                torch.cuda.synchronize()
-                zarg = int(zt.data_ptr())
-            results[rank] = [dp.prove(zarg, r + i, s + i, resident=resident) for i in range(proofs)]
-            barrier.wait()
-            dp.close(); spk.free(); rcm.free(); rctx.close()
-        except Exception as e:                    # surfaced below; release the others from the barrier
-            errors.append((rank, repr(e)))
-            barrier.abort()
-
-    threads = [threading.Thread(target=worker, args=(k,)) for k in range(world)]
-    for t in threads:
-        t.start()
-    for t in threads:
-        t.join()
-    assert not errors, errors
-    return results
-
-
 @pytest.mark.parametrize("size,world", [(8, 2), (16, 4), (16, 8)])
 def test_tile_sharded_prover_equals_single_gpu(b2z, ctx, codec, size, world):
     """ONE proof by `world` ranks with the witness map tile-sharded (layout changes fused into the pass stores, peers
@@ -354,10 +310,10 @@ def test_tile_sharded_prover_equals_single_gpu(b2z, ctx, codec, size, world):
     r, s = 1234567, 7654321
     want = [b2z.Groth16.create_proof_with_matrices(ctx, pk, cm, z, r + i, s + i) for i in range(2)]
     pk.free()
-    got = _dist_prove_virtual_ranks(b2z, codec, cm, pk, z, r, s, world, proofs=2)
+    got = dist_prove_virtual_ranks(b2z, codec, cm, pk, z, r, s, world, proofs=2)
     for rank in range(world):
         assert got[rank] == want, "rank %d" % rank
-    got = _dist_prove_virtual_ranks(b2z, codec, cm, pk, z, r, s, world, resident=True)
+    got = dist_prove_virtual_ranks(b2z, codec, cm, pk, z, r, s, world, resident=True)
     assert all(g == want[:1] for g in got)
     cm.free()
 
@@ -368,7 +324,7 @@ def test_tile_sharded_prover_2p22(b2z, ctx, codec, c5):
     r, s = 99, 101
     want = b2z.Groth16.create_proof_with_matrices(ctx, pk, cm, z, r, s)
     pk.free()
-    got = _dist_prove_virtual_ranks(b2z, codec, cm, pk, z, r, s, 8)
+    got = dist_prove_virtual_ranks(b2z, codec, cm, pk, z, r, s, 8)
     assert all(g == [want] for g in got)
 
 

@@ -38,13 +38,9 @@ import numpy as np
 import pytest
 
 from oracle import bls12_381 as O
-from helpers import scalar_mix
+from helpers import NAMES, R, KnownKey, add_point, c_point, check_partial, decode_partial, dot_mod_r, point, rand_k, scalar_mix
 
 pytestmark = pytest.mark.gpu
-R, Q = O.R_MOD, O.Q_MOD
-FR_RINV = pow(O.FR_MONT_R, -1, R)
-FQ_RINV = pow(O.FQ_MONT_R, -1, Q)
-NAMES = ("A", "sA", "rB1", "L", "H", "B")
 
 
 @pytest.fixture(scope="module")
@@ -80,33 +76,12 @@ def _assert_precomputed(b2z, m, l, log_n):
 
 
 # ------------------------------------------------------------------------------- scalars and exact sums
-def _rand_k(rs, n):
-    """n uniform multipliers < 2^254 as (n, 4) canonical limbs."""
-    a = rs.randint(0, 1 << 32, size=(n, 8), dtype=np.uint64)
-    a = (a[:, 0::2] | (a[:, 1::2] << np.uint64(32))).astype(np.uint64)
-    a[:, 3] &= np.uint64((1 << 62) - 1)
-    return np.ascontiguousarray(a)
-
-
 def _limb(v):
     return np.frombuffer((v % R).to_bytes(32, "little"), dtype=np.uint64)
 
 
 def _int(row):
     return int.from_bytes(np.ascontiguousarray(row).tobytes(), "little")
-
-
-def _dot(x, y):
-    """sum x_i y_i mod r of two (n, 4) limb arrays, exactly.  16-bit pieces make products < 2^32; 2^20 rows per
-    float64 matrix product keep every partial sum an integer below 2^52, so the products are exact."""
-    acc = 0
-    step = 1 << 20
-    for s in range(0, x.shape[0], step):
-        a = np.ascontiguousarray(x[s:s + step]).view(np.uint16).astype(np.float64)
-        b = np.ascontiguousarray(y[s:s + step]).view(np.uint16).astype(np.float64)
-        M = a.T @ b
-        acc += sum(int(M[p, q]) << (16 * (p + q)) for p in range(16) for q in range(16))
-    return acc % R
 
 
 def _boundary(rnd, cs, count):
@@ -132,109 +107,6 @@ def _z_mix(codec, kind, m, cs, seed):
     u = min(m, 1 << 15)
     vals = _boundary(rnd, cs, u) if kind == "boundary" else scalar_mix(rnd, u, "zero" if kind == "sparse" else kind)
     return (np.resize(codec.fr_to_bigint_limbs(vals), (m, 4)), np.resize(codec.fr_to_mont_limbs(vals), (m, 4)))
-
-
-# ------------------------------------------------------------------------------- partial-sum decoder
-def _fq(raw, i):
-    """Fq element i of a device point: 12 x u32 Montgomery limbs, lazily reduced (< 2q)."""
-    return int.from_bytes(raw[48 * i:48 * i + 48], "little") % Q * FQ_RINV % Q
-
-
-def _decode_g1(raw):
-    x, y, zz, zzz = (_fq(raw, i) for i in range(4))
-    if zz == 0:
-        return None
-    return x * pow(zz, -1, Q) % Q, y * pow(zzz, -1, Q) % Q
-
-
-def _decode_g2(raw):
-    F = O.Fq2Ops
-    f = [_fq(raw, i) for i in range(8)]
-    x, y, zz, zzz = (f[0], f[1]), (f[2], f[3]), (f[4], f[5]), (f[6], f[7])
-    if F.is_zero(zz):
-        return None
-    return F.mul(x, F.inv(zz)), F.mul(y, F.inv(zzz))
-
-
-def decode_partial(b2z, partial):
-    """B2Z_PARTIAL_BYTES -> {name: affine oracle point | None}: five G1 XYZZ points, then one G2."""
-    assert len(partial) == b2z._ffi.PARTIAL_BYTES == 5 * 192 + 384
-    out = {n: _decode_g1(partial[192 * i:192 * (i + 1)]) for i, n in enumerate(NAMES[:5])}
-    out["B"] = _decode_g2(partial[5 * 192:])
-    return out
-
-
-def _c_point(got):
-    C = None
-    for n in ("sA", "rB1", "L", "H"):
-        C = O.G1.add(C, got[n])
-    return C
-
-
-def _point(name, k):
-    """k G1, or k G2 for the B sum."""
-    return O.G2.mul(O.G2_GEN, k) if name == "B" else O.G1.mul(O.G1_GEN, k)
-
-
-def _add(name, p, q):
-    return O.G2.add(p, q) if name == "B" else O.G1.add(p, q)
-
-
-def check_partial(b2z, partial, want):
-    """Decode, check the decoder against b2z_groth16_combine, and return the names of the sums that differ from
-    the multipliers in `want`."""
-    got = decode_partial(b2z, partial)
-    assert b2z.Groth16.combine([partial]) == O.proof_serialize_compressed(got["A"], got["B"], _c_point(got)), \
-        "partial-sum decoder disagrees with b2z_groth16_combine"
-    return [n for n in NAMES if got[n] != _point(n, want[n])]
-
-
-# ------------------------------------------------------------------------------- keys of known multiples
-class KnownKey:
-    """A proving key with num_variables m, num_instance l and domain 2^log_n whose points are k G for multipliers
-    drawn here; `edit(key)` may change the multipliers (self.k, canonical limbs) before the points are made."""
-
-    def __init__(self, b2z, ctx, m, l, log_n, seed, edit=None):
-        rs = np.random.RandomState(seed)
-        self.m, self.l, self.log_n, self.n = m, l, log_n, 1 << log_n
-        self.k = {"a": _rand_k(rs, m), "b1": _rand_k(rs, m), "b2": _rand_k(rs, m), "l": _rand_k(rs, m - l),
-                  "h": _rand_k(rs, self.n - 1)}
-        rnd = random.Random(seed)
-        self.alpha, self.beta1, self.delta1, self.beta2, self.delta2 = (rnd.randrange(1, R) for _ in range(5))
-        if edit is not None:
-            edit(self)
-        g1 = lambda ks: b2z.FixedBase.msm_g1(ctx, ks)
-        g2 = lambda ks: b2z.FixedBase.msm_g2(ctx, ks)
-        big = b2z.codec.fr_to_bigint_limbs
-        s1, _ = g1(big([self.alpha, self.beta1, self.delta1]))
-        s2, _ = g2(big([self.beta2, self.delta2]))
-        self.pk = b2z.ProvingKey(m, l, self.n, g1(self.k["a"]), g1(self.k["b1"]), g2(self.k["b2"]), g1(self.k["h"]),
-                                 g1(self.k["l"]), s1[0], s1[1], s1[2], s2[0], s2[1])
-        rs2 = np.random.RandomState(seed + 1)
-        self.abc = tuple(_rand_k(rs2, self.n) for _ in range(3))     # arbitrary: prove_partial needs no satisfied system
-        self.h_k = None
-
-    def copy_pk(self, b2z):
-        p = self.pk
-        return b2z.ProvingKey(p.num_variables, p.num_instance, p.domain_size, p.a_query, p.b_g1_query, p.b_g2_query,
-                              p.h_query, p.l_query, p.alpha_g1, p.beta_g1, p.delta_g1, p.beta_g2, p.delta_g2)
-
-    def h_multiplier(self, cpu_oracle):
-        """sum_{j<n-1} h_j eta_j with h the oracle's witness map (natural order, Montgomery limbs)."""
-        if self.h_k is None:
-            self.h_k = 0 if self.n == 1 else _dot(cpu_oracle.witness_map(*self.abc)[:self.n - 1], self.k["h"]) * FR_RINV % R
-        return self.h_k
-
-    def sums(self, cpu_oracle, zc, r, s):
-        A = (_dot(zc, self.k["a"]) + self.alpha + r * self.delta1) % R
-        B1 = (_dot(zc, self.k["b1"]) + self.beta1 + s * self.delta1) % R
-        return {"A": A, "sA": s * A % R, "rB1": r * B1 % R,
-                "L": (_dot(zc[self.l:], self.k["l"]) - r * s * self.delta1) % R,
-                "H": self.h_multiplier(cpu_oracle),
-                "B": (_dot(zc, self.k["b2"]) + self.beta2 + s * self.delta2) % R}
-
-    def prove(self, b2z, ctx, pk, zm, r, s):
-        return b2z.Groth16.create_proof_partial(ctx, pk, *self.abc, zm, r, s)
 
 
 X, Y = 0x1b2c3d4e5f60718293a4b5c6d7e8f90a1b2c3d4e5f6071829, 0x5a4b3c2d1e0f1a2b3c4d5e6f708192a3b4c5d6e7f8091a2b
@@ -408,10 +280,10 @@ def test_shard_partials_sum_to_whole_key(b2z, ctx, codec, cpu_oracle, layout):
             pk.free()
         got = decode_partial(b2z, parts[-1])
         for n in NAMES:
-            total[n] = _add(n, total[n], got[n])
-    assert b2z.Groth16.combine(parts) == O.proof_serialize_compressed(total["A"], total["B"], _c_point(total)), \
+            total[n] = add_point(n, total[n], got[n])
+    assert b2z.Groth16.combine(parts) == O.proof_serialize_compressed(total["A"], total["B"], c_point(total)), \
         "partial-sum decoder disagrees with b2z_groth16_combine"
-    bad = [n for n in NAMES if total[n] != _point(n, want[n])]
+    bad = [n for n in NAMES if total[n] != point(n, want[n])]
     assert not bad, "%s: %s mismatch" % (layout, "/".join(bad))
 
 
@@ -425,7 +297,7 @@ def test_generic_msm_window_sizes(b2z, ctx, codec, group, c, end):
     n = (1 << (c + 3)) + 5 if end == "bottom" else 1 << (c + 4)
     assert _c_of(b2z, n, False) == c
     rs = np.random.RandomState(5000 + 100 * group + c)
-    ks = _rand_k(rs, n)
+    ks = rand_k(rs, n)
     curve = O.G1 if group == 1 else O.G2
     bases, inf = (b2z.FixedBase.msm_g1 if group == 1 else b2z.FixedBase.msm_g2)(ctx, ks)
     msm = b2z.VariableBaseMSM.msm_bigint_g1 if group == 1 else b2z.VariableBaseMSM.msm_bigint_g2
@@ -436,4 +308,4 @@ def test_generic_msm_window_sizes(b2z, ctx, codec, group, c, end):
         assert any(_digits(b2z, v, c)[-1] for v in vals[:64]), "no scalar reaches the top window"
         sc = np.resize(codec.fr_to_bigint_limbs(vals), (n, 4))
         got = curve.to_affine(proj(msm(ctx, bases, sc, inf)))
-        assert got == curve.mul(curve.gen, _dot(ks, sc)), "G%d c=%d n=%d %s scalars" % (group, c, n, kind)
+        assert got == curve.mul(curve.gen, dot_mod_r(ks, sc)), "G%d c=%d n=%d %s scalars" % (group, c, n, kind)

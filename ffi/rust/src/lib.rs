@@ -69,6 +69,8 @@ pub mod sys {
         pub fn b2z_ctx_destroy(ctx: *mut b2z_ctx);
         pub fn b2z_groth16_setup(ctx: *mut b2z_ctx, r1cs: *mut b2z_r1cs, desc: *const b2z_setup_desc,
                                  pk_out: *mut *mut b2z_pk, vk_out: *mut b2z_vk_out) -> i32;
+        pub fn b2z_groth16_setup_shard(ctx: *mut b2z_ctx, r1cs: *mut b2z_r1cs, desc: *const b2z_setup_desc, rank: u32,
+                                       world: u32, pk_out: *mut *mut b2z_pk, vk_out: *mut b2z_vk_out) -> i32;
         pub fn b2z_last_error(ctx: *const b2z_ctx) -> *const c_char;
         pub fn b2z_ntt_fr(ctx: *mut b2z_ctx, data: *mut u64, log_n: u32, inverse: i32, coset_gen: *const u64) -> i32;
         pub fn b2z_witness_map(ctx: *mut b2z_ctx, a: *const u64, b: *const u64, c: *const u64, log_n: u32, h: *mut u64) -> i32;
@@ -219,6 +221,15 @@ impl<'c> DeviceKey<'c> {
     /// verifying key equal what `Groth16::setup` returns for the same rng.  `m`: the circuit's matrices on `ctx`.
     pub fn setup<R: RngCore>(ctx: &'c Context, m: &DeviceMatrices<'c>, num_constraints: usize, num_instance: usize,
                              rng: &mut R) -> Result<(Self, VerifyingKey<Bls12_381>), SynthesisError> {
+        Self::setup_shard(ctx, m, num_constraints, num_instance, 0, 1, rng)
+    }
+    /// The same setup straight into shard `rank` of `world` of the key (b2z_groth16_setup_shard), the shard that
+    /// b2z_pk_upload_shard makes of the whole key: each GPU of a multi-GPU box calls this with an rng seeded alike, so
+    /// every rank makes the same draws, and gets its own key shard for the tile-sharded prover and the whole
+    /// verifying key.  world == 1: the whole key, as `setup`.
+    pub fn setup_shard<R: RngCore>(ctx: &'c Context, m: &DeviceMatrices<'c>, num_constraints: usize,
+                                   num_instance: usize, rank: u32, world: u32, rng: &mut R)
+                                   -> Result<(Self, VerifyingKey<Bls12_381>), SynthesisError> {
         let domain = ark_poly::Radix2EvaluationDomain::<Fr>::new(num_constraints + num_instance)
             .ok_or(SynthesisError::PolynomialDegreeTooLarge)?;
         let (alpha, beta, gamma, delta) = (Fr::rand(rng), Fr::rand(rng), Fr::rand(rng), Fr::rand(rng));
@@ -242,7 +253,7 @@ impl<'c> DeviceKey<'c> {
             gamma_abc_g1: gabc.as_mut_ptr(), gamma_abc_inf: gabc_inf.as_mut_ptr(),
         };
         let mut raw = ptr::null_mut();
-        status(ctx.raw, unsafe { b2z_groth16_setup(ctx.raw, m.raw, &desc, &mut raw, &mut vk) })?;
+        status(ctx.raw, unsafe { b2z_groth16_setup_shard(ctx.raw, m.raw, &desc, rank, world, &mut raw, &mut vk) })?;
         let g1_of = |l: &[u64], inf: bool| -> G1Affine {
             if inf { return G1Affine::identity(); }
             G1Affine::new_unchecked(unpack_fq(&l[0..6]), unpack_fq(&l[6..12]))

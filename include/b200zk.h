@@ -225,6 +225,22 @@ typedef struct b2z_vk_out {        /* filled by the call */
 } b2z_vk_out;
 B2Z_API b2z_status b2z_groth16_setup(b2z_ctx* ctx, b2z_r1cs* r1cs, const b2z_setup_desc* desc,
                                      b2z_pk** pk_out, b2z_vk_out* vk_out);
+/* The same setup straight into shard `rank` of `world`: each rank does only its own shard's fixed-base
+ * multiplications and window copies, and no query point leaves device memory.  Every rank passes the same desc
+ * and the same matrices (uploaded through its own context).
+ *  - *pk_out equals what b2z_pk_upload_shard(rank, world) makes from the arrays that b2z_pk_download returns for
+ *    b2z_groth16_setup's key, for the same desc and matrices.  Same sharding rule: variables in blocks of 64,
+ *    block-cyclic over the ranks; contiguous ranges instead when num_instance > 64; h positions in the contiguous
+ *    chunk [n rank/world, n (rank+1)/world) of the bit-reversed order; the alpha/beta/delta terms on rank 0 only;
+ *    precomputed window copies when 1/world of a whole key's copies fit in half the free device memory, decided
+ *    before the call's own allocations.  The shard is ready for b2z_groth16_prove_partial[_r1cs],
+ *    b2z_groth16_shard_* and b2z_dist_create.
+ *  - vk_out holds the full verifying key on every rank, identical across ranks.
+ *  - world == 1 gives the whole key: downloadable, and byte-equal to b2z_groth16_setup's key.
+ *  - rank >= world or world == 0: B2Z_EINVAL and *pk_out = NULL.  All of b2z_groth16_setup's checks apply unchanged
+ *    and run on the host before any GPU work.  b2z_pk_download on a shard returns B2Z_EINVAL.                     */
+B2Z_API b2z_status b2z_groth16_setup_shard(b2z_ctx* ctx, b2z_r1cs* r1cs, const b2z_setup_desc* desc, uint32_t rank,
+                                           uint32_t world, b2z_pk** pk_out, b2z_vk_out* vk_out);
 /* A whole key (b2z_pk_upload or b2z_groth16_setup) back in the b2z_pk_desc layout: h_query in natural order, n - 1
  * points.  The arrays are caller-allocated with b2z_pk_desc's sizes (h: NULL when n = 1, l: NULL when m = l); the
  * counts and the five single points are filled by the call.  A shard returns B2Z_EINVAL.  For callers that persist a

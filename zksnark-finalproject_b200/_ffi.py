@@ -93,6 +93,8 @@ SIGNATURES = {
     "b2z_fixed_base_mul_g1": (ctypes.c_int32, [vp, vp, ctypes.c_uint64, vp, vp]),
     "b2z_fixed_base_mul_g2": (ctypes.c_int32, [vp, vp, ctypes.c_uint64, vp, vp]),
     "b2z_groth16_setup": (ctypes.c_int32, [vp, vp, ctypes.POINTER(SetupDesc), ctypes.POINTER(vp), ctypes.POINTER(VkOut)]),
+    "b2z_groth16_setup_shard": (ctypes.c_int32, [vp, vp, ctypes.POINTER(SetupDesc), ctypes.c_uint32, ctypes.c_uint32,
+                                                 ctypes.POINTER(vp), ctypes.POINTER(VkOut)]),
     "b2z_pk_download": (ctypes.c_int32, [vp, vp, ctypes.POINTER(PkArrays)]),
     "b2z_profile_enable": (ctypes.c_int32, [vp, ctypes.c_int]),
     "b2z_profile_read": (ctypes.c_int32, [vp, vp, vp, vp, ctypes.c_int]),

@@ -51,12 +51,6 @@ __global__ void permute_bitrev_g1_kernel(const G1::Affine* __restrict__ src, con
   dst_flags[p] = inf ? 1u : 0u;
 }
 
-constexpr uint32_t kCycBlock = 64;   // variables per block of the block-cyclic point sharding
-
-// local variable j of a block-cyclic shard -> global variable index
-__host__ __device__ inline uint64_t cyc_global(uint64_t j, uint32_t rank, uint32_t world) {
-  return ((j / kCycBlock) * world + rank) * kCycBlock + (j % kCycBlock);
-}
 // zc[j] = canonical integer of z[global(j)]: this shard's MSM scalars
 __global__ void fr_from_mont_cyclic_kernel(const FrEl* __restrict__ z, FrEl* zc, uint32_t count, uint32_t rank,
                                            uint32_t world) {
@@ -85,30 +79,6 @@ void stage_points(Affine* d_dst, std::vector<uint32_t>& words, uint64_t at, cons
   if (inf != nullptr)
     for (uint64_t i = 0; i < count; i++)
       if ((inf[i >> 3] >> (i & 7)) & 1) words[(at + i) >> 5] |= 1u << ((at + i) & 31);
-}
-
-// `num` / `den` of the key's precomputed window copies fit in half the free device memory
-bool pk_precompute_fits_slice(uint32_t log_n, uint64_t m, uint64_t l, uint32_t num, uint32_t den) {
-  auto cost = [](uint64_t n, size_t pt) {
-    if (n == 0) return (size_t)0;
-    const uint32_t c = msm_pick_c(n, true);
-    return (size_t)n * pt * msm_windows(c);
-  };
-  const uint64_t n = 1ull << log_n;
-  const size_t bytes = 2 * cost(m + 2, 96) + cost(m - l + 1, 96) + cost(m + 2, 192) + cost(n, 96);
-  size_t free_b = 0, total_b = 0;
-  B2Z_CUDA(cudaMemGetInfo(&free_b, &total_b));
-  return bytes / den * num < free_b / 2;
-}
-
-// the sizes of a whole key
-void pk_init_whole(Ctx& c, PkImpl& P, uint32_t log_n, uint64_t m, uint64_t l) {
-  P.owner = &c;
-  P.log_n = log_n;
-  P.m = m;
-  P.l = l;
-  P.lo = 0; P.ma = (uint32_t)m; P.l_skip = (uint32_t)l; P.ml = (uint32_t)(m - l);
-  P.h_lo = 0; P.hn = 1u << log_n; P.with_vk = 1;
 }
 
 // per-proof scratch, the proof's sums (arena slot, stream, tail offset, result) and events; after the shard fields
@@ -408,16 +378,30 @@ PkImpl& pk_of(Ctx& c, const b2z_pk* pk, const char* who) {
                                                      "belongs to one context; upload one copy per context)"};
   return P;
 }
-bool pk_precompute_fits(uint32_t log_n, uint64_t m, uint64_t l) { return pk_precompute_fits_slice(log_n, m, l, 1, 1); }
-b2z_pk* pk_from_device_sets(Ctx& c, uint32_t log_n, uint64_t m, uint64_t l, const PkDeviceSets& S, bool pre) {
+// `num` / `den` of the key's precomputed window copies fit in half the free device memory
+bool pk_precompute_fits_slice(uint32_t log_n, uint64_t m, uint64_t l, uint32_t num, uint32_t den) {
+  auto cost = [](uint64_t n, size_t pt) {
+    if (n == 0) return (size_t)0;
+    const uint32_t c = msm_pick_c(n, true);
+    return (size_t)n * pt * msm_windows(c);
+  };
+  const uint64_t n = 1ull << log_n;
+  const size_t bytes = 2 * cost(m + 2, 96) + cost(m - l + 1, 96) + cost(m + 2, 192) + cost(n, 96);
+  size_t free_b = 0, total_b = 0;
+  B2Z_CUDA(cudaMemGetInfo(&free_b, &total_b));
+  return bytes / den * num < free_b / 2;
+}
+b2z_pk* pk_from_device_sets(Ctx& c, const PkShard& shard, const PkDeviceSets& S, bool pre) {
   std::unique_ptr<b2z_pk> pk(new b2z_pk());
   PkImpl& P = pk->impl;
-  pk_init_whole(c, P, log_n, m, l);
+  P.owner = &c;
+  static_cast<PkShard&>(P) = shard;
+  const uint32_t vk_terms = P.with_vk ? 2 : 0;   // alpha/beta/delta (a, b1, b2) and delta (l): shard 0 only
   cudaStream_t st = c.stream;
-  msm_bases_build<G1>(&c, P.a_set, S.a, S.a_words, (uint32_t)m + 2, pre, 0, st);
-  msm_bases_build<G1>(&c, P.b1_set, S.b1, S.b1_words, (uint32_t)m + 2, pre, 0, st);
-  msm_bases_build<G1>(&c, P.l_set, S.l, S.l_words, (uint32_t)(m - l) + 1, pre, 0, st);
-  msm_bases_build<G2>(&c, P.g2, S.b2, S.b2_words, (uint32_t)m + 2, pre, 0, st);
+  msm_bases_build<G1>(&c, P.a_set, S.a, S.a_words, P.ma + vk_terms, pre, 0, st);
+  msm_bases_build<G1>(&c, P.b1_set, S.b1, S.b1_words, P.ma + vk_terms, pre, 0, st);
+  msm_bases_build<G1>(&c, P.l_set, S.l, S.l_words, P.ml + vk_terms / 2, pre, 0, st);
+  msm_bases_build<G2>(&c, P.g2, S.b2, S.b2_words, P.ma + vk_terms, pre, 0, st);
   msm_bases_build<G1>(&c, P.h, S.h, S.h_words, P.hn, pre, 0, st);
   B2Z_CUDA(cudaStreamSynchronize(st));
   pk_alloc_scratch(c, P);
@@ -447,8 +431,7 @@ b2z_status b2z_fixed_base_mul_g2(b2z_ctx* ctx, const uint64_t* scalars, uint64_t
   return guarded(ctx, [&](Ctx& c) { fixed_base_entry<G2>(c, scalars, n, out_points, out_inf); });
 }
 
-// from / to / den: contiguous slice of the variables AND of the h positions.  cyc_world > 0: the h positions still
-// follow from / to / den, the variables are the block-cyclic subset of rank cyc_rank of cyc_world.
+// from / to / den, cyc_rank / cyc_world: the shard of pk_shard (prove_internal.hpp), assembled from the caller's arrays
 static b2z_status pk_upload_impl(b2z_ctx* ctx, const b2z_pk_desc* d, uint32_t from, uint32_t to, uint32_t den,
                                  uint32_t cyc_rank, uint32_t cyc_world, b2z_pk** out) {
   if (out) *out = nullptr;
@@ -466,27 +449,8 @@ static b2z_status pk_upload_impl(b2z_ctx* ctx, const b2z_pk_desc* d, uint32_t fr
                 B2Z_EINVAL, "b2z_pk_upload: NULL query array");
     std::unique_ptr<b2z_pk> pk(new b2z_pk());
     PkImpl& P = pk->impl;
-    pk_init_whole(c, P, d->log_domain, m, l);
-    // the variables of this shard, in local order
-    if (cyc_world > 0 && l > kCycBlock) cyc_world = 0;   // the instance variables must sit in block 0
-    uint64_t lo = m * from / den, hi = m * to / den;
-    std::vector<uint32_t> ids;                           // cyclic mode only
-    if (cyc_world > 0) {
-      for (uint64_t b = cyc_rank; b * kCycBlock < m; b += cyc_world)
-        for (uint64_t i = b * kCycBlock; i < (b + 1) * kCycBlock && i < m; i++) ids.push_back((uint32_t)i);
-      P.cyc_world = cyc_world; P.cyc_rank = cyc_rank;
-      P.lo = 0; P.ma = (uint32_t)ids.size();
-      P.l_skip = cyc_rank == 0 ? (uint32_t)(l < P.ma ? l : P.ma) : 0;
-      lo = 0; hi = P.ma;
-    } else {
-      const uint64_t l_lo = lo > l ? lo : l;             // first witness variable in the slice
-      P.lo = (uint32_t)lo; P.ma = (uint32_t)(hi - lo);
-      P.l_skip = (uint32_t)((l_lo < hi ? l_lo : hi) - lo);
-    }
-    P.ml = P.ma - P.l_skip;
-    const uint64_t h_lo = n * from / den, h_hi = n * to / den;
-    P.h_lo = (uint32_t)h_lo; P.hn = (uint32_t)(h_hi - h_lo);
-    P.with_vk = from == 0 ? 1u : 0u;
+    P.owner = &c;
+    static_cast<PkShard&>(P) = pk_shard(d->log_domain, m, l, from, to, den, cyc_rank, cyc_world);
     cudaStream_t st = c.stream;
     const bool pre = pk_precompute_fits_slice(P.log_n, m, l, to - from, den);
     // `count` points of a query, starting at local variable `skip` of this shard, as one contiguous host array
@@ -500,15 +464,14 @@ static b2z_status pk_upload_impl(b2z_ctx* ctx, const b2z_pk_desc* d, uint32_t fr
     auto pick = [&](Picked& out, const uint64_t* query, const uint8_t* inf, uint32_t skip, uint32_t count, uint64_t shift,
                     uint32_t limbs) {
       if (count == 0 || query == nullptr) return;
-      auto var = [&](uint32_t j) { return cyc_world > 0 ? (uint64_t)ids[j] : lo + j; };
-      if (cyc_world == 0) {
-        out.pts = query + (size_t)limbs * (var(skip) - shift);
+      if (P.cyc_world == 0) {
+        out.pts = query + (size_t)limbs * (P.var(skip) - shift);
       } else {
         out.own_pts.resize((size_t)limbs * count);
         for (uint32_t j = 0; j < count;) {               // copy block by block
-          const uint64_t q = var(skip + j) - shift;
+          const uint64_t q = P.var(skip + j) - shift;
           uint32_t run = 1;
-          while (j + run < count && var(skip + j + run) - shift == q + run) run++;
+          while (j + run < count && P.var(skip + j + run) - shift == q + run) run++;
           std::memcpy(&out.own_pts[(size_t)limbs * j], query + (size_t)limbs * q, (size_t)limbs * 8 * run);
           j += run;
         }
@@ -517,7 +480,7 @@ static b2z_status pk_upload_impl(b2z_ctx* ctx, const b2z_pk_desc* d, uint32_t fr
       if (inf != nullptr) {
         out.own_inf.assign((count + 7) / 8 + 1, 0);
         for (uint32_t j = 0; j < count; j++) {
-          const uint64_t q = var(skip + j) - shift;
+          const uint64_t q = P.var(skip + j) - shift;
           if ((inf[q >> 3] >> (q & 7)) & 1) out.own_inf[j >> 3] |= (uint8_t)(1u << (j & 7));
         }
         out.inf = out.own_inf.data();
@@ -576,8 +539,8 @@ static b2z_status pk_upload_impl(b2z_ctx* ctx, const b2z_pk_desc* d, uint32_t fr
       permute_bitrev_g1_kernel<<<nblocks(n, 256), 256, 0, st>>>(src.p, src_inf.p, (uint32_t)(n - 1), P.log_n, dst.p,
                                                                 flags.p);
       B2Z_LAUNCHED(&c);
-      pack_flags_device(&c, flags.p + h_lo, P.hn, words.p, st);
-      msm_bases_build<G1>(&c, P.h, dst.p + h_lo, words.p, P.hn, pre, 0, st);
+      pack_flags_device(&c, flags.p + P.h_lo, P.hn, words.p, st);
+      msm_bases_build<G1>(&c, P.h, dst.p + P.h_lo, words.p, P.hn, pre, 0, st);
       B2Z_CUDA(cudaStreamSynchronize(st));
     }
     pk_alloc_scratch(c, P);

@@ -21,22 +21,79 @@ struct R1csView {
 };
 R1csView r1cs_view(Ctx& c, b2z_r1cs* r, const char* who);
 
-// A whole key's five base sets in device memory (points + identity bitmap words), the layout b2z_pk_upload assembles:
-// a, b1, b2: m + 2 points [query | alpha_1 delta_1] / [query | beta_1 delta_1] / [query | beta_2 delta_2];
-// l: m - l + 1 points [l_query | delta_1]; h: n points, h_query in bit-reversed order, position n - 1 the flagged identity.
+// ---------------------------------------------------------------------------
+// Proving key
+// ---------------------------------------------------------------------------
+constexpr uint32_t kCycBlock = 64;   // variables per block of the block-cyclic point sharding
+
+// local variable j of a block-cyclic shard -> global variable index
+__host__ __device__ inline uint64_t cyc_global(uint64_t j, uint32_t rank, uint32_t world) {
+  return ((j / kCycBlock) * world + rank) * kCycBlock + (j % kCycBlock);
+}
+
+// Which part of a key a handle holds: a whole key, or one shard of it.
+// shard: `ma` variables of the a/b queries -- either the contiguous range [lo, lo+ma) (cyc_world == 0) or,
+// block-cyclic, the blocks cyc_rank, cyc_rank + cyc_world, ... of kCycBlock variables (balanced whatever the
+// witness structure: Groth16 assignments have long stretches of small / Boolean values); the first l_skip of
+// them are instance variables (not in l_query), ml = ma - l_skip; bit-reversed h positions [h_lo, h_lo+hn);
+// alpha/beta/delta terms on shard 0 only
+struct PkShard {
+  uint32_t log_n = 0;
+  uint64_t m = 0, l = 0;
+  uint32_t lo = 0, ma = 0, l_skip = 0, ml = 0, h_lo = 0, hn = 0, with_vk = 1;
+  uint32_t cyc_world = 0, cyc_rank = 0;
+  // global index of the shard's local variable j
+  __host__ __device__ uint64_t var(uint64_t j) const { return cyc_world ? cyc_global(j, cyc_rank, cyc_world) : lo + j; }
+  // every variable, every h position and the alpha/beta/delta terms: not a shard
+  bool whole() const { return with_vk && cyc_world == 0 && lo == 0 && ma == m && hn == (1ull << log_n); }
+};
+
+// The sharding rule of every key handle (b2z_pk_upload / _slice / _shard, b2z_groth16_setup[_shard]): the slice
+// [from, to) of den.  Variables: the contiguous range [m from/den, m to/den), or, for cyc_world > 1, the block-cyclic
+// variables of rank cyc_rank -- contiguous after all when l > kCycBlock (the instance variables must sit in block 0).
+// h positions: [n from/den, n to/den) of the bit-reversed order.  The slice with from == 0 keeps alpha/beta/delta.
+inline PkShard pk_shard(uint32_t log_n, uint64_t m, uint64_t l, uint32_t from, uint32_t to, uint32_t den,
+                        uint32_t cyc_rank, uint32_t cyc_world) {
+  PkShard S;
+  S.log_n = log_n;
+  S.m = m;
+  S.l = l;
+  if (cyc_world > 1 && l <= kCycBlock) {
+    uint64_t ma = 0;
+    for (uint64_t b = cyc_rank; b * kCycBlock < m; b += cyc_world)
+      ma += m - b * kCycBlock < kCycBlock ? m - b * kCycBlock : kCycBlock;
+    S.cyc_world = cyc_world; S.cyc_rank = cyc_rank;
+    S.lo = 0; S.ma = (uint32_t)ma;
+    S.l_skip = cyc_rank == 0 ? (uint32_t)(l < ma ? l : ma) : 0;
+  } else {
+    const uint64_t lo = m * from / den, hi = m * to / den;
+    const uint64_t l_lo = lo > l ? lo : l;             // first witness variable in the slice
+    S.lo = (uint32_t)lo; S.ma = (uint32_t)(hi - lo);
+    S.l_skip = (uint32_t)((l_lo < hi ? l_lo : hi) - lo);
+  }
+  S.ml = S.ma - S.l_skip;
+  const uint64_t n = 1ull << log_n, h_lo = n * from / den, h_hi = n * to / den;
+  S.h_lo = (uint32_t)h_lo; S.hn = (uint32_t)(h_hi - h_lo);
+  S.with_vk = from == 0 ? 1u : 0u;
+  return S;
+}
+
+// A key's five base sets in device memory (points + identity bitmap words), the layout b2z_pk_upload assembles, for
+// the shard's variables and h positions; the alpha/beta/delta terms only when S.with_vk:
+// a, b1, b2: ma (+ 2) points [query | alpha_1 delta_1] / [query | beta_1 delta_1] / [query | beta_2 delta_2];
+// l: ml (+ 1) points [l_query | delta_1]; h: hn points of h_query in bit-reversed order, position n - 1 the flagged
+// identity.
 struct PkDeviceSets {
   const G1::Affine *a, *b1, *l, *h;
   const G2::Affine* b2;
   const uint32_t *a_words, *b1_words, *l_words, *h_words, *b2_words;
 };
-// b2z_pk_upload's rule for precomputed window copies: they fit in half the free device memory
-bool pk_precompute_fits(uint32_t log_n, uint64_t m, uint64_t l);
-// the key handle for those sets (copied; the caller keeps its buffers); `pre` from pk_precompute_fits
-b2z_pk* pk_from_device_sets(Ctx& c, uint32_t log_n, uint64_t m, uint64_t l, const PkDeviceSets& sets, bool pre);
+// b2z_pk_upload's rule for precomputed window copies: `num` / `den` of a whole key's copies fit in half the free
+// device memory (a shard of `world`: 1 / world)
+bool pk_precompute_fits_slice(uint32_t log_n, uint64_t m, uint64_t l, uint32_t num, uint32_t den);
+// the key handle of shard S for its sets (copied; the caller keeps its buffers); `pre` from pk_precompute_fits_slice
+b2z_pk* pk_from_device_sets(Ctx& c, const PkShard& S, const PkDeviceSets& sets, bool pre);
 
-// ---------------------------------------------------------------------------
-// Proving key
-// ---------------------------------------------------------------------------
 // The five MSMs of a proof, the G1 ones first.  (The partial sums leave in the order A | sA | rB1 | L | H | B,
 // B2Z_PARTIAL_BYTES.)
 enum Sum { SUM_A, SUM_B1, SUM_L, SUM_H, SUM_B, SUM_COUNT };
@@ -54,20 +111,11 @@ struct ProofSum {
   template <class C> typename C::Xyzz* result() const { return static_cast<typename C::Xyzz*>(d_result); }
 };
 
-struct PkImpl {
+struct PkImpl : PkShard {
   // A key handle holds per-proof scratch (below), so it belongs to exactly ONE context: the one it was
   // uploaded through.  Every entry point checks this and returns B2Z_EINVAL for a foreign context.
   const Ctx* owner = nullptr;
   bool* assignment_flag = nullptr;   // b2z_groth16_shard_begin .. shard_finish window (r1cs.cu)
-  uint32_t log_n = 0;
-  uint64_t m = 0, l = 0;
-  // shard: `ma` variables of the a/b queries -- either the contiguous range [lo, lo+ma) (cyc_world == 0) or,
-  // block-cyclic, the blocks cyc_rank, cyc_rank + cyc_world, ... of kCycBlock variables (balanced whatever the
-  // witness structure: Groth16 assignments have long stretches of small / Boolean values); the first l_skip of
-  // them are instance variables (not in l_query), ml = ma - l_skip; bit-reversed h positions [h_lo, h_lo+hn);
-  // alpha/beta/delta terms on shard 0 only
-  uint32_t lo = 0, ma = 0, l_skip = 0, ml = 0, h_lo = 0, hn = 0, with_vk = 1;
-  uint32_t cyc_world = 0, cyc_rank = 0;
   MsmBases<G1> a_set;          // [a_query  | alpha_1 delta_1]
   MsmBases<G1> b1_set;         // [b_g1     | beta_1  delta_1]
   MsmBases<G1> l_set;          // [l_query  | delta_1]
@@ -83,8 +131,6 @@ struct PkImpl {
   FrEl r_c, s_c;                  // the proof's r, s as canonical integers (proof_begin -> proof_end)
   cudaEvent_t ev_z = nullptr;
   cudaEvent_t ev_wm = nullptr;       // witness-map transforms of the proof in flight are done (gates the first accumulation)
-  // every variable, every h position and the alpha/beta/delta terms: not a shard
-  bool whole() const { return with_vk && cyc_world == 0 && lo == 0 && ma == m && hn == (1ull << log_n); }
   ~PkImpl() {
     if (h_out) cudaFreeHost(h_out);
     if (h_planes) cudaFreeHost(h_planes);

@@ -11,6 +11,11 @@
 // Everything stays in device memory: the scalars go to the fixed-base multiplication as canonical integers, the h
 // scalars straight to their bit-reversed position of the prover's n-padded H set, and the point sets to the key
 // assembly that b2z_pk_upload uses (prove.cu: pk_from_device_sets).  Only the verifying key comes back to the host.
+//
+// One path for the whole key and for shard `rank` of `world` (b2z_groth16_setup_shard; the whole key is shard 0 of 1):
+// the Lagrange coefficients and the QAP evaluation are computed for every variable on every rank (a few ms at 2^22),
+// the scalars, the fixed-base multiplications and the window copies only for the shard's variables and h positions
+// (pk_shard, the rule of b2z_pk_upload_shard), the verifying key whole on every rank.
 #include <cstring>
 
 #include "api_glue.hpp"
@@ -198,32 +203,43 @@ void qap_eval(Ctx& c, const CsrDev& M, uint32_t nrows, uint32_t ncols, const FrE
   B2Z_CUDA(cudaStreamSynchronize(st));   // the scratch is freed on return
 }
 
-// ---- 3. scalars of the variable queries, as canonical integers:
-//   a[j] = A_j (+ L_{nc+j}),  b[j] = B_j,  abc = beta A_j + alpha B_j + C_j -> l[j - l] = abc / delta or g[j] = abc / gamma
-__global__ void setup_scalars_kernel(const FrEl* __restrict__ qa, const FrEl* __restrict__ qb,
-                                     const FrEl* __restrict__ qc, const FrEl* __restrict__ lag_inst, uint32_t m,
-                                     uint32_t l, const FrEl alpha, const FrEl beta, const FrEl ginv, const FrEl dinv,
-                                     FrEl* sa, FrEl* sb, FrEl* sl, FrEl* sg) {
-  const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
-  if (j >= m) return;
-  FrEl a = ld_vec(qa + j);
+// ---- 3. scalars of the variable queries, as canonical integers, for variable j:
+//   a = A_j (+ L_{nc+j}),  b = B_j,  abc = beta A_j + alpha B_j + C_j -> l = abc / delta (j >= l) or g = abc / gamma
+__device__ __forceinline__ FrEl setup_abc(const FrEl* __restrict__ qa, const FrEl* __restrict__ qb,
+                                          const FrEl* __restrict__ qc, const FrEl* __restrict__ lag_inst, uint64_t j,
+                                          uint64_t l, const FrEl& alpha, const FrEl& beta, FrEl& a, FrEl& b) {
+  a = ld_vec(qa + j);
   if (j < l) a = fadd(a, ld_vec(lag_inst + j));
-  const FrEl b = ld_vec(qb + j);
-  st_vec(sa + j, Fr::from_mont(a));
-  st_vec(sb + j, Fr::from_mont(b));
-  const FrEl abc = fadd(fadd(fmul(beta, a), fmul(alpha, b)), ld_vec(qc + j));
-  if (j < l) st_vec(sg + j, Fr::from_mont(fmul(abc, ginv)));
-  else st_vec(sl + j - l, Fr::from_mont(fmul(abc, dinv)));
+  b = ld_vec(qb + j);
+  return fadd(fadd(fmul(beta, a), fmul(alpha, b)), ld_vec(qc + j));
+}
+// thread t < S.ma: the shard's local variable t (global S.var(t)) -> sa[t], sb[t], and sl[t - l_skip] for a witness
+// variable; thread t < l: the gamma_abc scalar of (global) instance variable t, on every shard
+__global__ void setup_scalars_kernel(const FrEl* __restrict__ qa, const FrEl* __restrict__ qb,
+                                     const FrEl* __restrict__ qc, const FrEl* __restrict__ lag_inst, const PkShard S,
+                                     const FrEl alpha, const FrEl beta, const FrEl ginv, const FrEl dinv, FrEl* sa,
+                                     FrEl* sb, FrEl* sl, FrEl* sg) {
+  const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+  FrEl a, b;
+  if (t < S.ma) {
+    const FrEl abc = setup_abc(qa, qb, qc, lag_inst, S.var(t), S.l, alpha, beta, a, b);
+    st_vec(sa + t, Fr::from_mont(a));
+    st_vec(sb + t, Fr::from_mont(b));
+    if (t >= S.l_skip) st_vec(sl + (t - S.l_skip), Fr::from_mont(fmul(abc, dinv)));
+  }
+  if (t < S.l) st_vec(sg + t, Fr::from_mont(fmul(setup_abc(qa, qb, qc, lag_inst, t, S.l, alpha, beta, a, b), ginv)));
 }
 
-// h scalars tau^i Z(tau)/delta (i < n - 1) at bit-reversed position p = bitrev(i) of the n-padded H set; position
-// bitrev(n - 1) = n - 1 gets 0, whose multiple is the flagged identity the prover's padding expects
+// h scalars tau^i Z(tau)/delta (i < n - 1) at bit-reversed position p = bitrev(i) of the n-padded H set, for the
+// shard's positions p = h_lo + t (t < hn) -> sh[t]; position bitrev(n - 1) = n - 1 gets 0, whose multiple is the
+// flagged identity the prover's padding expects (on the shard that holds it)
 __global__ void setup_h_scalars_kernel(const FrEl* __restrict__ tlo, const FrEl* __restrict__ thi, const FrEl scale,
-                                       uint32_t log_n, FrEl* sh) {
-  const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
-  if (p >= (1u << log_n)) return;
+                                       uint32_t log_n, uint32_t h_lo, uint32_t hn, FrEl* sh) {
+  const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= hn) return;
+  const uint32_t p = h_lo + t;
   const uint32_t i = log_n == 0 ? 0 : (__brev(p) >> (32 - log_n));
-  st_vec(sh + p, i + 1 < (1u << log_n) ? Fr::from_mont(fmul(scale, pow_from_tables(tlo, thi, i))) : Fr::zero());
+  st_vec(sh + t, i + 1 < (1u << log_n) ? Fr::from_mont(fmul(scale, pow_from_tables(tlo, thi, i))) : Fr::zero());
 }
 
 // ---- host side (hostfr::Fr: 4 x u64 Montgomery limbs, the layout of FrEl)
@@ -253,25 +269,25 @@ bool fq_limbs_canonical(const uint64_t* v, int nfq) {
     if (host::fq_geq_q(v + 6 * k)) return false;
   return true;
 }
-void check_g1_generator(const uint64_t* g) {
-  B2Z_REQUIRE(!limbs_zero(g, 12), B2Z_EINVAL, "b2z_groth16_setup: g1_generator is the identity");
-  B2Z_REQUIRE(fq_limbs_canonical(g, 2), B2Z_EINVAL, "b2z_groth16_setup: g1_generator coordinate not below q");
+void check_g1_generator(const std::string& who, const uint64_t* g) {
+  B2Z_REQUIRE(!limbs_zero(g, 12), B2Z_EINVAL, who + ": g1_generator is the identity");
+  B2Z_REQUIRE(fq_limbs_canonical(g, 2), B2Z_EINVAL, who + ": g1_generator coordinate not below q");
   host::G1Aff p;
   std::memcpy(p.x.l, g, 48);
   std::memcpy(p.y.l, g + 6, 48);
   p.inf = false;
-  B2Z_REQUIRE(g1_on_curve(p.x, p.y), B2Z_EINVAL, "b2z_groth16_setup: g1_generator is not on the curve");
-  B2Z_REQUIRE(host::g1_in_subgroup(p), B2Z_EINVAL, "b2z_groth16_setup: g1_generator is not in the r-order subgroup");
+  B2Z_REQUIRE(g1_on_curve(p.x, p.y), B2Z_EINVAL, who + ": g1_generator is not on the curve");
+  B2Z_REQUIRE(host::g1_in_subgroup(p), B2Z_EINVAL, who + ": g1_generator is not in the r-order subgroup");
 }
-void check_g2_generator(const uint64_t* g) {
-  B2Z_REQUIRE(!limbs_zero(g, 24), B2Z_EINVAL, "b2z_groth16_setup: g2_generator is the identity");
-  B2Z_REQUIRE(fq_limbs_canonical(g, 4), B2Z_EINVAL, "b2z_groth16_setup: g2_generator coordinate not below q");
+void check_g2_generator(const std::string& who, const uint64_t* g) {
+  B2Z_REQUIRE(!limbs_zero(g, 24), B2Z_EINVAL, who + ": g2_generator is the identity");
+  B2Z_REQUIRE(fq_limbs_canonical(g, 4), B2Z_EINVAL, who + ": g2_generator coordinate not below q");
   host::G2Aff p;
   std::memcpy(&p.x, g, 96);
   std::memcpy(&p.y, g + 12, 96);
   p.inf = false;
-  B2Z_REQUIRE(g2_on_curve(p.x, p.y), B2Z_EINVAL, "b2z_groth16_setup: g2_generator is not on the curve");
-  B2Z_REQUIRE(host::g2_in_subgroup(p), B2Z_EINVAL, "b2z_groth16_setup: g2_generator is not in the r-order subgroup");
+  B2Z_REQUIRE(g2_on_curve(p.x, p.y), B2Z_EINVAL, who + ": g2_generator is not on the curve");
+  B2Z_REQUIRE(host::g2_in_subgroup(p), B2Z_EINVAL, who + ": g2_generator is not in the r-order subgroup");
 }
 
 // x^k for k < count as the tables lo (1024 entries) and hi (ceil(count / 1024) entries)
@@ -283,41 +299,47 @@ void pow_tables(Ctx& c, const hostfr::Fr& x, uint32_t count, DevBuf<FrEl>& lo, D
   fr_pow_table(&c, hi.p, dev_el(hostfr::fr_pow_u64(x, 1024)), nhi ? nhi : 1, st);
 }
 
-void groth16_setup(Ctx& c, b2z_r1cs* r1cs, const b2z_setup_desc* d, b2z_pk** pk_out, b2z_vk_out* vk) {
+// shard `rank` of `world` (pk_shard's rule, as b2z_pk_upload_shard applies it); world == 1: the whole key
+void groth16_setup(Ctx& c, const char* who_c, b2z_r1cs* r1cs, const b2z_setup_desc* d, uint32_t rank, uint32_t world,
+                   b2z_pk** pk_out, b2z_vk_out* vk) {
   using namespace hostfr;   // fr_* host arithmetic
-  B2Z_REQUIRE(d != nullptr && pk_out != nullptr && vk != nullptr, B2Z_EINVAL, "b2z_groth16_setup: NULL argument");
-  B2Z_REQUIRE(d->alpha && d->beta && d->gamma && d->delta && d->tau, B2Z_EINVAL,
-              "b2z_groth16_setup: NULL toxic-waste element");
-  B2Z_REQUIRE(vk->gamma_abc_g1 && vk->gamma_abc_inf, B2Z_EINVAL, "b2z_groth16_setup: NULL vk_out array");
-  const R1csView R = r1cs_view(c, r1cs, "b2z_groth16_setup");
+  const std::string who = who_c;
+  B2Z_REQUIRE(d != nullptr && pk_out != nullptr && vk != nullptr, B2Z_EINVAL, who + ": NULL argument");
+  B2Z_REQUIRE(world >= 1 && rank < world, B2Z_EINVAL, who + ": need rank < world");
+  B2Z_REQUIRE(d->alpha && d->beta && d->gamma && d->delta && d->tau, B2Z_EINVAL, who + ": NULL toxic-waste element");
+  B2Z_REQUIRE(vk->gamma_abc_g1 && vk->gamma_abc_inf, B2Z_EINVAL, who + ": NULL vk_out array");
+  const R1csView R = r1cs_view(c, r1cs, who_c);
   const uint64_t nc = R.nc, l = R.l, m = R.m;
   const uint32_t log_n = R.log_n;
-  B2Z_REQUIRE(log_n <= 26, B2Z_ENOMEM, "b2z_groth16_setup: domain does not fit this build's single-GPU plan");
-  B2Z_REQUIRE(m < (1ull << 26), B2Z_ESIZE, "b2z_groth16_setup: too many variables");
+  B2Z_REQUIRE(log_n <= 26, B2Z_ENOMEM, who + ": domain does not fit this build's single-GPU plan");
+  B2Z_REQUIRE(m < (1ull << 26), B2Z_ESIZE, who + ": too many variables");
   const char* names[5] = {"alpha", "beta", "gamma", "delta", "tau"};
   const uint64_t* els[5] = {d->alpha, d->beta, d->gamma, d->delta, d->tau};
   for (int k = 0; k < 5; k++)
-    B2Z_REQUIRE(fr_is_canonical(els[k]), B2Z_EINVAL, std::string("b2z_groth16_setup: ") + names[k] + " is not below r");
+    B2Z_REQUIRE(fr_is_canonical(els[k]), B2Z_EINVAL, who + ": " + names[k] + " is not below r");
   const hostfr::Fr alpha = host_el(d->alpha), beta = host_el(d->beta), gamma = host_el(d->gamma),
                    delta = host_el(d->delta), tau = host_el(d->tau);
-  B2Z_REQUIRE(!fr_is_zero(gamma), B2Z_EINVAL, "b2z_groth16_setup: gamma is zero (it has no inverse)");
-  B2Z_REQUIRE(!fr_is_zero(delta), B2Z_EINVAL, "b2z_groth16_setup: delta is zero (it has no inverse)");
+  B2Z_REQUIRE(!fr_is_zero(gamma), B2Z_EINVAL, who + ": gamma is zero (it has no inverse)");
+  B2Z_REQUIRE(!fr_is_zero(delta), B2Z_EINVAL, who + ": delta is zero (it has no inverse)");
   const uint64_t n = 1ull << log_n;
   hostfr::Fr tn = tau;
   for (uint32_t i = 0; i < log_n; i++) tn = fr_mul(tn, tn);
   const hostfr::Fr zt = fr_sub(tn, fr_one());   // Z(tau) = tau^n - 1
-  B2Z_REQUIRE(!fr_is_zero(zt), B2Z_EINVAL, "b2z_groth16_setup: tau lies in the evaluation domain (tau^n = 1)");
-  if (d->g1_generator) check_g1_generator(d->g1_generator);
-  if (d->g2_generator) check_g2_generator(d->g2_generator);
+  B2Z_REQUIRE(!fr_is_zero(zt), B2Z_EINVAL, who + ": tau lies in the evaluation domain (tau^n = 1)");
+  if (d->g1_generator) check_g1_generator(who, d->g1_generator);
+  if (d->g2_generator) check_g2_generator(who, d->g2_generator);
 
-  const bool pre = pk_precompute_fits(log_n, m, l);   // before this call's own allocations, as b2z_pk_upload decides
+  // the shard, and b2z_pk_upload_shard's decision on window copies, before this call's own allocations
+  const PkShard S = pk_shard(log_n, m, l, rank, rank + 1, world, rank, world);
+  const bool pre = pk_precompute_fits_slice(log_n, m, l, 1, world);
+  const uint32_t vk_terms = S.with_vk ? 2 : 0;   // alpha/beta/delta tails of the a, b1, b2 sets (l: delta)
   cudaStream_t st = c.stream;
   const uint32_t nl = (uint32_t)(nc + l);
   hostfr::Fr w = fr_two_adic_root();
   for (uint32_t i = log_n; i < 32; i++) w = fr_mul(w, w);
   const hostfr::Fr dinv = fr_inv(delta), ginv = fr_inv(gamma);
 
-  // 1. Lagrange coefficients
+  // 1. Lagrange coefficients (every variable's QAP terms need them, so every shard computes them all)
   DevBuf<FrEl> lag(nl);
   {
     DevBuf<FrEl> wlo, whi;
@@ -328,32 +350,41 @@ void groth16_setup(Ctx& c, b2z_r1cs* r1cs, const b2z_setup_desc* d, b2z_pk** pk_
     B2Z_LAUNCHED(&c);
     B2Z_CUDA(cudaStreamSynchronize(st));
   }
-  // 2. QAP evaluation
+  // 2. QAP evaluation, for all m variables (cheap: the shard's own are picked out by the scalar kernel)
   DevBuf<FrEl> q[3] = {DevBuf<FrEl>(m), DevBuf<FrEl>(m), DevBuf<FrEl>(m)};
   for (int k = 0; k < 3; k++) qap_eval(c, R.mat[k], (uint32_t)nc, (uint32_t)m, lag.p, q[k].p, st);
-  // 3. scalars; the set tails (alpha delta | beta delta | delta) as canonical integers from the host
-  DevBuf<FrEl> sa(m + 2), sb(m + 2), sl(m - l + 1), sg(l), sh(n), sgamma(1);
-  setup_scalars_kernel<<<nblocks(m, 128), 128, 0, st>>>(q[0].p, q[1].p, q[2].p, lag.p + nc, (uint32_t)m, (uint32_t)l,
-                                                         dev_el(alpha), dev_el(beta), dev_el(ginv), dev_el(dinv), sa.p,
-                                                         sb.p, sl.p, sg.p);
+  // 3. the shard's scalars and gamma_abc's; the set tails (alpha delta | beta delta | delta) and the verifying key's
+  // points (alpha after gamma_abc | beta gamma delta) as canonical integers from the host
+  DevBuf<FrEl> sa(S.ma + vk_terms), sb(S.ma + vk_terms), sl(S.ml + vk_terms / 2), sg(l + 1), sh(S.hn), sv2(3);
+  setup_scalars_kernel<<<nblocks(S.ma > l ? S.ma : l, 128), 128, 0, st>>>(
+      q[0].p, q[1].p, q[2].p, lag.p + nc, S, dev_el(alpha), dev_el(beta), dev_el(ginv), dev_el(dinv), sa.p, sb.p,
+      sl.p, sg.p);
   B2Z_LAUNCHED(&c);
   const hostfr::Fr tails[6] = {fr_into_bigint(alpha), fr_into_bigint(delta), fr_into_bigint(beta),
                                fr_into_bigint(delta), fr_into_bigint(gamma), fr_into_bigint(delta)};
-  B2Z_CUDA(cudaMemcpyAsync(sa.p + m, &tails[0], 64, cudaMemcpyHostToDevice, st));
-  B2Z_CUDA(cudaMemcpyAsync(sb.p + m, &tails[2], 64, cudaMemcpyHostToDevice, st));
-  B2Z_CUDA(cudaMemcpyAsync(sl.p + (m - l), &tails[5], 32, cudaMemcpyHostToDevice, st));
-  B2Z_CUDA(cudaMemcpyAsync(sgamma.p, &tails[4], 32, cudaMemcpyHostToDevice, st));
+  if (S.with_vk) {
+    B2Z_CUDA(cudaMemcpyAsync(sa.p + S.ma, &tails[0], 64, cudaMemcpyHostToDevice, st));
+    B2Z_CUDA(cudaMemcpyAsync(sb.p + S.ma, &tails[2], 64, cudaMemcpyHostToDevice, st));
+    B2Z_CUDA(cudaMemcpyAsync(sl.p + S.ml, &tails[5], 32, cudaMemcpyHostToDevice, st));
+  }
+  const hostfr::Fr vk_g2[3] = {tails[2], tails[4], tails[5]};   // beta | gamma | delta
+  B2Z_CUDA(cudaMemcpyAsync(sg.p + l, &tails[0], 32, cudaMemcpyHostToDevice, st));
+  B2Z_CUDA(cudaMemcpyAsync(sv2.p, vk_g2, 96, cudaMemcpyHostToDevice, st));
   {
     DevBuf<FrEl> tlo, thi;
     pow_tables(c, tau, (uint32_t)n, tlo, thi, st);
-    setup_h_scalars_kernel<<<nblocks(n, 128), 128, 0, st>>>(tlo.p, thi.p, dev_el(fr_mul(zt, dinv)), log_n, sh.p);
-    B2Z_LAUNCHED(&c);
+    if (S.hn) {
+      setup_h_scalars_kernel<<<nblocks(S.hn, 128), 128, 0, st>>>(tlo.p, thi.p, dev_el(fr_mul(zt, dinv)), log_n, S.h_lo,
+                                                                  S.hn, sh.p);
+      B2Z_LAUNCHED(&c);
+    }
     B2Z_CUDA(cudaStreamSynchronize(st));
   }
   lag.release();
   for (auto& v : q) v.release();
 
-  // 4. fixed-base multiplications with the caller's generators (a table of their own) or the standard ones (cached)
+  // 4. fixed-base multiplications with the caller's generators (a table of their own) or the standard ones (cached),
+  // on the shard's scalars only
   FbTable<G1> own1;
   FbTable<G2> own2;
   if (d->g1_generator) {
@@ -369,32 +400,34 @@ void groth16_setup(Ctx& c, b2z_r1cs* r1cs, const b2z_setup_desc* d, b2z_pk** pk_
   const FbTable<G1>& t1 = d->g1_generator ? own1 : fb_standard_table<G1>(&c, st);
   const FbTable<G2>& t2 = d->g2_generator ? own2 : fb_standard_table<G2>(&c, st);
   auto words = [](uint64_t count) { return DevBuf<uint32_t>((count + 31) / 32 + 1); };
-  DevBuf<G1::Affine> pa(m + 2), pb1(m + 2), pl(m - l + 1), ph(n), pg(l);
-  DevBuf<G2::Affine> pb2(m + 2), pgamma(1);
-  DevBuf<uint32_t> wa = words(m + 2), wb1 = words(m + 2), wl = words(m - l + 1), wh = words(n), wg = words(l),
-                   wb2 = words(m + 2), wgamma = words(1);
-  fixed_base_mul<G1>(&c, t1, sa.p, pa.p, wa.p, (uint32_t)m + 2, st);
-  fixed_base_mul<G1>(&c, t1, sb.p, pb1.p, wb1.p, (uint32_t)m + 2, st);
-  fixed_base_mul<G1>(&c, t1, sl.p, pl.p, wl.p, (uint32_t)(m - l) + 1, st);
-  fixed_base_mul<G1>(&c, t1, sh.p, ph.p, wh.p, (uint32_t)n, st);
-  fixed_base_mul<G1>(&c, t1, sg.p, pg.p, wg.p, (uint32_t)l, st);
-  fixed_base_mul<G2>(&c, t2, sb.p, pb2.p, wb2.p, (uint32_t)m + 2, st);
-  fixed_base_mul<G2>(&c, t2, sgamma.p, pgamma.p, wgamma.p, 1, st);
+  const uint32_t na = S.ma + vk_terms, nl1 = S.ml + vk_terms / 2;
+  DevBuf<G1::Affine> pa(na), pb1(na), pl(nl1), ph(S.hn), pg(l + 1);
+  DevBuf<G2::Affine> pb2(na), pv2(3);
+  DevBuf<uint32_t> wa = words(na), wb1 = words(na), wl = words(nl1), wh = words(S.hn), wg = words(l + 1),
+                   wb2 = words(na), wv2 = words(3);
+  fixed_base_mul<G1>(&c, t1, sa.p, pa.p, wa.p, na, st);
+  fixed_base_mul<G1>(&c, t1, sb.p, pb1.p, wb1.p, na, st);
+  fixed_base_mul<G1>(&c, t1, sl.p, pl.p, wl.p, nl1, st);
+  fixed_base_mul<G1>(&c, t1, sh.p, ph.p, wh.p, S.hn, st);
+  fixed_base_mul<G1>(&c, t1, sg.p, pg.p, wg.p, (uint32_t)l + 1, st);
+  fixed_base_mul<G2>(&c, t2, sb.p, pb2.p, wb2.p, na, st);
+  fixed_base_mul<G2>(&c, t2, sv2.p, pv2.p, wv2.p, 3, st);
 
-  // 5. verifying key: alpha_1 and beta_2, delta_2 from the set tails, gamma_2, gamma_abc
+  // 5. verifying key, whole on every shard: alpha_1, beta_2 gamma_2 delta_2, gamma_abc
   std::vector<uint32_t> gw((l + 31) / 32);
-  B2Z_CUDA(cudaMemcpyAsync(vk->alpha_g1, pa.p + m, sizeof(G1::Affine), cudaMemcpyDeviceToHost, st));
-  B2Z_CUDA(cudaMemcpyAsync(vk->beta_g2, pb2.p + m, sizeof(G2::Affine), cudaMemcpyDeviceToHost, st));
-  B2Z_CUDA(cudaMemcpyAsync(vk->delta_g2, pb2.p + m + 1, sizeof(G2::Affine), cudaMemcpyDeviceToHost, st));
-  B2Z_CUDA(cudaMemcpyAsync(vk->gamma_g2, pgamma.p, sizeof(G2::Affine), cudaMemcpyDeviceToHost, st));
+  B2Z_CUDA(cudaMemcpyAsync(vk->alpha_g1, pg.p + l, sizeof(G1::Affine), cudaMemcpyDeviceToHost, st));
+  B2Z_CUDA(cudaMemcpyAsync(vk->beta_g2, pv2.p, sizeof(G2::Affine), cudaMemcpyDeviceToHost, st));
+  B2Z_CUDA(cudaMemcpyAsync(vk->gamma_g2, pv2.p + 1, sizeof(G2::Affine), cudaMemcpyDeviceToHost, st));
+  B2Z_CUDA(cudaMemcpyAsync(vk->delta_g2, pv2.p + 2, sizeof(G2::Affine), cudaMemcpyDeviceToHost, st));
   B2Z_CUDA(cudaMemcpyAsync(vk->gamma_abc_g1, pg.p, l * sizeof(G1::Affine), cudaMemcpyDeviceToHost, st));
   B2Z_CUDA(cudaMemcpyAsync(gw.data(), wg.p, gw.size() * 4, cudaMemcpyDeviceToHost, st));
   B2Z_CUDA(cudaStreamSynchronize(st));
   std::memcpy(vk->gamma_abc_inf, gw.data(), (l + 7) / 8);
+  if (l % 8) vk->gamma_abc_inf[l / 8] &= (uint8_t)((1u << (l % 8)) - 1);   // not alpha_1's bit
 
-  // 6. the key, assembled as b2z_pk_upload assembles it
+  // 6. the key, assembled as b2z_pk_upload_shard assembles it
   const PkDeviceSets sets{pa.p, pb1.p, pl.p, ph.p, pb2.p, wa.p, wb1.p, wl.p, wh.p, wb2.p};
-  *pk_out = pk_from_device_sets(c, log_n, m, l, sets, pre);
+  *pk_out = pk_from_device_sets(c, S, sets, pre);
 }
 
 }  // namespace
@@ -403,5 +436,15 @@ void groth16_setup(Ctx& c, b2z_r1cs* r1cs, const b2z_setup_desc* d, b2z_pk** pk_
 extern "C" b2z_status b2z_groth16_setup(b2z_ctx* ctx, b2z_r1cs* r1cs, const b2z_setup_desc* desc, b2z_pk** pk_out,
                                         b2z_vk_out* vk_out) {
   if (pk_out) *pk_out = nullptr;
-  return b2z::guarded(ctx, [&](b2z::Ctx& c) { b2z::groth16_setup(c, r1cs, desc, pk_out, vk_out); });
+  return b2z::guarded(ctx, [&](b2z::Ctx& c) {
+    b2z::groth16_setup(c, "b2z_groth16_setup", r1cs, desc, 0, 1, pk_out, vk_out);
+  });
+}
+
+extern "C" b2z_status b2z_groth16_setup_shard(b2z_ctx* ctx, b2z_r1cs* r1cs, const b2z_setup_desc* desc, uint32_t rank,
+                                              uint32_t world, b2z_pk** pk_out, b2z_vk_out* vk_out) {
+  if (pk_out) *pk_out = nullptr;
+  return b2z::guarded(ctx, [&](b2z::Ctx& c) {
+    b2z::groth16_setup(c, "b2z_groth16_setup_shard", r1cs, desc, rank, world, pk_out, vk_out);
+  });
 }

@@ -733,12 +733,18 @@ class Groth16:
         return pk, vk
 
     @staticmethod
-    def generate_parameters_on_device(ctx, cm, alpha, beta, gamma, delta, tau, g1_generator=None, g2_generator=None):
+    def generate_parameters_on_device(ctx, cm, alpha, beta, gamma, delta, tau, g1_generator=None, g2_generator=None,
+                                      rank=0, world=1):
         """generate_parameters_with_qap for uploaded matrices, entirely on the GPU (b2z_groth16_setup), with the
         caller's toxic waste (canonical ints) and generators (affine Montgomery limb arrays, 12 / 24 uint64; None = the
         standard ones) -- what Groth16::setup does after its draws (oracle/ark_rng.py: setup_draws gives them in ark's
         order).  Returns (ProvingKey, VerifyingKey).  The ProvingKey is already uploaded through ctx; its host arrays
-        stay None until pk.download()."""
+        stay None until pk.download().
+
+        rank / world (b2z_groth16_setup_shard): only shard `rank` of `world` of the key is made, the shard that
+        pk.upload(ctx, rank, world) makes of the whole key; the ProvingKey is that shard (DistributedProver and
+        create_proof_partial* take it as it is) and cannot be downloaded.  The VerifyingKey is the whole one on every
+        rank.  Every rank passes the same toxic waste and generators."""
         cm.upload(ctx)
         els = codec.fr_to_mont_limbs([alpha, beta, gamma, delta, tau])
         keep = [els]
@@ -757,11 +763,16 @@ class Groth16:
         vk_out = _ffi.VkOut()
         vk_out.gamma_abc_g1, vk_out.gamma_abc_inf = _ptr(gabc), _ptr(gabc_inf)
         h = ctypes.c_void_p()
-        ctx.check(ctx._lib.b2z_groth16_setup(ctx.handle, cm._handle, ctypes.byref(d), ctypes.byref(h),
-                                             ctypes.byref(vk_out)))
+        rank, world = int(rank), int(world)
+        if (rank, world) == (0, 1):
+            ctx.check(ctx._lib.b2z_groth16_setup(ctx.handle, cm._handle, ctypes.byref(d), ctypes.byref(h),
+                                                 ctypes.byref(vk_out)))
+        else:
+            ctx.check(ctx._lib.b2z_groth16_setup_shard(ctx.handle, cm._handle, ctypes.byref(d), rank, world,
+                                                       ctypes.byref(h), ctypes.byref(vk_out)))
         pk = ProvingKey(m, l, n, None, None, None, None, None, None, None, None, None, None)
-        pk._ctx, pk._handle, pk._spec = ctx, h, (0, 1, None)
-        pk.shard = (0, 1)
+        pk._ctx, pk._handle, pk._spec = ctx, h, (rank, world, None)
+        pk.shard = (rank, world)
         pt = lambda arr, w: np.array(arr[:w], dtype=np.uint64)
         vk = VerifyingKey(pt(vk_out.alpha_g1, 12), pt(vk_out.beta_g2, 24), pt(vk_out.gamma_g2, 24),
                           pt(vk_out.delta_g2, 24), (gabc, gabc_inf))

@@ -8,6 +8,7 @@
 //! | `Radix2EvaluationDomain::{fft,ifft}_in_place`, `get_coset`                                | [`ntt_in_place`] |
 //! | `prepare_verifying_key` + `serialize_compressed` (matrix_proof.rs:134-136, io.rs:62-68)    | [`prepared_vk_bytes`] |
 //! | `Groth16::verify_with_processed_vk` (matrix_proof.rs:199-206)                              | [`verify_with_processed_vk`] |
+//! | the same for many proofs against one pvk, on the GPU, one verdict per proof                | [`verify_batch_with_processed_vk`] |
 //! | `Groth16::<Bls12_381>::setup` (matrix_proof.rs:128-131, fibbonaci_handler.rs:107)          | [`DeviceKey::setup`] |
 //!
 //! SOURCE ONLY -- never compiled in the build image (no Rust toolchain there).  arkworks' `Fp` / `Affine` are
@@ -97,6 +98,8 @@ pub mod sys {
         pub fn b2z_groth16_prepare_verifying_key(vk: *const b2z_vk_desc, pvk_out: *mut u8, capacity: u64, pvk_len: *mut u64) -> i32;
         pub fn b2z_groth16_verify_with_processed_vk(pvk: *const u8, pvk_len: u64, public_inputs: *const u64, num_inputs: u64,
                                                     proof: *const u8, valid: *mut i32) -> i32;
+        pub fn b2z_groth16_verify_batch(ctx: *mut b2z_ctx, pvk: *const u8, pvk_len: u64, public_inputs: *const u64,
+                                        num_inputs: u64, proofs: *const u8, count: u64, results: *mut i32) -> i32;
         // key-generation scalars on the host cores (no ctx): see INTEGRATION.md section 7
         pub fn b2z_fr_lagrange_at(log_n: u32, tau: *const u64, count: u64, threads: u32, out: *mut u64) -> i32;
         pub fn b2z_fr_geometric(base: *const u64, scale: *const u64, count: u64, threads: u32, out: *mut u64) -> i32;
@@ -460,6 +463,30 @@ pub fn verify_with_processed_vk(pvk: &[u8], public_inputs: &[Fr], proof: &[u8; 1
     };
     if st != B2Z_OK { return Err(SynthesisError::MalformedVerifyingKey); }
     Ok(valid == 1)
+}
+
+/// `verify_with_processed_vk` for many proofs against one pvk on ctx's GPU (b2z_groth16_verify_batch): one verdict
+/// per proof, `None` where the single-proof call would return an error (malformed encoding, point outside the
+/// subgroup).  Every proof takes the same number of inputs.  Err for what fails the whole call: malformed pvk, a
+/// wrong input count, more than 1024 inputs.
+pub fn verify_batch_with_processed_vk(ctx: &Context, pvk: &[u8], inputs: &[Vec<Fr>], proofs: &[[u8; 192]])
+                                      -> Result<Vec<Option<bool>>, SynthesisError> {
+    if inputs.len() != proofs.len() { return Err(SynthesisError::MalformedVerifyingKey); }
+    if proofs.is_empty() { return Ok(Vec::new()); }
+    let n = inputs[0].len();
+    if inputs.iter().any(|x| x.len() != n) { return Err(SynthesisError::MalformedVerifyingKey); }
+    let x: Vec<u64> = inputs.iter().flat_map(|v| pack_fr(v)).collect();
+    let bytes: Vec<u8> = proofs.iter().flat_map(|p| p.iter().copied()).collect();
+    let mut results = vec![0i32; proofs.len()];
+    let st = unsafe {
+        b2z_groth16_verify_batch(ctx.raw, pvk.as_ptr(), pvk.len() as u64, if n > 0 { x.as_ptr() } else { ptr::null() },
+                                 n as u64, bytes.as_ptr(), proofs.len() as u64, results.as_mut_ptr())
+    };
+    match st {
+        B2Z_OK => Ok(results.iter().map(|&r| if r < 0 { None } else { Some(r == 1) }).collect()),
+        B2Z_EINVAL | B2Z_ESIZE => Err(SynthesisError::MalformedVerifyingKey),
+        _ => status(ctx.raw, st).map(|_| Vec::new()),
+    }
 }
 
 #[allow(dead_code)]

@@ -285,6 +285,23 @@ B2Z_API b2z_status b2z_groth16_verify_with_processed_vk(const uint8_t* pvk, uint
                                                         const uint64_t* public_inputs, uint64_t num_inputs,
                                                         const uint8_t proof[192], int32_t* valid);
 
+/* Groth16::verify_with_processed_vk for `count` proofs against ONE prepared verifying key, on ctx's GPU.
+ *   pvk, pvk_len  : PreparedVerifyingKey::serialize_compressed bytes (as for b2z_groth16_verify_with_processed_vk)
+ *   public_inputs : count x num_inputs Fr elements (Montgomery limbs, WITHOUT the leading 1), proof-major
+ *   proofs        : count x 192 bytes (A 48 | B 96 | C 48, compressed)
+ *   results       : count int32: 1 valid, 0 not valid, -1 = b2z_groth16_verify_with_processed_vk would return
+ *                   B2Z_EINVAL for this proof alone (malformed encoding, point off the curve or outside the
+ *                   subgroup, an input >= r)
+ * For every i, results[i] is what b2z_groth16_verify_with_processed_vk gives for (pvk, inputs_i, proof_i): one
+ * verdict per proof, not a single check of the whole batch.
+ * B2Z_EINVAL, results not written: malformed pvk, num_inputs + 1 != the pvk's gamma_abc count, NULL buffers with
+ * count > 0, a prepared G2 line list that is neither infinite nor 68 long (the host verifier's call-level errors).
+ * B2Z_ESIZE: num_inputs > 1024.  count == 0: B2Z_OK, no GPU work.  Host buffers; proofs go through the device in
+ * chunks of 65536, so device memory stays bounded whatever count is.                                              */
+B2Z_API b2z_status b2z_groth16_verify_batch(b2z_ctx* ctx, const uint8_t* pvk, uint64_t pvk_len,
+                                            const uint64_t* public_inputs, uint64_t num_inputs,
+                                            const uint8_t* proofs, uint64_t count, int32_t* results);
+
 /* ---- key-generation scalars on the host, multithreaded (row f3; no GPU, no ctx) ---------------------------------
  * ark_groth16's generate_parameters_with_qap (Groth16::setup, matrix_proof.rs:128-131) = O(n) scalar preparation + fixed-
  * base multiplications.  The multiplications are b2z_fixed_base_mul_g1/g2 (and b2z_spmv_fr for the QAP evaluation at
@@ -496,6 +513,15 @@ B2Z_API uint32_t b2z_host_msm_window_bits(uint64_t n, int precomputed);
  * serialised compressed (48 / 96 bytes) into out                                                                */
 B2Z_API int b2z_host_planes_horner(int group /*1|2*/, const uint32_t* planes_xyzz, uint32_t nplanes, uint32_t chunk_log,
                                    uint8_t* out);
+/* b2z_groth16_verify_batch's per-proof device code (csrc/pairing.cuh: decode, Miller loop, final exponentiation) run
+ * on the host for one proof, with the batch call's call-level checks and statuses; *result = 1 / 0 / -1.          */
+B2Z_API b2z_status b2z_host_verify_one(const uint8_t* pvk, uint64_t pvk_len, const uint64_t* public_inputs,
+                                       uint64_t num_inputs, const uint8_t proof[192], int32_t* result);
+/* pairing.cuh's tower pieces next to csrc/host_pairing.hpp's on canonical Montgomery limbs (Fq12 = 144 u32 in tower
+ * order c0.c0.c0 .. c1.c2.c1, Fq2 = 24 u32): op 0 a * b, 1 a^2, 2 a^q, 3 final exponentiation, 4 an Fq2 square root
+ * (the root that is not lexicographically largest).  out_dev / out_host: the two results, canonical.  Returns 0; for
+ * op 3, 1 when a != 0 (-2 when the sides disagree); for op 4, (root on the device side) + 2 (root on the host side). */
+B2Z_API int b2z_host_pairing_op(int op, const uint32_t* a, const uint32_t* b, uint32_t* out_dev, uint32_t* out_host);
 
 #ifdef __cplusplus
 }

@@ -108,6 +108,8 @@ SIGNATURES = {
                                                             ctypes.POINTER(ctypes.c_uint64)]),
     "b2z_groth16_verify_with_processed_vk": (ctypes.c_int32, [vp, ctypes.c_uint64, vp, ctypes.c_uint64, vp,
                                                                ctypes.POINTER(ctypes.c_int32)]),
+    "b2z_groth16_verify_batch": (ctypes.c_int32, [vp, vp, ctypes.c_uint64, vp, ctypes.c_uint64, vp, ctypes.c_uint64,
+                                                   vp]),
     "b2z_dist_shared_bytes": (ctypes.c_uint64, [ctypes.c_uint32]),
     "b2z_dist_combine_shared": (ctypes.c_int32, [vp, ctypes.c_uint32, ctypes.c_uint32, ctypes.POINTER(ctypes.c_uint32), vp,
                                                   vp]),
@@ -140,6 +142,8 @@ SIGNATURES = {
     "b2z_host_msm_digits": (ctypes.c_uint32, [vp, ctypes.c_uint32, vp]),
     "b2z_host_msm_window_bits": (ctypes.c_uint32, [ctypes.c_uint64, ctypes.c_int]),
     "b2z_host_planes_horner": (ctypes.c_int, [ctypes.c_int, vp, ctypes.c_uint32, ctypes.c_uint32, vp]),
+    "b2z_host_verify_one": (ctypes.c_int32, [vp, ctypes.c_uint64, vp, ctypes.c_uint64, vp, ctypes.POINTER(ctypes.c_int32)]),
+    "b2z_host_pairing_op": (ctypes.c_int, [ctypes.c_int, vp, vp, vp, vp]),
 }
 
 _lib = None

@@ -10,6 +10,7 @@
 #include "host_fq.hpp"
 #include "inv_gcd.cuh"
 #include "msm.hpp"
+#include "verify_key.hpp"
 
 using namespace b2z;
 
@@ -115,6 +116,13 @@ int accum_affine_check(const uint32_t* points_raw, const uint32_t* sorted, const
   return bad;
 }
 
+template <class T>
+T load(const uint32_t* src) {
+  T v;
+  std::memcpy(&v, src, sizeof(T));
+  return v;
+}
+
 }  // namespace
 
 extern "C" {
@@ -169,5 +177,84 @@ int b2z_host_planes_horner(int group, const uint32_t* planes_xyzz, uint32_t npla
 }
 
 uint32_t b2z_host_msm_window_bits(uint64_t n, int precomputed) { return msm_pick_c(n, precomputed != 0); }
+
+// Groth16::verify_with_processed_vk for one proof through the per-thread code of b2z_groth16_verify_batch's three
+// kernels (pairing.cuh), with the same call-level checks.  *result: 1 / 0 / -1 as in the batch call.
+b2z_status b2z_host_verify_one(const uint8_t* pvk, uint64_t pvk_len, const uint64_t* public_inputs, uint64_t num_inputs,
+                               const uint8_t proof[192], int32_t* result) {
+  if (pvk == nullptr || proof == nullptr || result == nullptr || (num_inputs && public_inputs == nullptr))
+    return B2Z_EINVAL;
+  if (num_inputs > pairing::kMaxInputs) return B2Z_ESIZE;
+  host::PreparedVk k;
+  if (!host::pvk_deserialize(pvk, pvk_len, &k) || pairing::key_error(k, num_inputs) != nullptr) return B2Z_EINVAL;
+  const pairing::KeyArrays ka = pairing::key_arrays(k);
+  const pairing::KeyView kv = pairing::key_view(ka, ka.abc.data(), ka.abc_inf.data(), ka.lines.data());
+  pairing::ProofPoints pts;
+  pairing::verify_decode(proof, reinterpret_cast<const FrEl*>(public_inputs), kv, &pts);
+  if (pts.flags & pairing::PT_MALFORMED) {
+    *result = -1;
+    return B2Z_OK;
+  }
+  pairing::Fq12El f;
+  pairing::verify_miller(pts, kv, &f);
+  *result = pairing::verify_final(f, ka.fp.alpha_beta, ka.fp.fc);
+  return B2Z_OK;
+}
+
+// The tower pieces of pairing.cuh next to host_pairing.hpp's, on canonical Montgomery limbs (Fq12: 144 u32, Fq2: 24):
+// op 0 a * b, 1 a^2, 2 a^q, 3 final exponentiation of a, 4 a square root of the Fq2 element a (out: the root that is
+// not lexicographically largest).  out_dev / out_host receive the two results (canonical).  Returns 0, except for
+// op 3: 1 when a != 0 (both sides), and op 4: 1 when a root exists on the device side + 2 when on the host side.
+int b2z_host_pairing_op(int op, const uint32_t* a, const uint32_t* b, uint32_t* out_dev, uint32_t* out_host) {
+  using pairing::Fq12El;
+  if (a == nullptr || out_dev == nullptr || out_host == nullptr || (op == 0 && b == nullptr)) return -1;
+  if (op == 4) {
+    const Fq2El x = load<Fq2El>(a);
+    Fq2El r;
+    const bool dev_ok = pairing::fq2_sqrt(x, &r);
+    if (dev_ok && pairing::fq2_is_larger(r)) r = Fq2::neg(r);
+    r = Fq2::reduce(r);
+    std::memcpy(out_dev, &r, sizeof(r));
+    host::Fq2 h, hr;
+    std::memcpy(&h, a, sizeof(h));
+    const bool host_ok = host::fq2_sqrt(h, &hr);
+    if (host_ok && host::fq2_is_larger(hr)) hr = host::fq2_neg(hr);
+    std::memcpy(out_host, &hr, sizeof(hr));
+    return (dev_ok ? 1 : 0) + (host_ok ? 2 : 0);
+  }
+  if (op < 0 || op > 3) return -1;
+  const Fq12El x = load<Fq12El>(a);
+  const pairing::FrobConsts fc = pairing::frobenius_consts();
+  host::Fq12 hx, hy, hr;
+  std::memcpy(&hx, a, sizeof(hx));
+  Fq12El r = pairing::fq12_one();
+  int ret = 0;
+  switch (op) {
+    case 0:
+      std::memcpy(&hy, b, sizeof(hy));
+      r = pairing::fq12_mul(x, load<Fq12El>(b));
+      hr = host::fq12_mul(hx, hy);
+      break;
+    case 1:
+      r = pairing::fq12_sqr(x);
+      hr = host::fq12_sqr(hx);
+      break;
+    case 2:
+      r = pairing::fq12_frobenius(x, fc);
+      hr = host::fq12_frobenius(hx);
+      break;
+    default: {
+      const bool dev_ok = pairing::final_exponentiation(x, fc, &r);
+      const bool host_ok = host::final_exponentiation(hx, &hr);
+      if (dev_ok != host_ok) return -2;
+      if (!dev_ok) { r = Fq12El{pairing::fq6_zero(), pairing::fq6_zero()}; hr = host::Fq12{host::fq6_zero(), host::fq6_zero()}; }
+      ret = dev_ok ? 1 : 0;
+    }
+  }
+  r = pairing::fq12_reduce(r);
+  std::memcpy(out_dev, &r, sizeof(r));
+  std::memcpy(out_host, &hr, sizeof(hr));
+  return ret;
+}
 
 }  // extern "C"

@@ -959,3 +959,32 @@ class Groth16:
         if st != _ffi.B2Z_OK:
             raise SynthesisError("MalformedVerifyingKey / malformed proof or inputs (status %d)" % st)
         return bool(ok.value)
+
+    @staticmethod
+    def verify_batch_with_processed_vk(ctx, pvk_bytes, public_inputs, proofs):
+        """verify_with_processed_vk for many proofs against one pvk, on ctx's GPU (b2z_groth16_verify_batch).
+        public_inputs: one list of canonical ints per proof (WITHOUT the leading 1), all of one length; proofs: 192
+        bytes each.  Returns one verdict per proof: True / False, or None where the single-proof call would raise
+        SynthesisError (malformed encoding, point outside the subgroup, input >= r).  Raises SynthesisError for what
+        fails the whole call: malformed pvk, a wrong number of inputs, more than 1024 inputs."""
+        count = len(proofs)
+        if len(public_inputs) != count:
+            raise ValueError("one list of public inputs per proof")
+        if count == 0:
+            return []
+        n = len(public_inputs[0])
+        if any(len(x) != n for x in public_inputs):
+            raise SynthesisError("MalformedVerifyingKey: proofs of one batch take the same number of inputs")
+        blob = b"".join(bytes(p) for p in proofs)
+        if len(blob) != 192 * count or any(len(bytes(p)) != 192 for p in proofs):
+            raise SynthesisError("proof must be 192 bytes")
+        pvk = np.frombuffer(bytes(pvk_bytes), dtype=np.uint8).copy()
+        pr = np.frombuffer(blob, dtype=np.uint8).copy()
+        x = codec.fr_to_mont_limbs([int(v) for row in public_inputs for v in row]) if n else None
+        res = np.zeros(count, dtype=np.int32)
+        st = _ffi.lib().b2z_groth16_verify_batch(ctx.handle, _ptr(pvk), pvk.size, _ptr(x) if n else None, n, _ptr(pr),
+                                                 count, _ptr(res))
+        if st in (_ffi.B2Z_EINVAL, _ffi.B2Z_ESIZE):
+            raise SynthesisError("MalformedVerifyingKey / malformed batch (status %d)" % st)
+        ctx.check(st)
+        return [None if r < 0 else bool(r) for r in res.tolist()]
